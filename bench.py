@@ -1,6 +1,7 @@
 """Benchmark of the sharded-retraining hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c3|c4|c5]
+                    [--dump-outputs DIR]
 
 --config c2 (default; BASELINE.json configs[1], the configuration the metric is quoted on): ml1m-shaped SISA,
     K=5 shards, retrain-after-delete with --delper 2 --deltype rand: route the 120 deleted users to their shards,
@@ -22,6 +23,10 @@
     ranks, column marginals reduced between the GPUs every iteration; float64 NumPy Sinkhorn timed beside it.
 --impl reference : the oracle port of the reference's CPU path (oracle/mf.py, oracle/evalm.py, oracle/ot.py --
     vectorised PyTorch-CPU / NumPy on all host threads) on the same config; rank 0 alone runs it.
+--dump-outputs DIR (--config c2, our arm): after the timed steps, what the last one returned to its caller (rank 0's
+    view) is written as DIR/<name>.npy -- user_mat (the merged user table), item_mat (the item table of every shard
+    on the rank), metrics (total RMSE / NDCG@10 / HR@10) and train_loss (every epoch of every retrained shard).  The inputs depend
+    on the arguments only, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -271,6 +276,9 @@ def run_c2_ours(args):
         ms = e0.elapsed_time(e1)
         if it >= args.warmup:
             step_ms.append(d.max_float(ms))
+    if args.dump_outputs and rank == 0:
+        # before anything reruns the batch: the kernel-alone repeats below retrain its tables in place
+        dump_outputs(args.dump_outputs, un)
     if os.environ.get("URE_BENCH_TIMELINE") and rank == 0:
         # CUPTI timeline of one more device-resident step on rank 0 (every rank runs the step: collectives)
         from torch.profiler import ProfilerActivity, profile
@@ -434,6 +442,19 @@ def run_c2_ours(args):
             raise SystemExit(f"bench self-check failed: GPU RMSE {gpu_rmse} vs CPU port {det['rmse']}")
     if rank == 0:
         print(json.dumps(line))
+
+
+def dump_outputs(out_dir, sisa):
+    """What Sisa.unlearn gave its caller, as float32 / float64 .npy files under `out_dir` (about 1.5 MB at N=1)."""
+    import torch
+    mine = [m for m in sisa.model_list if getattr(m, "item_mat", None) is not None]
+    arrays = {"user_mat": sisa.model_list[0].user_mat.weight.data,
+              "item_mat": torch.stack([m.item_mat.weight.data for m in mine]),
+              "metrics": np.array([sisa.final_log[k] for k in ("total_rmse", "total_ndcg", "total_hr")], dtype=np.float64),
+              "train_loss": np.asarray(sisa.log["train_loss"], dtype=np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy() if torch.is_tensor(a) else a)
 
 
 def ot_sharded_leg(d_, dev, n=2_000_000, k=8, dim=64, iters=100):
@@ -863,7 +884,13 @@ def main():
                     help="epochs per CPU sample of --impl reference (0 = all at N=1, epochs/N at N>1)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline / check legs")
     ap.add_argument("--no-extra", action="store_true", help="skip the epoch_eval_modes / c4_strong legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (--config c2, --impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config != "c2"):
+        ap.error("--dump-outputs is implemented for --impl ours --config c2")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_c2_reference(args) if args.config == "c2" else run_reference_other(args)

@@ -34,8 +34,10 @@ def test_struct_layouts_match_the_header():
 
 def test_sass_has_blackwell_tensor_and_bulk_copy_instructions():
     """tcgen05.mma -> UTC*MMA, tcgen05.ld -> LDTM, cp.async.bulk -> UBLKCP, red.v4.f32 -> REDG...F32x4."""
+    from ultrare_b200 import build
     so = os.path.join(ROOT, "ultrare_b200", "libultrare_b200.so")
-    sass = subprocess.run(["cuobjdump", "-sass", so], capture_output=True, text=True).stdout
+    cuobjdump = os.path.join(os.path.dirname(build.NVCC), "cuobjdump")      # the toolkit that built the library
+    sass = subprocess.run([cuobjdump, "-sass", so], capture_output=True, text=True).stdout
     assert re.search(r"UTC[A-Z]*MMA", sass), "no tcgen05 MMA in SASS"
     assert "LDTM" in sass and "UBLKCP" in sass
     assert re.search(r"RED[G]?\.E\.ADD\.F32x4", sass)

@@ -1,5 +1,5 @@
 import sys, os
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 from ultrare_b200 import kernels as kn, synth
 dev = torch.device("cuda:0")
