@@ -377,6 +377,44 @@ int64_t ure_user_segments_scratch_bytes(int64_t n, int n_user);
 int ure_user_segments(const ure_inter_t* d_inter, int64_t n, int n_user, int32_t* d_order, int64_t* d_seg,
                       void* d_scratch, void* stream);
 
+/* ---- Top-N recommendation over the whole catalogue (no counterpart in the reference, whose baseTest ranks each
+ * user's test items only).  score(u, i) = scale * sum_t P[u,t] * S[i,t] in fp32, S = sum_k Q_k, scale = 1/K. */
+
+/* Seen lists: d_off int64 [n_user + 1], d_items int32 [n]: the items of user u's records in ascending order at
+ * d_items[d_off[u] .. d_off[u+1]) (a stable radix sort by item, then by user; no host pass).  User and item ids must lie
+ * in [0, n_user) and [0, n_item); the library does not check them (that would need a synchronisation): the Python
+ * wrapper kernels.seen_lists does.  d_scratch: ure_seen_lists_scratch_bytes(n, n_user) bytes. */
+int64_t ure_seen_lists_scratch_bytes(int64_t n, int n_user);
+int ure_seen_lists(const ure_inter_t* d_inter, int64_t n, int n_user, int n_item, int64_t* d_off, int32_t* d_items,
+                   void* d_scratch, void* stream);
+
+/* d_S [n_item, d] = sum over k < n_models of d_Q[k] (a device array of table addresses), summed in k order.
+ * d a multiple of 4. */
+int ure_item_sum(const float* const* d_Q, int n_models, int64_t n_item, int d, float* d_S, void* stream);
+
+/* d_lo[j] = d_X[j] - trunc_tf32(d_X[j]) for j < n (n a multiple of 4): the lo operand of the 3-term tf32 split. */
+int ure_split_lo(const float* d_X, int64_t n, float* d_lo, void* stream);
+
+/* Per requested user d_users[r] (r < m; any order, duplicates allowed), the top_n items by score, descending, ties to
+ * the smaller item id, never an item of the user's seen list (d_seen_off / d_seen from ure_seen_lists, or both NULL:
+ * nothing excluded).  d_items int32 [m, top_n], d_scores fp32 [m, top_n]; a list with fewer eligible items than top_n
+ * is padded with item -1 and score -inf, as is the row of an id outside [0, n_user).  d_S_lo: ure_split_lo of d_S.
+ * tcgen05 kind::tf32 with the 3-term hi/lo split (fp32-accurate); the top-N is kept in the epilogue, the score matrix
+ * is never written.  d in {8,16,32,64,128}, 1 <= top_n <= 64 (else URE_EUNSUPPORTED), scale > 0.
+ * d_scratch: ure_topn_scratch_bytes(m, n_item, d, top_n) bytes (0: may be NULL). */
+int64_t ure_topn_scratch_bytes(int64_t m, int64_t n_item, int d, int top_n);
+int ure_topn(const float* d_P, int n_user, const float* d_S, const float* d_S_lo, int64_t n_item, int d,
+             const int32_t* d_users, int64_t m, const int64_t* d_seen_off, const int32_t* d_seen, int top_n, float scale,
+             int32_t* d_items, float* d_scores, void* d_scratch, void* stream);
+
+/* Full-catalogue metrics of top-N lists (d_items [m, top_n] for d_users [m]) against test records grouped by
+ * ure_user_segments (d_order may be NULL when the records are already grouped; d_seg int64 [n_user + 1]).  rel(u) =
+ * the user's distinct test items with rating >= 4/5 (method/utils.py:175,180); rows whose user has none are skipped.
+ * d_out fp64 [4] += (sum HR@N, sum Recall@N = hits/|rel|, sum NDCG@N, rows counted), with
+ * NDCG@N = sum_{p < N, hit} 1/log2(p+2) / sum_{p < min(N, |rel|)} 1/log2(p+2).  top_n <= 64 (else URE_EUNSUPPORTED). */
+int ure_topn_metrics(const int32_t* d_items, const int32_t* d_users, int64_t m, int top_n, const ure_inter_t* d_test,
+                     const int32_t* d_order, const int64_t* d_seg, int n_user, double* d_out, void* stream);
+
 /* Affected-shard routing (method/sisa.py:76-81): flags[owner[u]] = 1 for u in del. */
 int ure_route_deletions(const int32_t* d_owner, int32_t n_user, const int32_t* d_del, int32_t n_del,
                         int32_t* d_flags, int32_t n_shards, void* stream);

@@ -109,6 +109,13 @@ SIGNATURES = {
     "ure_host_stage_copy": (C.c_int, [_p, _p, _i64]),
     "ure_user_segments_scratch_bytes": (_i64, [_i64, C.c_int]),
     "ure_user_segments": (C.c_int, [_p, _i64, C.c_int, _p, _p, _p, _p]),
+    "ure_seen_lists_scratch_bytes": (_i64, [_i64, C.c_int]),
+    "ure_seen_lists": (C.c_int, [_p, _i64, C.c_int, C.c_int, _p, _p, _p, _p]),
+    "ure_item_sum": (C.c_int, [_p, C.c_int, _i64, C.c_int, _p, _p]),
+    "ure_split_lo": (C.c_int, [_p, _i64, _p, _p]),
+    "ure_topn_scratch_bytes": (_i64, [_i64, _i64, C.c_int, C.c_int]),
+    "ure_topn": (C.c_int, [_p, C.c_int, _p, _p, _i64, C.c_int, _p, _i64, _p, _p, C.c_int, _f32, _p, _p, _p, _p]),
+    "ure_topn_metrics": (C.c_int, [_p, _p, _i64, C.c_int, _p, _p, _p, C.c_int, _p, _p]),
     "ure_route_deletions": (C.c_int, [_p, _i32, _p, _i32, _p, _i32, _p]),
     "ure_merge_user_rows": (C.c_int, [_p, _p, _p, _p, _p, _i32, C.c_int, C.c_int, _p]),
     "ure_cost_matrix": (C.c_int, [_p, _i64, C.c_int, _p, C.c_int, C.c_int, _p, _p, _p]),

@@ -19,7 +19,7 @@ import numpy as np
 from .group import DATA_DIR, SAVE_DIR, Group
 from .method.scratch import Scratch
 from .method.sisa import Sisa
-from .method.utils import saveObject
+from .method.utils import recommend, saveObject, topn_metrics
 from .read import RatingData, loadData, readRating, readRatingDevice
 
 DATASETS = {
@@ -71,6 +71,8 @@ class InsParam(object):
 
 
 class Instance(object):
+    recommend_n = 0          # > 0: every pass also writes top-N recommendations and their metrics (main.py --recommend)
+
     def __init__(self, param):
         self.param = param
         prefix = '/test/' if self.param.del_type == 'test' else '/' + str(self.param.del_per) + '/' + self.param.del_type + '/'
@@ -126,7 +128,10 @@ class Instance(object):
         test_data = loadData(test[0], self.param.batch, self.param.n_worker, False)
         save_dir = self._save_dir(is_save, saving_name)
         model = Scratch(self.param, model_type)
-        model.train(train_data, test_data, [], verbose, save_dir)
+        trained = model.train(train_data, test_data, [], verbose, save_dir)
+        if self.recommend_n > 0:
+            self._save_recommendations(save_dir, *recommend([trained], None, self.recommend_n, exclude=train_data),
+                                       test_data)
         print('End of training', self.name, saving_name)
         print()
         return model
@@ -188,8 +193,25 @@ class Instance(object):
                     del_user.append(rating[0])
             model.unlearn(model_list, train_dlist, test_dlist, test_data, del_user, verbose, save_dir)
             self.timing['unlearn_s'] = time.time() - t0
+        if self.recommend_n > 0:
+            # seen items: this pass's training data (after the unlearn pass, deleted users' old items are gone)
+            self._save_recommendations(save_dir, *model.recommend(None, self.recommend_n, exclude=train_dlist), test_data)
         self.last_sisa = model
         return model.model_list
+
+    def _save_recommendations(self, save_dir, items, scores, test_data):
+        """rec{N}.npy (int32 [n_user, N] item ids), rec{N}_score.npy (fp32) and rec{N}_metrics.npy (fp64 [4]: HR@N,
+        Recall@N, NDCG@N over the whole catalogue, users counted) into the pass's save directory."""
+        from . import dist as udist
+        N = self.recommend_n
+        met = topn_metrics(items, None, test_data, N)
+        print(f'Top-{N} over the catalogue - HR: {met["hr"]:>.4f}, Recall: {met["recall"]:>.4f}, '
+              f'NDCG: {met["ndcg"]:>.4f} ({met["users"]} users)')
+        if len(save_dir) > 0 and udist.get().rank == 0:
+            np.save(f'{save_dir}/rec{N}', items.cpu().numpy())
+            np.save(f'{save_dir}/rec{N}_score', scores.cpu().numpy())
+            np.save(f'{save_dir}/rec{N}_metrics',
+                    np.array([met['hr'], met['recall'], met['ndcg'], met['users']], dtype=np.float64))
 
     # ---------------------------------------------------------------- calling functions
     def runFull(self, is_save=True, verbose=1):

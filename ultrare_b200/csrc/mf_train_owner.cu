@@ -1858,6 +1858,88 @@ extern "C" int ure_user_segments(const ure_inter_t* d_inter, int64_t n, int n_us
   return 0;
 }
 
+// ---------------------------------------------------------------- per-user seen lists (recommendation)
+// A user's training items in ascending order: the same stable radix sort, keyed first by item (the item side of the
+// set-up's passes, one (shard, side) row per launch) and then by user, so that the user passes keep the item order.
+namespace ure {
+namespace {
+__global__ void __launch_bounds__(kRadixThreads)
+radix_hist_row_kernel(const ure_mf_shard_t* shards, int pass, int npass, int* __restrict__ hist, int y) {
+  __shared__ int s_h[256];
+  radix_hist_body(shards, pass, npass, hist, nullptr, s_h, blockIdx.x, y, gridDim.x);
+}
+__global__ void __launch_bounds__(256)
+radix_scan_row_kernel(int* __restrict__ hist, int n_blocks, int y) {
+  __shared__ int s_tot[256];
+  radix_scan_body(hist, n_blocks, nullptr, s_tot, y);
+}
+__global__ void __launch_bounds__(kRadixThreads)
+radix_scatter_row_kernel(const ure_mf_shard_t* shards, int pass, int npass, const int* __restrict__ hist, int y) {
+  __shared__ int s_wh[kRadixWarps * 256];
+  radix_scatter_body(shards, pass, npass, hist, nullptr, s_wh, blockIdx.x, y, gridDim.x);
+}
+__global__ void seen_extract_kernel(const ure_inter_t* __restrict__ sorted, long long n, const int32_t* __restrict__ off_u,
+                                    int n_user, int32_t* __restrict__ items, long long* __restrict__ off) {
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  for (long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x; j < n; j += stride) items[j] = sorted[j].item;
+  for (long long u = (long long)blockIdx.x * blockDim.x + threadIdx.x; u <= n_user; u += stride) off[u] = off_u[u];
+}
+}  // namespace
+}  // namespace ure
+
+extern "C" int64_t ure_seen_lists_scratch_bytes(int64_t n, int n_user) {
+  using namespace ure;
+  return 512 + seg_align(((int64_t)n_user + 2) * 4) + 3 * seg_align(n * 16) + seg_align(2 * 256ll * kRadixBlocks * 4) + 256;
+}
+
+extern "C" int ure_seen_lists(const ure_inter_t* d_inter, int64_t n, int n_user, int n_item, int64_t* d_off,
+                              int32_t* d_items, void* d_scratch, void* stream) {
+  using namespace ure;
+  URE_REQUIRE(d_off && d_scratch && n >= 0 && n_user > 0 && n_item > 0 && n < (1ll << 31) && (n == 0 || (d_inter && d_items)),
+              URE_EINVAL, "ure_seen_lists: bad argument (n=%lld, n_user=%d, n_item=%d)", (long long)n, n_user, n_item);
+  auto st = static_cast<cudaStream_t>(stream);
+  char* base = static_cast<char*>(d_scratch);
+  auto* d_desc = reinterpret_cast<ure_mf_shard_t*>(base);   // [0]: item passes, [1]: user passes
+  auto* off_u = reinterpret_cast<int32_t*>(base + 512);
+  char* p = base + 512 + seg_align(((int64_t)n_user + 2) * 4);
+  auto* by_item = reinterpret_cast<ure_inter_t*>(p); p += seg_align(n * 16);
+  auto* tmp = reinterpret_cast<ure_inter_t*>(p); p += seg_align(n * 16);
+  auto* sorted = reinterpret_cast<ure_inter_t*>(p); p += seg_align(n * 16);
+  auto* hist = reinterpret_cast<int*>(p); p += seg_align(2 * 256ll * kRadixBlocks * 4);
+  int* bad = reinterpret_cast<int*>(p);
+  ure_mf_shard_t h[2];
+  memset(h, 0, sizeof(h));
+  h[0].inter = d_inter; h[0].inter_i = by_item; h[0].tmp_i = tmp; h[0].n = (int32_t)n; h[0].n_item = n_item;
+  h[1].inter = by_item; h[1].inter_u = sorted; h[1].tmp_u = tmp; h[1].off_u = off_u; h[1].n = (int32_t)n; h[1].n_user = n_user;
+  URE_CUDA(cudaMemcpyAsync(d_desc, h, sizeof(h), cudaMemcpyHostToDevice, st));
+  URE_CUDA(cudaMemsetAsync(off_u, 0, ((size_t)n_user + 2) * 4, st));
+  URE_CUDA(cudaMemsetAsync(bad, 0, 4, st));
+  long long blocks = (n + 1023) / 1024;
+  if (blocks > 2 * num_sms()) blocks = 2 * num_sms();
+  if (blocks < 1) blocks = 1;
+  if (n > 0) {
+    seg_count_kernel<<<(unsigned)blocks, 256, 0, st>>>(d_inter, n, n_user, off_u, bad);
+    int npass = 1;
+    while (npass < 4 && (n_item - 1) >> (8 * npass)) ++npass;
+    for (int pass = 0; pass < npass; ++pass) {          // row y = 1: shard 0, item side
+      radix_hist_row_kernel<<<kRadixBlocks, kRadixThreads, 0, st>>>(d_desc, pass, npass, hist, 1);
+      radix_scan_row_kernel<<<1, 256, 0, st>>>(hist, kRadixBlocks, 1);
+      radix_scatter_row_kernel<<<kRadixBlocks, kRadixThreads, 0, st>>>(d_desc, pass, npass, hist, 1);
+    }
+    npass = 1;
+    while (npass < 4 && (n_user - 1) >> (8 * npass)) ++npass;
+    for (int pass = 0; pass < npass; ++pass) {          // grid.y = 1: shard 0 of d_desc + 1, user side
+      radix_hist_kernel<<<dim3(kRadixBlocks, 1), kRadixThreads, 0, st>>>(d_desc + 1, pass, npass, hist, nullptr);
+      radix_scan_kernel<<<1, 256, 0, st>>>(hist, kRadixBlocks, nullptr);
+      radix_scatter_kernel<<<dim3(kRadixBlocks, 1), kRadixThreads, 0, st>>>(d_desc + 1, pass, npass, hist, nullptr);
+    }
+  }
+  csr_scan_kernel<<<1, 1024, 0, st>>>(d_desc + 1);
+  seen_extract_kernel<<<(unsigned)blocks, 256, 0, st>>>(sorted, n, off_u, n_user, d_items, reinterpret_cast<long long*>(d_off));
+  URE_CUDA(cudaGetLastError());
+  return 0;
+}
+
 extern "C" int64_t ure_mf_owner_radix_bytes(int n_shards) { return 2ll * n_shards * 256 * ure::kRadixBlocks * 4; }
 
 namespace ure {

@@ -1591,3 +1591,95 @@ def balance_labels(M, k, label, cnt, max_aug: int = 1 << 14):
         check(L.ure_balance_labels(_ptr(M), n, k, kp, _ptr(label), _ptr(cnt), int(max_aug), _ptr(ws), _stream()),
               "ure_balance_labels")
     return ws[128:140].view(torch.int32)
+
+
+# ------------------------------------------------------------------------------ top-N recommendation
+def _records_of(inters) -> torch.Tensor:
+    """One int32 [n, 4] record tensor from one or several (device-to-device copies, no kernel)."""
+    if isinstance(inters, torch.Tensor):
+        return inters.contiguous()
+    inters = [r for r in inters if r.shape[0] > 0] or list(inters[:1])
+    if len(inters) == 1:
+        return inters[0].contiguous()
+    out = torch.empty((sum(r.shape[0] for r in inters), 4), dtype=torch.int32, device=inters[0].device)
+    o = 0
+    for r in inters:
+        out[o:o + r.shape[0]].copy_(r, non_blocking=True)
+        o += r.shape[0]
+    return out
+
+
+def seen_lists(inter, n_user: int, n_item: int):
+    """(off int64 [n_user + 1], items int32 [n]): every user's training items in ascending order, built on the device by
+    ure_seen_lists (the owner set-up's stable radix sort, by item and then by user).  `inter`: an int32 [n, 4] record
+    tensor or a list of them (the shards' training sets); ids outside [0, n_user) / [0, n_item) raise ValueError."""
+    inter = _records_of(inter)
+    _need_cuda(inter)
+    n, dev = inter.shape[0], inter.device
+    if n > 0:           # the radix passes are sized by n_user / n_item: an id outside them would be mis-sorted silently
+        u, i = inter[:, 0], inter[:, 1]
+        if bool(((u < 0) | (u >= n_user) | (i < 0) | (i >= n_item)).any()):
+            raise ValueError(f"seen_lists: user ids must lie in [0, {n_user}) and item ids in [0, {n_item})")
+    L = _lib.lib()
+    off = torch.empty(n_user + 1, dtype=torch.int64, device=dev)
+    items = torch.empty(max(1, n), dtype=torch.int32, device=dev)
+    scratch = torch.empty(int(L.ure_seen_lists_scratch_bytes(n, n_user)), dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        check(L.ure_seen_lists(_ptr(inter), n, n_user, n_item, _ptr(off), _ptr(items), _ptr(scratch), _stream()),
+              "ure_seen_lists")
+    return off, items[:n]
+
+
+def item_sum(Q_list) -> torch.Tensor:
+    """S [n_item, d] = sum_k Q_k, summed in list order (ure_item_sum)."""
+    _need_cuda(*Q_list)
+    dev = Q_list[0].device
+    n_item, d = Q_list[0].shape
+    S = torch.empty((n_item, d), dtype=torch.float32, device=dev)
+    qs = [q.contiguous() for q in Q_list]
+    tab = pointer_table(qs, dev)
+    with torch.cuda.device(dev):
+        check(_lib.lib().ure_item_sum(_ptr(tab), len(qs), n_item, d, _ptr(S), _stream()), "ure_item_sum")
+    S._keep = (tab, qs)
+    return S
+
+
+def recommend_topn(P, S, users, top_n: int, scale: float, seen=None):
+    """(items int32 [m, top_n], scores fp32 [m, top_n]): for every id in `users` (int32 device tensor, any order,
+    duplicates allowed) the top_n items of scale * P[u].S[i] over the whole catalogue, score descending, ties to the
+    smaller item id, items of the user's seen list (``seen_lists``) excluded; short lists are padded with (-1, -inf).
+    One tcgen05 launch (plus a merge launch when the item range is split over CTAs), no synchronisation."""
+    _need_cuda(P, S, users)
+    dev = P.device
+    P, S = P.contiguous(), S.contiguous()
+    users = users.to(device=dev, dtype=torch.int32).contiguous()
+    n_user, d = P.shape
+    n_item, m = S.shape[0], users.shape[0]
+    L = _lib.lib()
+    S_lo = torch.empty_like(S)
+    items = torch.empty((m, top_n), dtype=torch.int32, device=dev)
+    scores = torch.empty((m, top_n), dtype=torch.float32, device=dev)
+    nb = int(L.ure_topn_scratch_bytes(m, n_item, d, top_n))
+    scratch = torch.empty(nb, dtype=torch.uint8, device=dev) if nb > 0 else None
+    off, seen_items = seen if seen is not None else (None, None)
+    with torch.cuda.device(dev):
+        check(L.ure_split_lo(_ptr(S), S.numel(), _ptr(S_lo), _stream()), "ure_split_lo")
+        check(L.ure_topn(_ptr(P), n_user, _ptr(S), _ptr(S_lo), n_item, d, _ptr(users), m, _ptr(off), _ptr(seen_items),
+                         int(top_n), float(scale), _ptr(items), _ptr(scores), _ptr(scratch), _stream()), "ure_topn")
+    return items, scores
+
+
+def topn_metrics(items, users, test_inter, n_user: int, seg=None, order=None) -> torch.Tensor:
+    """fp64 [4] = (sum HR@N, sum Recall@N, sum NDCG@N, rows counted) of top-N lists against test records
+    (ure_topn_metrics); the per-user test segments come from ``user_segments_device`` unless given."""
+    _need_cuda(items, users, test_inter)
+    dev = items.device
+    out = torch.zeros(4, dtype=torch.float64, device=dev)
+    if seg is None:
+        order, seg = user_segments_device(test_inter, n_user)
+    users = users.to(device=dev, dtype=torch.int32).contiguous()
+    with torch.cuda.device(dev):
+        check(_lib.lib().ure_topn_metrics(_ptr(items.contiguous()), _ptr(users), items.shape[0], items.shape[1],
+                                          _ptr(test_inter.contiguous()), _ptr(order), _ptr(seg), n_user, _ptr(out),
+                                          _stream()), "ure_topn_metrics")
+    return out

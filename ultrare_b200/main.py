@@ -1,5 +1,5 @@
 """Command line of the drop-in: the reference's flags with the reference's defaults and value checks
-(reference main.py:5-14 flags, :21-53 checks, :56-70 dispatch), plus two optional flags whose defaults keep the
+(reference main.py:5-14 flags, :21-53 checks, :56-70 dispatch), plus optional flags whose defaults keep the
 reference behaviour.  `python main.py --dataset ml1m --epoch 50 --group 5 --learn sisa --delper 2 --deltype rand`
 """
 import argparse
@@ -29,6 +29,8 @@ def _build_parser():
                    help='write a deterministic synthetic ML-1M-shaped data/ml1m/squ0_{train,test}.csv if absent')
     p.add_argument('--epoch-eval', default=None, choices=['faithful', 'final', 'none'],
                    help='per-epoch in-training evaluation fidelity of the SISA path')
+    p.add_argument('--recommend', type=int, default=0, metavar='N',
+                   help='also write every pass\'s top-N recommendations (rec{N}*.npy, seen items excluded); 0 = off')
     return p
 
 
@@ -41,6 +43,7 @@ def _checked(args):
         v = getattr(args, name)
         assert ok(v) if callable(ok) else v in ok, f'--{name} {v!r} is not accepted'
     assert all(isinstance(w, int) for w in args.layer)
+    assert 0 <= args.recommend <= 64, f'--recommend {args.recommend!r} is not accepted (0 .. 64)'
     return args
 
 
@@ -55,6 +58,7 @@ def main(argv=None):
         from . import synth
         synth.ensure_dataset(a.dataset)
     ins = Instance(InsParam(a.dataset, a.epoch, a.worker, a.layer, a.group, a.delper, a.deltype))
+    ins.recommend_n = a.recommend
     if a.group == 0:
         ins.runFull(is_save=True, verbose=a.verbose)
         return ins

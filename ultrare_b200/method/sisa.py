@@ -38,7 +38,7 @@ from torch import nn
 from .. import dist as udist
 from .. import kernels as kn
 from .scratch import Scratch
-from .utils import baseTest, base_test_device, base_test_values
+from .utils import _request_users, baseTest, base_test_device, base_test_values, recommend_from_tables
 
 
 class _Table:
@@ -168,6 +168,58 @@ class Sisa(Scratch):
             np.save(save_dir + '/log0', log)
         self.final_log = log
         return log
+
+    RECOMMEND_GATHER_BYTES = 256 << 20      # device memory of one chunk of gathered item tables (Sisa.recommend)
+
+    def _item_sum_in_shard_order(self):
+        """S = sum_k Q_k [n_item, d], summed in shard order k = 0 .. K-1 by ure_item_sum: the same bits at every world
+        size.  On several GPUs the ranks all-gather their item tables chunk by chunk of item rows (shard s lives on rank
+        s mod world) and every rank sums all K in order; an all-reduce of per-rank partial sums would associate the
+        additions by rank and change the last bits of S, and with them near-tied lists."""
+        K, world, rank = self.n_group, self.dist.world, self.dist.rank
+        if world == 1:
+            return kn.item_sum([self.model_list[s].item_mat.weight.data for s in range(K)])
+        slots = -(-K // world)
+        rows = max(1, min(self.n_item, self.RECOMMEND_GATHER_BYTES // (world * slots * self.k * 4)))
+        part = torch.zeros((slots, rows, self.k), dtype=torch.float32, device=self.device)
+        full = torch.empty((world * slots, rows, self.k), dtype=torch.float32, device=self.device)
+        S = torch.empty((self.n_item, self.k), dtype=torch.float32, device=self.device)
+        mine = list(range(rank, K, world))
+        for r0 in range(0, self.n_item, rows):
+            n = min(self.n_item, r0 + rows) - r0
+            for j, s in enumerate(mine):
+                part[j, :n].copy_(self.model_list[s].item_mat.weight.data[r0:r0 + n])
+            self.dist.all_gather_into(full, part)
+            S[r0:r0 + n].copy_(kn.item_sum([full[(s % world) * slots + s // world, :n] for s in range(K)]))
+        return S
+
+    def recommend(self, users=None, top_n=10, exclude=None):
+        """Top-N items per requested user from the ensemble of ``model_list`` (see utils.recommend): (items int32
+        [m, top_n], scores fp32 [m, top_n]) on the device, the same on every rank.  ``exclude``: the seen items to leave
+        out (records, dataset, DataLoader or a list of them, e.g. the shards' training loaders).
+
+        The item tables are summed in shard order whatever the number of GPUs (_item_sum_in_shard_order), so the
+        result is the same bit for bit on one GPU and on several.  With several GPUs each rank recommends for the
+        requested users whose owner shard it holds (users in no group: rank 0), because it holds those shards' training
+        records, and the rows, placed by request position into zero-filled outputs, are all-reduced (every row has one
+        non-zero contribution, so the sum is exact)."""
+        qsum = self._item_sum_in_shard_order()
+        P = self.model_list[0].user_mat.weight.data
+        u = _request_users(users, self.n_user, self.device)
+        if self.dist.world == 1:
+            return recommend_from_tables(P, qsum, self.n_group, u, top_n, exclude)
+        owner = self._owner[u.long()]
+        rank_of = torch.where(owner >= 0, owner % self.dist.world, torch.zeros_like(owner))
+        pos = torch.nonzero(rank_of == self.dist.rank).flatten()
+        items = torch.zeros((u.shape[0], top_n), dtype=torch.int32, device=self.device)
+        scores = torch.zeros((u.shape[0], top_n), dtype=torch.float32, device=self.device)
+        if pos.numel() > 0:
+            it, sc = recommend_from_tables(P, qsum, self.n_group, u[pos], top_n, exclude)
+            items[pos] = it
+            scores[pos] = sc
+        self.dist.all_reduce(items)
+        self.dist.all_reduce(scores)
+        return items, scores
 
     def _ensemble_test_sharded(self, test_dlist):
         """Multi-GPU evaluation with the TEST ROWS sharded: every rank scores the test sets of its own shards (the

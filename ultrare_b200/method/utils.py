@@ -191,6 +191,79 @@ def baseTest(dataloader, models, loss_fn, device, verbose, top_k=10):
     return rmse, ndcg, hr
 
 
+def _exclude_records(exclude, device):
+    """Training records whose items are excluded: None, an int32 [n, 4] records tensor, a dataset / DataLoader, or a
+    list of them; returns a records tensor, a list of them, or None."""
+    if exclude is None:
+        return None
+    if isinstance(exclude, torch.Tensor):
+        if exclude.dim() != 2 or exclude.shape[1] != 4 or exclude.dtype != torch.int32:
+            raise ValueError("exclude: a records tensor must be int32 [n, 4]")
+        return exclude.to(device)
+    if isinstance(exclude, (list, tuple)):
+        return [_exclude_records(e, device) for e in exclude]
+    ds = getattr(exclude, 'dataset', exclude)
+    return ds.records(device)
+
+
+def _request_users(users, n_user, device):
+    """The requested user ids as an int32 device tensor (all users when None); ids outside [0, n_user) raise."""
+    if users is None:
+        return torch.arange(n_user, dtype=torch.int32, device=device)
+    u = torch.as_tensor(users).to(device=device, dtype=torch.int32).reshape(-1)
+    if u.numel() > 0 and (int(u.min()) < 0 or int(u.max()) >= n_user):
+        raise ValueError(f"recommend: user ids must lie in [0, {n_user})")
+    return u
+
+
+def recommend_from_tables(P, S, n_models, users=None, top_n=10, exclude=None):
+    """(items int32 [m, top_n], scores fp32 [m, top_n]) of the ensemble mean (1/n_models) P[u].S[i], S the sum of the
+    models' item tables; see ``recommend``."""
+    dev = P.device
+    u = _request_users(users, P.shape[0], dev)
+    recs = _exclude_records(exclude, dev)
+    seen = kn.seen_lists(recs, P.shape[0], S.shape[0]) if recs is not None else None
+    return kn.recommend_topn(P, S, u, top_n, 1.0 / n_models, seen)
+
+
+def recommend(models, users=None, top_n=10, exclude=None):
+    """Top-N items per user over the whole catalogue: (items int32 [m, top_n], scores fp32 [m, top_n]) on the device.
+
+    score(u, i) = (1/K) sum_k P_k[u].Q_k[i] (the baseTest ensemble mean) for the K models, which must share one user
+    table (every SISA shard model does after the merge; a single model is a list of one).  Lists are sorted by score,
+    ties to the smaller item id, and padded with item -1 / score -inf when fewer than top_n items are eligible.
+    ``users``: ids in any order, duplicates allowed (None: every user).  ``exclude``: items a user has seen and must
+    not be shown -- None, an int32 [n, 4] records tensor, a dataset or DataLoader, or a list of them.
+    """
+    if not models:
+        raise ValueError("recommend: no models")
+    P = models[0].user_mat.weight.data
+    for m in models[1:]:
+        Pm = m.user_mat.weight.data
+        if Pm.data_ptr() != P.data_ptr() and (Pm.shape != P.shape or not torch.equal(Pm, P)):
+            raise ValueError("recommend: the models' user tables differ (only ensembles sharing one user table are "
+                             "supported)")
+    S = kn.item_sum([m.item_mat.weight.data for m in models])
+    return recommend_from_tables(P, S, len(models), users, top_n, exclude)
+
+
+def topn_metrics(items, users, test_data, top_n):
+    """Full-catalogue HR@N / Recall@N / NDCG@N of top-N lists (``recommend``'s items for ``users``; None = every user,
+    row u for user u) against ``test_data`` (dataset, DataLoader or records tensor): relevant items are a user's
+    distinct test items with normalised rating >= 4/5 (utils.py:175,180), users without one are not counted.
+    Returns dict(hr, recall, ndcg, users) with the three metrics averaged over the counted users."""
+    items = items[:, :top_n]
+    dev = items.device
+    inter = _exclude_records(test_data, dev)
+    inter = kn._records_of(inter) if isinstance(inter, list) else inter
+    u = torch.arange(items.shape[0], dtype=torch.int32, device=dev) if users is None else \
+        torch.as_tensor(users).to(device=dev, dtype=torch.int32).reshape(-1)
+    n_user = 1 + max(int(u.max()) if u.numel() else 0, int(inter[:, 0].max()) if inter.shape[0] else 0)
+    vals = kn.download_many([kn.topn_metrics(items, u, inter, n_user)])[0]
+    cnt = max(vals[3], 1.0)
+    return dict(hr=float(vals[0] / cnt), recall=float(vals[1] / cnt), ndcg=float(vals[2] / cnt), users=int(vals[3]))
+
+
 def computeNDCG(r, top_k):
     """reference utils.py:190-207 (host helper; the GPU path is ure_rank_metrics)."""
     r = np.asarray(r, dtype=np.float64)
