@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define URE_ABI_VERSION 6
+#define URE_ABI_VERSION 7
 #define URE_MAX_SHARDS 256        /* shard models batched in one launch           */
 #define URE_TOP_K 10              /* baseTest(top_k=10), method/utils.py:115      */
 
@@ -110,14 +110,6 @@ typedef struct {
                             * then trains nothing.  A caller may thus queue both launches with the capacities of an earlier
                             * plan of the same shapes instead of waiting for this plan's read-back (and skip the plan
                             * kernel: URE_BATCH_NO_PLAN), and repeats the pass with the exact plan when the code comes back */
-  uint32_t* owner_ready;   /* OWNER: NULL (the default), or DEVICE flags [#SMs][owner_sched_rows], zero on entry: the
-                            * CONCURRENT schedule pre-pass, an experiment that needs a library built with
-                            * -DURE_OWNER_REGS=96 (ure_mf_owner_concurrent_ok tells).  ure_mf_train then queues, on a side
-                            * stream of the library, a pre-pass that runs on the registers and shared memory the training
-                            * kernel leaves free, produces the rows in epoch order and raises flag [cta][row] for each;
-                            * the training kernel waits per row.  ure_mf_owner_schedule must not be called; the window
-                            * must cover the whole training (owner_sched_rows >= epochs).  Error code 3 in the workspace
-                            * (int32 at byte 16): a row did not arrive within ~2 s.  Measured: no gain (DESIGN.md).      */
 } ure_mf_hparams_t;
 
 /* RUNS schedule: per-shard state next to the ure_mf_shard_t entry, which still carries inter_u / inter_i of
@@ -201,22 +193,6 @@ int64_t ure_mf_owner_smem_bytes(int d, int cap_rows, int cap_slots, int cap_list
  * ure_mf_train may then run any steps [a, b) with step0 <= a whose epochs lie inside the window
  * (hparams.owner_sched_step0 = step0); a step outside it stops the shard and raises the workspace's error
  * word (int32 at byte 16). */
-/* Pipelined set-up: shards [shard0, shard0 + n_part) of the batch only (count, scan, radix passes; no plan kernel, no
- * inverse visiting orders: shards with explicit orders use ure_mf_owner_prepare) on a workspace the caller has cleared;
- * ure_mf_owner_cta_split gives the training CTAs per shard (h_c[n_shards], from the shard sizes h_n alone), and
- * ure_mf_owner_schedule_part runs the pre-pass for the CTAs [cta0, cta0 + cta_n) of shards that are set up -- so a
- * caller that uploads shard after shard overlaps set-up + pre-pass of one shard with the upload of the next
- * (capacities from a remembered plan, hparams.owner_plan set: no plan exists yet). */
-int ure_mf_owner_prepare_part(const ure_mf_shard_t* d_shards, int n_shards, int shard0, int n_part,
-                              const ure_mf_hparams_t* h_hp, int epochs, int max_rows, int32_t* d_radix_hist,
-                              void* d_workspace, void* stream);
-int ure_mf_owner_cta_split(const int32_t* h_n, int n_shards, int32_t* h_c);
-int ure_mf_owner_schedule_part(const ure_mf_shard_t* d_shards, int n_shards, const ure_mf_hparams_t* h_hp, int epochs,
-                               int64_t step0, int cta0, int cta_n, void* stream);
-
-/* 1 when a batch with these (planned) hparams can run the schedule pre-pass concurrently with the training kernel
- * (hparams.owner_ready): short epochs, d <= 32, one window for all epochs, both kernels' shared memory on one SM. */
-int ure_mf_owner_concurrent_ok(const ure_mf_hparams_t* h_hp, int epochs);
 int ure_mf_owner_schedule(const ure_mf_shard_t* d_shards, int n_shards, const ure_mf_hparams_t* h_hp,
                           int epochs, int64_t step0, void* stream);
 
@@ -244,7 +220,6 @@ typedef struct {            /* byte offsets into the arena (multiples of 256) an
   int64_t sse;              /* fp64 [K][max(1, epochs)] (zeroed by setup)                                          */
   int64_t zero_end;         /* end of the region setup clears                                                     */
   int64_t rec, off, radix, perm_inv, sched, sched_off;   /* owner schedule only                                   */
-  int64_t ready;            /* owner schedule: uint32 [grid][sched_rows] row flags (hparams.owner_ready), zeroed by setup */
   int64_t rows_total, n_total, sched_stride;
   int32_t spe_cap, max_rows, max_n, grid, owner, sched_rows;
 } ure_mf_batch_layout_t;
@@ -258,8 +233,6 @@ int ure_mf_batch_layout(const ure_mf_batch_shard_t* h_shards, int n_shards, int 
  * reused before the stream has passed this call), clears momentum / gradient scratch / losses / workspace / row
  * offsets, queues ure_mf_owner_prepare when lay->owner, and queues the copy of the plan (4 int32, see
  * ure_mf_owner_prepare) to h_stage + 176*K.  The weights (lay->W) are left to the caller. */
-#define URE_BATCH_NO_PREPARE 2    /* flags: do not queue ure_mf_owner_prepare either: the caller sets the shards up one by one
-                                   * (ure_mf_owner_prepare_part), each as soon as its records have arrived            */
 #define URE_BATCH_NO_PLAN 1       /* flags: do not compute / copy the plan (the launch runs on remembered capacities,
                                    * hparams.owner_plan set) */
 int ure_mf_batch_setup(const ure_mf_batch_shard_t* h_shards, int n_shards, int n_item, const ure_mf_hparams_t* h_hp,

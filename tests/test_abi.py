@@ -20,14 +20,14 @@ def test_header_symbols_are_exported_and_bound():
     for name in declared:
         assert hasattr(handle, name), f"{name} declared in the header but not exported"
     assert declared == set(_lib.SIGNATURES), declared ^ set(_lib.SIGNATURES)
-    assert handle.ure_abi_version() == 6
+    assert handle.ure_abi_version() == 7
     handle.ure_last_error.restype = ctypes.c_char_p
     assert isinstance(handle.ure_last_error(), bytes)
 
 
 def test_struct_layouts_match_the_header():
     from ultrare_b200 import _lib
-    assert ctypes.sizeof(_lib.MFShard) == 176 and ctypes.sizeof(_lib.MFHParams) == 144
+    assert ctypes.sizeof(_lib.MFShard) == 176 and ctypes.sizeof(_lib.MFHParams) == 136
     assert _lib.MFShard.inter_u.offset == 96 and _lib.MFShard.n.offset == 152 and _lib.MFShard.perm_seed.offset == 168
     assert _lib.MFHParams.mode.offset == 28 and _lib.MFHParams.decay.offset == 32 and _lib.MFHParams.owner_cap_rows.offset == 44
 

@@ -526,19 +526,6 @@ def test_optimistic_owner_launch_hit_and_miss(cuda_dev):
     assert kn._PLAN_HINTS[sig] == good
     assert torch.equal(p0, p2) and all(torch.equal(a, b) for a, b in zip(q0, q2))
     assert same_log(un2.final_log, un0.final_log)
-    # fresh loaders on page-locked arrays (an end-to-end pass): the records go up on a side stream and the shards are
-    # set up group by group as they arrive (kernels.PIPELINE_GROUPS) -- same tables bit for bit
-    pinned = [kn.pinned_copy(a) for a in trd]
-    groups_before = kn.PIPELINE_GROUPS
-    for groups_now in (2, 5):
-        kn.PIPELINE_GROUPS = groups_now
-        un3 = new()
-        out3 = un3.unlearn(models, mk(pinned, True), tdl, tdata, del_user, 0, '')
-        assert un3._last_batch.optimistic and un3._last_batch.pipelined
-        assert torch.equal(out3[0].user_mat.weight.data, p0)
-        assert all(torch.equal(m.item_mat.weight.data, b) for m, b in zip(out3, q0))
-        assert same_log(un3.final_log, un0.final_log)
-    kn.PIPELINE_GROUPS = groups_before
 
 
 @pytest.mark.gpu

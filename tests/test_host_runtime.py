@@ -43,8 +43,7 @@ def test_batch_layout_regions_are_aligned_disjoint_and_large_enough():
     assert lay.max_rows == max(I, max(nu for _, nu in ML1M_SHARDS)) and lay.max_n == max(n for n, _ in ML1M_SHARDS)
     assert lay.sched_stride == 2 * n_tot and 2 <= lay.sched_rows <= E + 1
     # every region starts on a 256-byte boundary, in this order, and holds what its consumer indexes
-    order = ["table", "W", "ws", "Z", "sse", "off", "ready", "zero_end", "rec", "radix", "perm_inv", "sched", "sched_off",
-             "total"]
+    order = ["table", "W", "ws", "Z", "sse", "off", "zero_end", "rec", "radix", "perm_inv", "sched", "sched_off", "total"]
     offs = [getattr(lay, nm) for nm in order]
     assert all(o % 256 == 0 for o in offs) and offs == sorted(offs) and offs[0] == 0
     size = {a: getattr(lay, b) - getattr(lay, a) for a, b in zip(order, order[1:])}
@@ -53,7 +52,6 @@ def test_batch_layout_regions_are_aligned_disjoint_and_large_enough():
     assert size["ws"] >= h.ure_mf_train_workspace_bytes()
     assert size["sse"] >= K * E * 8
     assert size["off"] >= sum(nu + I + 4 for _, nu in ML1M_SHARDS) * 4
-    assert size["ready"] >= lay.grid * lay.sched_rows * 4
     assert size["rec"] >= 4 * n_tot * 16                          # user-sorted, item-sorted, two radix scratch copies
     assert size["radix"] >= h.ure_mf_owner_radix_bytes(K)
     assert size["perm_inv"] == 0                                  # no explicit visiting orders
@@ -97,33 +95,6 @@ def test_batch_layout_rejects_bad_arguments_with_a_message():
     assert rc != 0                                                # more than URE_MAX_SHARDS
     rc, lay = _layout([(50, 5)] * L.URE_MAX_SHARDS)               # more shards than SMs: no owner schedule (one CTA each at least)
     assert rc == 0 and (lay.owner == 0 or lay.grid >= L.URE_MAX_SHARDS)
-
-
-def _cta_split_ref(ns, grid):
-    """make_plan's apportioning (csrc/mf_train_owner.cu): one CTA per shard, the spare ones by interaction count,
-    largest remainders first (the first shard wins a tie)."""
-    K, N = len(ns), max(1, sum(ns))
-    spare = grid - K
-    c = [1 + spare * n // N for n in ns]
-    rem = [spare * n % N for n in ns]
-    for _ in range(grid - sum(c)):
-        best = max(range(K), key=lambda s: (rem[s], -s))
-        c[best] += 1
-        rem[best] = -1
-    return c
-
-
-@pytest.mark.parametrize("ns", [[n for n, _ in ML1M_SHARDS], [1, 1, 1], [10, 0, 0, 990], [7] * 64, [123_456],
-                                [3, 1_000_000, 5, 17, 250_000, 1]])
-def test_cta_split_is_the_largest_remainder_apportioning(ns):
-    L, h = _lib()
-    _, lay = _layout([(max(n, 1), 8) for n in ns])
-    grid = lay.grid
-    n_arr, c_arr = (C.c_int32 * len(ns))(*ns), (C.c_int32 * len(ns))()
-    assert h.ure_mf_owner_cta_split(n_arr, len(ns), c_arr) == 0
-    got = list(c_arr)
-    assert sum(got) == grid and min(got) >= 1
-    assert got == _cta_split_ref(ns, grid)
 
 
 def _plan(lay, plan, d=16, allow_cache=1, force=(-1, 0)):

@@ -9,7 +9,7 @@ import ctypes as C
 import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("URE_LIB") or os.path.join(HERE, "libultrare_b200.so")   # URE_LIB: experiment builds (tools/)
+LIB_PATH = os.path.join(HERE, "libultrare_b200.so")
 
 URE_MAX_SHARDS = 256
 URE_TOP_K = 10
@@ -36,8 +36,7 @@ class MFHParams(C.Structure):
                 ("owner_spe_cap", _i32), ("owner_sched_rows", _i32), ("owner_sched", _p), ("owner_sched_off", _p),
                 ("owner_sched_step0", _i64), ("owner_sched_stride", _i64),
                 ("owner_cap_list", _i32), ("owner_max_n", _i32),
-                ("runs", _p), ("runs_rows", _i32), ("runs_spe_cap", _i32), ("runs_step0", _i64), ("owner_plan", _p),
-                ("owner_ready", _p)]
+                ("runs", _p), ("runs_rows", _i32), ("runs_spe_cap", _i32), ("runs_step0", _i64), ("owner_plan", _p)]
 
 
 class MFRuns(C.Structure):
@@ -59,14 +58,14 @@ class MFBatchShard(C.Structure):
 class MFBatchLayout(C.Structure):
     """ure_mf_batch_layout_t"""
     _fields_ = [(nm, _i64) for nm in ("total", "table", "ws", "W", "Z", "sse", "zero_end", "rec", "off", "radix",
-                                       "perm_inv", "sched", "sched_off", "ready", "rows_total", "n_total", "sched_stride")] + \
+                                       "perm_inv", "sched", "sched_off", "rows_total", "n_total", "sched_stride")] + \
                [(nm, _i32) for nm in ("spe_cap", "max_rows", "max_n", "grid", "owner", "sched_rows")]
 
 
 MF_DENSE, MF_LAZY, MF_OWNER, MF_RUNS = 0, 1, 2, 3
 
-assert C.sizeof(MFShard) == 176 and C.sizeof(MFHParams) == 144 and C.sizeof(MFRuns) == 64
-assert C.sizeof(MFBatchShard) == 32 and C.sizeof(MFBatchLayout) == 160
+assert C.sizeof(MFShard) == 176 and C.sizeof(MFHParams) == 136 and C.sizeof(MFRuns) == 64
+assert C.sizeof(MFBatchShard) == 32 and C.sizeof(MFBatchLayout) == 152
 
 # name -> (restype, argtypes); every symbol include/ultrare_b200.h declares
 SIGNATURES = {
@@ -78,10 +77,6 @@ SIGNATURES = {
     "ure_mf_owner_prepare": (C.c_int, [_p, C.c_int, C.POINTER(MFHParams), C.c_int, C.c_int, _p, _p, _p]),
     "ure_mf_owner_smem_bytes": (_i64, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
     "ure_mf_owner_schedule": (C.c_int, [_p, C.c_int, C.POINTER(MFHParams), C.c_int, _i64, _p]),
-    "ure_mf_owner_concurrent_ok": (C.c_int, [C.POINTER(MFHParams), C.c_int]),
-    "ure_mf_owner_prepare_part": (C.c_int, [_p, C.c_int, C.c_int, C.c_int, C.POINTER(MFHParams), C.c_int, C.c_int, _p, _p, _p]),
-    "ure_mf_owner_cta_split": (C.c_int, [C.POINTER(_i32), C.c_int, C.POINTER(_i32)]),
-    "ure_mf_owner_schedule_part": (C.c_int, [_p, C.c_int, C.POINTER(MFHParams), C.c_int, _i64, C.c_int, C.c_int, _p]),
     "ure_mf_batch_layout": (C.c_int, [C.POINTER(MFBatchShard), C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _i64,
                                        C.POINTER(MFBatchLayout)]),
     "ure_mf_batch_setup": (C.c_int, [C.POINTER(MFBatchShard), C.c_int, C.c_int, C.POINTER(MFHParams), C.c_int, C.c_uint32,
@@ -155,7 +150,7 @@ def lib() -> C.CDLL:
     for name, (res, args) in SIGNATURES.items():
         fn = getattr(handle, name)           # AttributeError if the .so lacks a declared symbol
         fn.restype, fn.argtypes = res, args
-    if handle.ure_abi_version() != 6:
+    if handle.ure_abi_version() != 7:
         raise RuntimeError("ultrare_b200: ABI version mismatch; rebuild the shared library")
     _lib = handle
     return handle

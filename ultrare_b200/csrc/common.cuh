@@ -28,7 +28,6 @@ int mf_train_runs(const ure_mf_shard_t* d_shards, int n_shards, const ure_mf_hpa
 int mf_train_owner(const ure_mf_shard_t* d_shards, int n_shards, const ure_mf_hparams_t* hp, int epochs,
                    long long step_begin, long long step_end, void* d_workspace, cudaStream_t st);
 int64_t mf_owner_workspace_bytes();
-void mf_owner_debug(unsigned flags);
 int mf_owner_trace(void* d_workspace, long long* d_trace, int steps, cudaStream_t st);
 
 #define URE_CUDA(call)                                      \

@@ -6,7 +6,6 @@
 // the descriptor table, the training workspace), writes the descriptor table, clears what must be zero and queues
 // the owner set-up kernels; a second call turns the plan those kernels leave into the launch parameters.  The host
 // does no per-shard tensor bookkeeping before the training kernel is queued (round 1: ~0.5 ms of Python per step).
-#include <stdlib.h>
 #include <string.h>
 
 #include "common.cuh"
@@ -19,7 +18,7 @@ int mf_owner_prepare_impl(const ure_mf_shard_t* d_shards, int n_shards, const ur
                           int max_rows, int32_t* d_radix_hist, void* d_workspace, void* stream, int flags);
 }
 
-static_assert(sizeof(ure_mf_batch_shard_t) == 32 && sizeof(ure_mf_batch_layout_t) == 160, "ctypes mirrors in _lib.py");
+static_assert(sizeof(ure_mf_batch_shard_t) == 32 && sizeof(ure_mf_batch_layout_t) == 152, "ctypes mirrors in _lib.py");
 
 namespace ure {
 namespace {
@@ -67,7 +66,6 @@ extern "C" int ure_mf_batch_layout(const ure_mf_batch_shard_t* h_shards, int n_s
     n_rows = sched_bytes_cap / row_bytes;
     if (n_rows < 2) n_rows = 2;
     if (n_rows > epochs + 1) n_rows = epochs + 1;
-    out->ready = o; o = align_up(o + (int64_t)grid * n_rows * 4);       // row flags of the concurrent pre-pass
   }
   out->zero_end = o;
   out->rows_total = rows;
@@ -131,7 +129,7 @@ extern "C" int ure_mf_batch_setup(const ure_mf_batch_shard_t* h_shards, int n_sh
   }
   URE_CUDA(cudaMemcpyAsync(base + lay->table, tab, (size_t)n_shards * sizeof(ure_mf_shard_t), cudaMemcpyHostToDevice, st));
   URE_CUDA(cudaMemsetAsync(base + lay->ws, 0, (size_t)(lay->zero_end - lay->ws), st));
-  if (lay->owner && !(flags & URE_BATCH_NO_PREPARE)) {
+  if (lay->owner) {
     bool any_perm = false;
     for (int s = 0; s < n_shards; ++s) any_perm |= h_shards[s].perm != nullptr;
     const bool no_plan = (flags & URE_BATCH_NO_PLAN) != 0;
@@ -197,10 +195,7 @@ extern "C" int ure_mf_batch_plan(const int32_t* h_plan, int n_shards, ure_mf_hpa
   hp->owner_sched = reinterpret_cast<uint16_t*>(base + lay->sched);
   hp->owner_sched_off = reinterpret_cast<int32_t*>(base + lay->sched_off);
   hp->owner_sched_rows = lay->sched_rows; hp->owner_sched_stride = lay->sched_stride; hp->owner_sched_step0 = 0;
-  {
-    static const int fast = getenv("URE_SCHED_FAST") ? atoi(getenv("URE_SCHED_FAST")) : 1;      // 0: general pre-pass (A/B)
-    hp->owner_max_n = fast ? lay->max_n : 0;
-  }
+  hp->owner_max_n = lay->max_n;
   // the offsets table was laid out for the host-side steps-per-epoch bound; the plan's is the same number
   URE_REQUIRE(spe_cap <= lay->spe_cap, URE_EINVAL, "ure_mf_batch_plan: plan steps per epoch %d above the layout's %d",
               spe_cap, lay->spe_cap);

@@ -496,7 +496,6 @@ extern "C" int ure_mf_debug_flags(void* d_workspace, unsigned flags, void* strea
   URE_REQUIRE(d_workspace, URE_EINVAL, "ure_mf_debug_flags: null workspace");
   auto* ws = static_cast<Workspace*>(d_workspace);
   g_force_warps_g0 = (int)((flags >> 8) & 63u) ? (int)((flags >> 8) & 63u) : -1;
-  mf_owner_debug(flags);
   URE_CUDA(cudaMemcpyAsync(&ws->debug_flags, &flags, sizeof(flags), cudaMemcpyHostToDevice,
                            static_cast<cudaStream_t>(stream)));
   URE_CUDA(cudaStreamSynchronize(static_cast<cudaStream_t>(stream)));

@@ -783,53 +783,39 @@ owner_schedule_kernel(const ure_mf_shard_t* __restrict__ shards, int K, ure_mf_h
 //   * the (L, R) halves of a slot's record index -- what every epoch's inverse network starts from -- are split once
 //     per launch and kept as one packed word per slot, in doubled units so that a half IS the byte offset into a
 //     16-bit round table;
-//   * NT of the four rounds of the inverse network read a per-epoch table (one LDS of random lanes: ~3.5 bank
-//     wavefronts), the others evaluate the round function (6 ALU instructions): the mix keeps the shared-memory
-//     pipe and the issue slots equally busy;
+//   * the four rounds of the inverse network read a per-epoch table (one LDS of random lanes: ~3.5 bank wavefronts);
 //   * cycle walking (x >= n, one slot in ~400) is a rare divergent loop instead of a second trip of the whole group;
 //   * step and rank of a slot share one 16-bit word; the per-(step, warp) counts are scanned by the whole CTA.
 // Lists are identical to the general kernel's (same stable order), so either serves the training kernel.
-__host__ __device__ inline long long schedule_tab_smem_bytes(int cap_slots, int tab_cap, int n_tab) {
+__host__ __device__ inline long long schedule_tab_smem_bytes(int cap_slots, int tab_cap) {
   // packed halves / record index [cap] u32 | step + rank [cap] u16 | counters [warps][64] int | scan scratch |
-  // round tables 2 sets x n_tab x [tab_cap] u16
-  return 4ll * cap_slots + 2ll * cap_slots + 4ll * kSchedWarps * 64 + 4ll * (kSchedWarps + 4) + 2ll * 2 * n_tab * tab_cap + 64;
+  // round tables 2 sets x 4 x [tab_cap] u16
+  return 4ll * cap_slots + 2ll * cap_slots + 4ll * kSchedWarps * 64 + 4ll * (kSchedWarps + 4) + 2ll * 2 * 4 * tab_cap + 64;
 }
 
-// CO (concurrent mode, hp.owner_ready): ONE 256-thread CTA per training CTA, launched next to the training kernel on
-// the registers and shared memory it leaves free (56 x 256 registers, ~40 KB); the rows are produced in epoch order
-// and published one by one (ready[cta * rows + row] = 1, release); the packed halves live in the radix scratch of
-// the set-up (tmp_u / tmp_i, free by now) instead of shared memory.
-template <int NT, int NTHR, bool CO>
-__global__ void __maxnreg__(CO ? 56 : 64)
+__global__ void __maxnreg__(64)
 owner_schedule_tab_kernel(const ure_mf_shard_t* __restrict__ shards, int K, ure_mf_hparams_t hp, int epochs,
-                          long long step0, int tab_cap, int sb, int cta0, int n_cta) {
-  const int cta = cta0 + (int)blockIdx.x;  // the training CTA this block serves (a launch may cover a sub-range)
-  constexpr int kSchedThreads = NTHR;      // (shadows the namespace constant: every loop below strides by the CTA size)
-  constexpr int NW = NTHR / 32;
+                          long long step0, int tab_cap, int sb) {
+  constexpr int NW = kSchedWarps;
   constexpr unsigned FULL = 0xffffffffu;
   constexpr int NI = 4;
   extern __shared__ __align__(16) unsigned char dyn[];
   __shared__ PlanScratch s_ps;
   __shared__ Plan s_pl;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  make_plan(shards, K, cta, n_cta, s_pl, s_ps);
+  make_plan(shards, K, blockIdx.x, gridDim.x, s_pl, s_ps);
   const ure_mf_shard_t& sh = shards[s_pl.shard];
   const int mU = s_pl.mU, m = mU + s_pl.mI;
   const int B = hp.batch, n = sh.n;
   const int spe = (n + B - 1) / B;
-  if (plan_not_covered(hp, s_pl, spe)) {
-    if (CO)                                // the training CTA of this index is (or will be) waiting: tell it to give up
-      for (int r = tid; r < hp.owner_sched_rows; r += kSchedThreads)
-        asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(hp.owner_ready + (long long)cta * hp.owner_sched_rows + r),
-                     "r"(2u) : "memory");
-    return;
-  }
+  if (plan_not_covered(hp, s_pl, spe)) return;
   if (spe == 0) return;
   const int cap = hp.owner_cap_slots, spe_cap = hp.owner_spe_cap;
-  unsigned short* const s_sr = reinterpret_cast<unsigned short*>(reinterpret_cast<uint32_t*>(dyn) + (CO ? 0 : cap));   // [cap] step | rank << sb
+  uint32_t* const s_lr = reinterpret_cast<uint32_t*>(dyn);                       // [cap] packed halves / record index
+  unsigned short* const s_sr = reinterpret_cast<unsigned short*>(s_lr + cap);    // [cap] step | rank << sb
   int* const s_wh = reinterpret_cast<int*>(s_sr + cap);                          // [NW][64]
   int* const s_wtot = s_wh + NW * 64;                                            // [NW + 4]
-  unsigned char* const s_tab = reinterpret_cast<unsigned char*>(s_wtot + NW + 4);   // NT x [tab_cap] u16
+  unsigned char* const s_tab = reinterpret_cast<unsigned char*>(s_wtot + NW + 4);   // 2 sets x 4 x [tab_cap] u16
   const uint32_t tab_bytes = 2u * (uint32_t)tab_cap;
   const int4* const recU = reinterpret_cast<const int4*>(sh.inter_u + s_pl.su0);
   const int4* const recI = reinterpret_cast<const int4*>(sh.inter_i + s_pl.si0) - mU;
@@ -837,16 +823,11 @@ owner_schedule_tab_kernel(const ure_mf_shard_t* __restrict__ shards, int K, ure_
   dom.init((uint32_t)n);
   const bool explicit_order = sh.perm_inv != nullptr;
   const bool trivial = n <= 1;
-  // packed halves of every slot: shared memory, or (CO) the set-up's radix scratch -- 16 bytes per record and side,
-  // 4 needed; slot sl of the user side at tmp_u[su0 ..], of the item side at tmp_i[si0 ..]
-  uint32_t* const lrU = CO ? reinterpret_cast<uint32_t*>(sh.tmp_u) + s_pl.su0 : reinterpret_cast<uint32_t*>(dyn);
-  uint32_t* const lrI = CO ? reinterpret_cast<uint32_t*>(sh.tmp_i) + s_pl.si0 - mU : lrU;
-  auto lr_at = [&](int sl) -> uint32_t& { return (sl >= mU ? lrI : lrU)[sl]; };
   for (int sl = tid; sl < m; sl += kSchedThreads) {
     const uint32_t j = (uint32_t)__ldg(&((sl >= mU ? recI : recU) + sl)->w);
     uint32_t L, R;
     dom.split(j, L, R);
-    lr_at(sl) = explicit_order || trivial ? j : (L << 17) | (R << 1);
+    s_lr[sl] = explicit_order || trivial ? j : (L << 17) | (R << 1);
   }
   const uint32_t B2 = 2u * (uint32_t)B;
   const uint32_t magic2 = (uint32_t)(0x100000000ull / B2);                       // floor(2^32 / 2B): quotient low by <= 1
@@ -856,21 +837,18 @@ owner_schedule_tab_kernel(const ure_mf_shard_t* __restrict__ shards, int K, ure_
   const unsigned lt = (1u << lane) - 1u;
   const uint32_t qmask = (1u << sb) - 1u;
 
-  // round tables of one epoch (rounds 3, 2 when NT >= 2; 1, 0 when NT == 4), doubled values, built by threads
-  // t0, t0 + nthr, ... of the CTA
+  // round tables of one epoch (rounds 3, 2, 1, 0), doubled values, built by threads t0, t0 + nthr, ... of the CTA
   auto build_tables = [&](int epoch, unsigned char* tab, int t0, int nthr) {
-    if (explicit_order || trivial || NT == 0 || t0 < 0) return;
+    if (explicit_order || trivial || t0 < 0) return;
     FeistelKeys kt;
     kt.init(perm_key(sh.perm_seed, (uint32_t)sh.shard_id, (uint32_t)epoch));
     for (int x = t0; x < (int)dom.a; x += nthr) {
       *reinterpret_cast<unsigned short*>(tab + 2 * x) = (unsigned short)(2u * mulhi32(round_hash((uint32_t)x ^ kt.rk[3]), dom.b));
-      if (NT >= 4)
-        *reinterpret_cast<unsigned short*>(tab + 2 * tab_bytes + 2 * x) = (unsigned short)(2u * mulhi32(round_hash((uint32_t)x ^ kt.rk[1]), dom.b));
+      *reinterpret_cast<unsigned short*>(tab + 2 * tab_bytes + 2 * x) = (unsigned short)(2u * mulhi32(round_hash((uint32_t)x ^ kt.rk[1]), dom.b));
     }
     for (int x = t0; x < (int)dom.b; x += nthr) {
       *reinterpret_cast<unsigned short*>(tab + tab_bytes + 2 * x) = (unsigned short)(2u * mulhi32(round_hash((uint32_t)x ^ kt.rk[2]), dom.a));
-      if (NT >= 4)
-        *reinterpret_cast<unsigned short*>(tab + 3 * tab_bytes + 2 * x) = (unsigned short)(2u * mulhi32(round_hash((uint32_t)x ^ kt.rk[0]), dom.a));
+      *reinterpret_cast<unsigned short*>(tab + 3 * tab_bytes + 2 * x) = (unsigned short)(2u * mulhi32(round_hash((uint32_t)x ^ kt.rk[0]), dom.a));
     }
   };
   const int e_first = (int)(step0 / spe);
@@ -883,27 +861,18 @@ owner_schedule_tab_kernel(const ure_mf_shard_t* __restrict__ shards, int K, ure_
     const int epoch = e_first + r;
     if (epoch >= epochs) break;
     unsigned short* const out = hp.owner_sched + (long long)r * hp.owner_sched_stride + s_pl.slot_base;
-    int* const off = hp.owner_sched_off + ((long long)r * n_cta + cta) * (spe_cap + 1);
-    FeistelKeys ks;
-    ks.init(perm_key(sh.perm_seed, (uint32_t)sh.shard_id, (uint32_t)epoch));
+    int* const off = hp.owner_sched_off + ((long long)r * gridDim.x + blockIdx.x) * (spe_cap + 1);
     const int32_t* const pinv = explicit_order ? sh.perm_inv + (long long)epoch * n : nullptr;
-    const unsigned char* const tabs = s_tab + (it & 1) * NT * tab_bytes;        // tables alternate between two sets
+    const unsigned char* const tabs = s_tab + (it & 1) * 4 * tab_bytes;         // tables alternate between two sets
     // one round of the inverse network in doubled units: h -= 2 f(o) (mod m2)
     auto round_tab = [&](uint32_t& h, uint32_t o2, uint32_t t, uint32_t m2) {
       const uint32_t f = *reinterpret_cast<const unsigned short*>(tabs + t * tab_bytes + o2);
       const uint32_t d = h - f;
       h = min(d, d + m2);                  // unsigned: the wrapped difference is the larger one
     };
-    auto round_alu = [&](uint32_t& h, uint32_t o2, uint32_t key, uint32_t mod, uint32_t m2) {
-      const uint32_t f = mulhi32(round_hash((o2 >> 1) ^ key), mod);
-      const uint32_t d = h - 2u * f;
-      h = min(d, d + m2);
-    };
     auto inverse2 = [&](uint32_t Ls, uint32_t Rs) {       // -> 2 x position
-      if (NT >= 2) { round_tab(Rs, Ls, 0, b2); round_tab(Ls, Rs, 1, a2); }
-      else { round_alu(Rs, Ls, ks.rk[3], dom.b, b2); round_alu(Ls, Rs, ks.rk[2], dom.a, a2); }
-      if (NT >= 4) { round_tab(Rs, Ls, 2, b2); round_tab(Ls, Rs, 3, a2); }
-      else { round_alu(Rs, Ls, ks.rk[1], dom.b, b2); round_alu(Ls, Rs, ks.rk[0], dom.a, a2); }
+      round_tab(Rs, Ls, 0, b2); round_tab(Ls, Rs, 1, a2);
+      round_tab(Rs, Ls, 2, b2); round_tab(Ls, Rs, 3, a2);
       return (Ls >> 1) * b2 + Rs;
     };
     // ---- pass 1: step of every slot; rank among the warp's slots of the same step, in slot order.  No CTA barrier
@@ -915,7 +884,7 @@ owner_schedule_tab_kernel(const ure_mf_shard_t* __restrict__ shards, int K, ure_
       for (int u = 0; u < NI; ++u) {
         const int sl = base + 32 * u + lane;
         live[u] = sl < w1;
-        x2[u] = live[u] ? lr_at(sl) : 0u;
+        x2[u] = live[u] ? s_lr[sl] : 0u;
       }
       if (explicit_order) {
 #pragma unroll
@@ -983,7 +952,7 @@ owner_schedule_tab_kernel(const ure_mf_shard_t* __restrict__ shards, int K, ure_
     } else {
       const int rn = r + gridDim.y;
       if (rn < hp.owner_sched_rows && e_first + rn < epochs)
-        build_tables(e_first + rn, s_tab + ((it + 1) & 1) * NT * tab_bytes, tid - 32, kSchedThreads - 32);
+        build_tables(e_first + rn, s_tab + ((it + 1) & 1) * 4 * tab_bytes, tid - 32, kSchedThreads - 32);
     }
     __syncthreads();
     // ---- pass 2: position = start of (step, warp) + rank; then the warp clears its counters for the next row
@@ -995,13 +964,6 @@ owner_schedule_tab_kernel(const ure_mf_shard_t* __restrict__ shards, int K, ure_
     s_wh[warp * 64 + lane] = 0;
     s_wh[warp * 64 + 32 + lane] = 0;
     __syncwarp();
-    if (CO) {                              // the row is complete: tell the training CTA of the same index
-      __threadfence();
-      __syncthreads();
-      if (tid == 0)
-        asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(hp.owner_ready + (long long)cta * hp.owner_sched_rows + r),
-                     "r"(1u) : "memory");
-    }
   }
 }
 
@@ -1010,37 +972,18 @@ owner_schedule_tab_kernel(const ure_mf_shard_t* __restrict__ shards, int K, ure_
 // 32-bit shared-memory indexing, packed cache records and compile-time CACHED keep its instruction count down.
 // LONGLIST: the launch's owner_cap_list is below owner_cap_slots, so a batch list may have to be read from the
 // schedule table in global memory (generic loads); false keeps every list access a shared-memory load.
-// -DURE_OWNER_REGS=96: narrow rows (d <= 32) compiled for 96 registers (no spills, 6.85 vs 6.79 us per step with the 122
-// the compiler takes when left alone): 512 x 96 leaves a quarter of the SM's register file to the concurrent schedule
-// pre-pass experiment (owner_schedule_tab_kernel<.., 256, true>).
 template <int D, bool CACHED, bool LONGLIST>
-#ifndef URE_OWNER_REGS
-#define URE_OWNER_REGS 0                  // 96: the build the concurrent pre-pass experiment needs (tools/build_variant.sh)
-#endif
-#if URE_OWNER_REGS
-__global__ void __maxnreg__(D <= 32 ? URE_OWNER_REGS : 128)
-#else
 __global__ void __launch_bounds__(kOwnThreads, 1)
-#endif
 mf_owner_kernel(const ure_mf_shard_t* __restrict__ shards, int K, ure_mf_hparams_t hp, int epochs,
-                long long step_begin, long long step_end, OwnerWs* ws, unsigned dbg) {
+                long long step_begin, long long step_end, OwnerWs* ws) {
   constexpr int CH = D / 4;                // float4 chunks of a row
   // lanes per interaction and chunks per lane: one chunk per lane up to d=32; wide rows give every lane V=4 chunks
   // (chunk gl + v*G: a load instruction of the group still covers G*16 contiguous bytes), which divides the
   // shuffle reductions and the per-interaction bookkeeping (the loop is issue-bound) by four.
-#ifndef URE_OWNER_V16
-#define URE_OWNER_V16 1
-#endif
-#ifndef URE_OWNER_PREFETCH
-#define URE_OWNER_PREFETCH 0
-#endif
-#ifndef URE_OWNER_QB16
-#define URE_OWNER_QB16 4
-#endif
-  constexpr int V = D >= 64 ? 4 : D == 16 ? URE_OWNER_V16 : 1;
+  constexpr int V = D >= 64 ? 4 : 1;
   constexpr int G = CH / V;                // lanes per interaction
   constexpr int GPW = 32 / G;              // lane groups per warp
-  constexpr int QB = V == 4 ? 2 : D == 16 ? URE_OWNER_QB16 : 4;   // interactions a group handles per wave (QB*V gathers in flight per lane)
+  constexpr int QB = V == 4 ? 2 : 4;       // interactions a group handles per wave (QB*V gathers in flight per lane)
   constexpr int WAVE = GPW * QB;           // interactions per warp and wave
   constexpr int NW = kOwnWarps;
   constexpr int RS = 2 * D;                // row stride in floats: [w | momentum, pre-scaled: mu*buf + wd*w]
@@ -1051,12 +994,11 @@ mf_owner_kernel(const ure_mf_shard_t* __restrict__ shards, int K, ure_mf_hparams
   __shared__ ure_mf_shard_t s_sh;
   __shared__ float s_wsse[NW];
   __shared__ int s_total;                  // entries of the batch list in s_list
-  __shared__ int s_abort;
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, gl = lane % G, gw = lane / G;
   if (hp.owner_plan && ld_acquire_u32(reinterpret_cast<const unsigned*>(&ws->error)) == 2u) return;   // uniform over the grid: the pre-pass found the remembered capacities too small
   make_plan(shards, K, blockIdx.x, gridDim.x, s_pl, s_ps);
-  if (tid == 0) { s_sh = shards[s_pl.shard]; s_abort = 0; }
+  if (tid == 0) s_sh = shards[s_pl.shard];
   __syncthreads();
   const ure_mf_shard_t& sh = s_sh;
   const int ru0 = s_pl.ru0, ri0 = s_pl.ri0, mU = s_pl.mU;
@@ -1095,27 +1037,11 @@ mf_owner_kernel(const ure_mf_shard_t* __restrict__ shards, int K, ure_mf_hparams
   const int* const sched_off = hp.owner_sched_off + (long long)blockIdx.x * (hp.owner_spe_cap + 1);
   const long long off_row = (long long)gridDim.x * (hp.owner_spe_cap + 1);
   // where the batch list of (epoch ep, step kk) lives: false = outside the scheduled window
-  // concurrent pre-pass (hp.owner_ready): row r of THIS CTA's lists is complete once ready[blockIdx.x * rows + r] is
-  // non-zero (written with release semantics by the pre-pass CTA of the same index, which runs on this SM's spare
-  // registers while the kernel trains).  A row that does not arrive within ~2 s raises error 3 for the whole grid.
-  int ready_rows = hp.owner_ready ? 0 : 0x7fffffff;            // rows known to be complete
   auto find_list = [&](int ep, int kk, const unsigned short*& src, int& len) {
     const int row = ep - sched_e0;
     src = sched;
     len = 0;
     if (row < 0 || row >= hp.owner_sched_rows) return false;
-    if (row >= ready_rows) {
-      const unsigned* const flag = reinterpret_cast<const unsigned*>(hp.owner_ready) +
-                                   (long long)blockIdx.x * hp.owner_sched_rows + row;
-      long long spins = 0;
-      unsigned v;
-      while ((v = ld_acquire_u32(flag)) == 0u) {
-        if (++spins > (1ll << 22)) { atomicMax(&ws->error, 3); v = 2u; break; }
-        __nanosleep(64);
-      }
-      if (v != 1u) return false;           // timed out, or the pre-pass found the remembered capacities too small
-      ready_rows = row + 1;
-    }
     const int* o = sched_off + row * off_row + kk;
     const int a = __ldcg(o), b = __ldcg(o + 1);
     src = sched + row * hp.owner_sched_stride + a;
@@ -1193,7 +1119,6 @@ mf_owner_kernel(const ure_mf_shard_t* __restrict__ shards, int K, ure_mf_hparams
       if (tid == 0) atomicMax(&ws->error, 1);
       break;
     }
-    if (hp.owner_ready && ld_acquire_u32(reinterpret_cast<const unsigned*>(&ws->error)) >= 2u) break;
     const bool rd = (t - step_begin) & 1;
     const float* const Pr = rd ? sh.gP : sh.P;
     const float* const Qr = rd ? sh.gQ : sh.Q;
@@ -1265,20 +1190,6 @@ mf_owner_kernel(const ure_mf_shard_t* __restrict__ shards, int K, ure_mf_hparams
 #pragma unroll
         for (int v = 0; v < V; ++v) o4[q][v] = __ldca(reinterpret_cast<const float4*>(src + 4 * v * G));
       }
-#if URE_OWNER_PREFETCH
-      // experiment (tools/build_variant.sh -DURE_OWNER_PREFETCH=1|2): the NEXT wave's gathered rows on their way into
-      // L1 while this wave computes, no registers held.  Measured SLOWER (7.3-7.5 vs 6.9 us per step): the loop is bound
-      // by its dependent instruction stream, not by the L2 latency of the gathers.
-      if (wv + 1 < wv1) {
-#pragma unroll
-        for (int q = 0; q < QB; ++q) {
-          const uint2 rec = rec_at(min(ent0 + WAVE + q, ent1 - 1));
-          const int r = (int)(rec.x >> kOtherBits);
-          const float* const src = (r >= rowsU ? Pr : Qr) + (size_t)(rec.x & ((1u << kOtherBits) - 1u)) * D;
-          if (URE_OWNER_PREFETCH == 2 || gl == 0) asm volatile("prefetch.global.L1 [%0];" ::"l"(src + 4 * gl));
-        }
-      }
-#endif
       int key;
       float4 acc[V];
       if constexpr (V == 4) {
@@ -1477,16 +1388,9 @@ mf_owner_kernel(const ure_mf_shard_t* __restrict__ shards, int K, ure_mf_hparams
         if (epoch_sse != 0.0) atomicAdd(sh.sse + e, epoch_sse);
         epoch_sse = 0.0;
       }
-      unsigned polls = 0;
-      while (ld_acquire_u32(counter) < bar_target) {
-        if (hp.owner_ready && (++polls & 1023u) == 0u && ld_acquire_u32(reinterpret_cast<const unsigned*>(&ws->error)) >= 2u) {
-          s_abort = 1;                         // a CTA gave up waiting for its lists: nobody may wait for it
-          break;
-        }
-      }
+      while (ld_acquire_u32(counter) < bar_target) {}
     }
     __syncthreads();
-    if (s_abort) break;
     URE_STAMP(5)
     if (last_of_epoch) { ++e; k = 0; nlr = -lr_of(e); }
     else ++k;
@@ -1513,108 +1417,19 @@ int max_dyn_smem(int* out) {
   return 0;
 }
 
-// side stream + events of the concurrent pre-pass: one set per device, created on first use and kept for the life of
-// the process (the one piece of state the library holds; nothing the caller owns is referenced by it)
-struct CoStreams {
-  cudaStream_t side;
-  cudaEvent_t ev_in, ev_out;
-};
-int co_streams(CoStreams** out) {
-  static CoStreams table[64];
-  static bool made[64] = {};
-  int dev = 0;
-  URE_CUDA(cudaGetDevice(&dev));
-  URE_REQUIRE(dev >= 0 && dev < 64, URE_EUNSUPPORTED, "device index %d", dev);
-  if (!made[dev]) {
-    URE_CUDA(cudaStreamCreateWithFlags(&table[dev].side, cudaStreamNonBlocking));
-    URE_CUDA(cudaEventCreateWithFlags(&table[dev].ev_in, cudaEventDisableTiming));
-    URE_CUDA(cudaEventCreateWithFlags(&table[dev].ev_out, cudaEventDisableTiming));
-    made[dev] = true;
-  }
-  *out = &table[dev];
-  return 0;
-}
-
-constexpr int kCoThreads = 256;
-constexpr int kCoWarps = kCoThreads / 32;
-inline long long schedule_co_smem_bytes(int cap_slots, int tab_cap) {
-  // step + rank [cap] u16 | counters [warps][64] int | scan scratch | round tables 2 sets x 4 x [tab_cap] u16
-  return 2ll * cap_slots + 4ll * kCoWarps * 64 + 4ll * (kCoWarps + 4) + 2ll * 2 * 4 * tab_cap + 64;
-}
-// tab_cap / sb of the concurrent pre-pass, or tab_cap = 0 when the batch does not qualify (long epochs, halves beyond
-// the table size, per-warp ranges beyond the packed rank, a window shorter than the training)
-void schedule_co_params(const ure_mf_hparams_t& hp, int epochs, int* tab_cap, int* sb) {
-  *tab_cap = 0;
-  *sb = 1;
-  while ((1 << *sb) < hp.owner_spe_cap) ++*sb;
-  if (hp.owner_max_n <= 1 || hp.owner_spe_cap > 64 || hp.owner_sched_rows < epochs || hp.d > 32) return;
-  FeistelDomain dom;
-  dom.init((uint32_t)hp.owner_max_n);
-  const int cap = (int)((dom.a > dom.b ? dom.a : dom.b) + 2 + 7) / 8 * 8;
-  const int per = (((hp.owner_cap_slots + kCoWarps - 1) / kCoWarps) + 31) & ~31;
-  if (cap > kTabMaxHalf || per >= (1 << (16 - *sb))) return;
-  *tab_cap = cap;
-}
-int launch_schedule_co(const ure_mf_shard_t* d_shards, int K, const ure_mf_hparams_t& hp, int epochs, long long step0,
-                       cudaStream_t side) {
-  int tab_cap = 0, sb = 1;
-  schedule_co_params(hp, epochs, &tab_cap, &sb);
-  URE_REQUIRE(tab_cap > 0 && step0 == hp.owner_sched_step0, URE_EINVAL,
-              "ure_mf_train(owner): hparams.owner_ready is set but the batch does not qualify for the concurrent "
-              "pre-pass (ure_mf_owner_concurrent_ok)");
-  const long long need = schedule_co_smem_bytes(hp.owner_cap_slots, tab_cap);
-  auto kern = owner_schedule_tab_kernel<4, kCoThreads, true>;
-  URE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need));
-  URE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-  kern<<<dim3(num_sms(), 1), kCoThreads, (size_t)need, side>>>(d_shards, K, hp, epochs, step0, tab_cap, sb, 0, num_sms());
-  URE_CUDA(cudaGetLastError());
-  return 0;
-}
-
 template <int D>
 int launch_owner(const ure_mf_shard_t* d_shards, int K, const ure_mf_hparams_t& hp, int epochs, long long s0,
-                 long long s1, OwnerWs* ws, int smem, bool cached, unsigned dbg, cudaStream_t st) {
+                 long long s1, OwnerWs* ws, int smem, bool cached, cudaStream_t st) {
   const bool longlist = hp.owner_cap_list < hp.owner_cap_slots;
   auto kern = cached ? mf_owner_kernel<D, true, false>
                      : longlist ? mf_owner_kernel<D, false, true> : mf_owner_kernel<D, false, false>;
   URE_REQUIRE(!(cached && longlist), URE_EINVAL, "ure_mf_train(owner): the record cache needs owner_cap_list == owner_cap_slots");
   URE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   URE_CUDA(cudaMemsetAsync(ws->bar, 0, sizeof(ws->bar), st));
-  void* args[] = {(void*)&d_shards, (void*)&K,  (void*)&hp, (void*)&epochs,
-                  (void*)&s0,       (void*)&s1, (void*)&ws, (void*)&dbg};
-  if (!hp.owner_ready) {
-    URE_CUDA(cudaLaunchCooperativeKernel((void*)kern, dim3(num_sms()), dim3(kOwnThreads), args, (size_t)smem, st));
-    return 0;
-  }
-  // ---- concurrent schedule pre-pass (experiment, kernels.CONCURRENT_SCHEDULE / URE_SCHED_CO=1; off by default).
-  // The pre-pass is queued on a side stream behind everything the caller's stream holds up to here (the owner
-  // set-up), then the training kernel on the caller's stream -- an ordinary launch: a cooperative one does not share
-  // the device with a kernel of another stream; one CTA per SM is all that fits, so the grid is co-resident all the
-  // same -- and the caller's stream waits for the side stream after it.  All of an SM's shared memory is asked for,
-  // so that the second kernel fits the carve-out the first one set.  The pre-pass never waits for the training
-  // kernel, so nothing can dead-lock; the training kernel gives up on a row after ~2 s (error 3).
-  // MEASURED (C2 step, profiles/r2_notes.md): the two kernels do share the SMs (pre-pass 1.24 ms next to training),
-  // but the training kernel -- a dependent instruction stream at 16 warps per SM -- slows by as much as the pre-pass
-  // costs alone (2.27 -> 2.61 ms): device-resident step 3.22 vs 3.20 ms, end to end 3.75 vs 3.82 ms.
-  static const int seq = getenv("URE_SCHED_CO_SEQ") ? atoi(getenv("URE_SCHED_CO_SEQ")) : 0;
-  if (seq) {                               // debugging aid: the same two kernels one after the other on one stream
-    if (int rc = launch_schedule_co(d_shards, K, hp, epochs, s0, st)) return rc;
-    URE_CUDA(cudaLaunchCooperativeKernel((void*)kern, dim3(num_sms()), dim3(kOwnThreads), args, (size_t)smem, st));
-    return 0;
-  }
-  CoStreams* cs = nullptr;
-  if (int rc = co_streams(&cs)) return rc;
-  URE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-  URE_CUDA(cudaEventRecord(cs->ev_in, st));
-  URE_CUDA(cudaStreamWaitEvent(cs->side, cs->ev_in, 0));
-  if (int rc = launch_schedule_co(d_shards, K, hp, epochs, s0, cs->side)) return rc;
-  URE_CUDA(cudaEventRecord(cs->ev_out, cs->side));
-  URE_CUDA(cudaLaunchKernel((void*)kern, dim3(num_sms()), dim3(kOwnThreads), args, (size_t)smem, st));
-  URE_CUDA(cudaStreamWaitEvent(st, cs->ev_out, 0));
+  void* args[] = {(void*)&d_shards, (void*)&K, (void*)&hp, (void*)&epochs, (void*)&s0, (void*)&s1, (void*)&ws};
+  URE_CUDA(cudaLaunchCooperativeKernel((void*)kern, dim3(num_sms()), dim3(kOwnThreads), args, (size_t)smem, st));
   return 0;
 }
-
-unsigned g_owner_dbg = 0;
 
 }  // namespace
 
@@ -1626,7 +1441,6 @@ int mf_owner_trace(void* d_workspace, long long* d_trace, int steps, cudaStream_
   URE_CUDA(cudaStreamSynchronize(st));
   return 0;
 }
-void mf_owner_debug(unsigned flags) { g_owner_dbg = flags; }
 
 // called by ure_mf_train when hparams.mode == URE_MF_OWNER; the capacities in hparams are the plan's maxima the
 // caller read back after ure_mf_owner_prepare (the library never synchronises)
@@ -1656,11 +1470,11 @@ int mf_train_owner(const ure_mf_shard_t* d_shards, int n_shards, const ure_mf_hp
   auto* ws = static_cast<OwnerWs*>(d_workspace);
   const int smem = (int)need;
   switch (hp->d) {
-    case 8: return launch_owner<8>(d_shards, n_shards, *hp, epochs, step_begin, step_end, ws, smem, cached, g_owner_dbg, st);
-    case 16: return launch_owner<16>(d_shards, n_shards, *hp, epochs, step_begin, step_end, ws, smem, cached, g_owner_dbg, st);
-    case 32: return launch_owner<32>(d_shards, n_shards, *hp, epochs, step_begin, step_end, ws, smem, cached, g_owner_dbg, st);
-    case 64: return launch_owner<64>(d_shards, n_shards, *hp, epochs, step_begin, step_end, ws, smem, cached, g_owner_dbg, st);
-    case 128: return launch_owner<128>(d_shards, n_shards, *hp, epochs, step_begin, step_end, ws, smem, cached, g_owner_dbg, st);
+    case 8: return launch_owner<8>(d_shards, n_shards, *hp, epochs, step_begin, step_end, ws, smem, cached, st);
+    case 16: return launch_owner<16>(d_shards, n_shards, *hp, epochs, step_begin, step_end, ws, smem, cached, st);
+    case 32: return launch_owner<32>(d_shards, n_shards, *hp, epochs, step_begin, step_end, ws, smem, cached, st);
+    case 64: return launch_owner<64>(d_shards, n_shards, *hp, epochs, step_begin, step_end, ws, smem, cached, st);
+    case 128: return launch_owner<128>(d_shards, n_shards, *hp, epochs, step_begin, step_end, ws, smem, cached, st);
     default:
       set_error("ure_mf_train(owner): d=%d not in {8,16,32,64,128}", hp->d);
       return URE_EUNSUPPORTED;
@@ -1669,79 +1483,17 @@ int mf_train_owner(const ure_mf_shard_t* d_shards, int n_shards, const ure_mf_hp
 
 }  // namespace ure
 
-extern "C" int ure_mf_owner_concurrent_ok(const ure_mf_hparams_t* h_hp, int epochs) {
-  using namespace ure;
-  if (!h_hp || h_hp->mode != URE_MF_OWNER) return 0;
-#if !URE_OWNER_REGS
-  return 0;                                // the training kernel of this build leaves no registers for a second kernel
-#endif
-  int tab_cap = 0, sb = 1, avail = 0;
-  schedule_co_params(*h_hp, epochs, &tab_cap, &sb);
-  if (tab_cap <= 0 || max_dyn_smem(&avail) != 0) return 0;
-  // both kernels on one SM: the training CTA's shared memory + the pre-pass CTA's + static and reserved parts
-  const long long train = owner_smem_bytes(h_hp->d, h_hp->owner_cap_rows, h_hp->owner_cap_slots, h_hp->owner_cap_list,
-                                           (h_hp->owner_flags & 1) != 0);
-  return train + schedule_co_smem_bytes(h_hp->owner_cap_slots, tab_cap) + 20 * 1024 <= (long long)avail + 8 * 1024 ? 1 : 0;
-}
-
 extern "C" int64_t ure_mf_owner_smem_bytes(int d, int cap_rows, int cap_slots, int cap_list, int spe_cap, int flags) {
   const long long a = ure::owner_smem_bytes(d, cap_rows, cap_slots, cap_list, (flags & 1) != 0);
   const long long b = ure::schedule_smem_bytes(cap_slots, spe_cap, (flags & 2) == 0);
   return a > b ? a : b;
 }
 
-namespace ure {
-int mf_owner_schedule_impl(const ure_mf_shard_t* d_shards, int n_shards, const ure_mf_hparams_t* h_hp, int epochs,
-                           int64_t step0, void* stream, int cta0, int cta_n);
-}
 extern "C" int ure_mf_owner_schedule(const ure_mf_shard_t* d_shards, int n_shards, const ure_mf_hparams_t* h_hp,
                                      int epochs, int64_t step0, void* stream) {
-  return ure::mf_owner_schedule_impl(d_shards, n_shards, h_hp, epochs, step0, stream, 0, ure::num_sms());
-}
-
-// CTAs of the training grid per shard (make_plan's apportioning, on the host): h_c[s], and their sum = the grid
-extern "C" int ure_mf_owner_cta_split(const int32_t* h_n, int n_shards, int32_t* h_c) {
-  using namespace ure;
-  URE_REQUIRE(h_n && h_c && n_shards >= 1 && n_shards <= num_sms(), URE_EINVAL, "ure_mf_owner_cta_split: bad argument");
-  const int n_cta = num_sms();
-  long long N = 0;
-  for (int s = 0; s < n_shards; ++s) N += h_n[s];
-  if (N < 1) N = 1;
-  const long long spare = n_cta - n_shards;
-  long long rem[URE_MAX_SHARDS];
-  int used = 0;
-  for (int s = 0; s < n_shards; ++s) {
-    const long long x = spare * (long long)h_n[s];
-    h_c[s] = 1 + (int)(x / N);
-    rem[s] = x % N;
-    used += h_c[s];
-  }
-  for (int left = n_cta - used; left > 0; --left) {
-    int best = 0;
-    for (int s = 1; s < n_shards; ++s)
-      if (rem[s] > rem[best]) best = s;
-    ++h_c[best];
-    rem[best] = -1;
-  }
-  return 0;
-}
-
-// The pre-pass for the training CTAs [cta0, cta0 + cta_n) only -- the CTAs of the shards whose set-up is done
-// (ure_mf_owner_cta_split tells which): short epochs with round tables only (URE_EUNSUPPORTED otherwise).
-extern "C" int ure_mf_owner_schedule_part(const ure_mf_shard_t* d_shards, int n_shards, const ure_mf_hparams_t* h_hp,
-                                          int epochs, int64_t step0, int cta0, int cta_n, void* stream) {
-  using namespace ure;
-  URE_REQUIRE(cta0 >= 0 && cta_n >= 1 && cta0 + cta_n <= num_sms(), URE_EINVAL, "ure_mf_owner_schedule_part: CTA range");
-  return mf_owner_schedule_impl(d_shards, n_shards, h_hp, epochs, step0, stream, cta0, cta_n);
-}
-
-int ure::mf_owner_schedule_impl(const ure_mf_shard_t* d_shards, int n_shards, const ure_mf_hparams_t* h_hp, int epochs,
-                                int64_t step0, void* stream, int cta0, int cta_n) {
   using namespace ure;
   URE_REQUIRE(d_shards && h_hp && h_hp->owner_sched && h_hp->owner_sched_off, URE_EINVAL,
               "ure_mf_owner_schedule: null argument");
-  URE_REQUIRE(!h_hp->owner_ready, URE_EINVAL,
-              "ure_mf_owner_schedule: hparams.owner_ready is set -- the concurrent pre-pass is launched by ure_mf_train");
   URE_REQUIRE(h_hp->owner_sched_rows >= 1 && h_hp->owner_spe_cap >= 1 && h_hp->owner_spe_cap <= kMaxSpe &&
                   h_hp->owner_cap_slots % 16 == 0 && h_hp->owner_cap_slots <= 65520,
               URE_EUNSUPPORTED, "ure_mf_owner_schedule: rows=%d spe_cap=%d cap_slots=%d outside the supported range",
@@ -1760,30 +1512,19 @@ int ure::mf_owner_schedule_impl(const ure_mf_shard_t* d_shards, int n_shards, co
     const int cap = (int)((dom.a > dom.b ? dom.a : dom.b) + 2 + 7) / 8 * 8;
     if (cap <= kTabMaxHalf && schedule_smem_bytes(h_hp->owner_cap_slots, h_hp->owner_spe_cap, cache_j, cap) <= avail) tab_cap = cap;
   }
-  // short epochs with round tables: the tight kernel (two CTAs per SM)
-  {
-    static const int nt_env = getenv("URE_SCHED_NT") ? atoi(getenv("URE_SCHED_NT")) : 4;       // -1: general kernel (A/B)
-    int sb = 1;
-    while ((1 << sb) < h_hp->owner_spe_cap) ++sb;
-    const int per = (((h_hp->owner_cap_slots + kSchedWarps - 1) / kSchedWarps) + 31) & ~31;
-    const int nt = nt_env >= 4 ? 4 : nt_env >= 2 ? 2 : 0;
-    const long long need_t = schedule_tab_smem_bytes(h_hp->owner_cap_slots, tab_cap, nt);
-    if (nt_env >= 0 && tab_cap > 0 && h_hp->owner_spe_cap <= 64 && per < (1 << (16 - sb)) && need_t <= avail) {
-      auto kern = nt == 4 ? owner_schedule_tab_kernel<4, kSchedThreads, false>
-                          : nt == 2 ? owner_schedule_tab_kernel<2, kSchedThreads, false> : owner_schedule_tab_kernel<0, kSchedThreads, false>;
-      URE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need_t));
-      // 2 CTAs per SM: one wave -- of the whole grid, or (a part of the training CTAs) with more row classes per CTA
-      int ny2 = (2 * num_sms() + cta_n - 1) / cta_n;
-      if (ny2 > h_hp->owner_sched_rows) ny2 = h_hp->owner_sched_rows;
-      if (ny2 < 1) ny2 = 1;
-      kern<<<dim3(cta_n, ny2), kSchedThreads, (size_t)need_t, static_cast<cudaStream_t>(stream)>>>(
-          d_shards, n_shards, hp, epochs, step0, tab_cap, sb, cta0, num_sms());
-      URE_CUDA(cudaGetLastError());
-      return 0;
-    }
+  // short epochs with round tables: the tight kernel (two CTAs per SM, one wave)
+  int sb = 1;
+  while ((1 << sb) < h_hp->owner_spe_cap) ++sb;
+  const int per = (((h_hp->owner_cap_slots + kSchedWarps - 1) / kSchedWarps) + 31) & ~31;
+  const long long need_t = schedule_tab_smem_bytes(h_hp->owner_cap_slots, tab_cap);
+  if (tab_cap > 0 && h_hp->owner_spe_cap <= 64 && per < (1 << (16 - sb)) && need_t <= avail) {
+    URE_CUDA(cudaFuncSetAttribute(owner_schedule_tab_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need_t));
+    const int ny2 = h_hp->owner_sched_rows < 2 ? h_hp->owner_sched_rows : 2;
+    owner_schedule_tab_kernel<<<dim3(num_sms(), ny2), kSchedThreads, (size_t)need_t, static_cast<cudaStream_t>(stream)>>>(
+        d_shards, n_shards, hp, epochs, step0, tab_cap, sb);
+    URE_CUDA(cudaGetLastError());
+    return 0;
   }
-  URE_REQUIRE(cta0 == 0 && cta_n == num_sms(), URE_EUNSUPPORTED,
-              "ure_mf_owner_schedule_part: only the short-epoch pre-pass runs on a part of the grid");
   const long long need = schedule_smem_bytes(h_hp->owner_cap_slots, h_hp->owner_spe_cap, cache_j, tab_cap);
   URE_REQUIRE(need <= avail, URE_EUNSUPPORTED, "ure_mf_owner_schedule: %lld bytes of shared memory needed, %d available",
               need, avail);
@@ -1945,19 +1686,10 @@ extern "C" int64_t ure_mf_owner_radix_bytes(int n_shards) { return 2ll * n_shard
 namespace ure {
 int mf_owner_prepare_impl(const ure_mf_shard_t* d_shards, int n_shards, const ure_mf_hparams_t* h_hp, int epochs,
                           int max_rows, int32_t* d_radix_hist, void* d_workspace, void* stream, int flags);
-int mf_owner_prepare_part(const ure_mf_shard_t* d_all, int n_all, int shard0, int n_shards, const ure_mf_hparams_t* h_hp,
-                          int epochs, int max_rows, int32_t* d_radix_all, void* d_workspace, void* stream, int flags);
 }
 extern "C" int ure_mf_owner_prepare(const ure_mf_shard_t* d_shards, int n_shards, const ure_mf_hparams_t* h_hp,
                                     int epochs, int max_rows, int32_t* d_radix_hist, void* d_workspace, void* stream) {
   return ure::mf_owner_prepare_impl(d_shards, n_shards, h_hp, epochs, max_rows, d_radix_hist, d_workspace, stream, 0);
-}
-
-extern "C" int ure_mf_owner_prepare_part(const ure_mf_shard_t* d_shards, int n_shards, int shard0, int n_part,
-                                         const ure_mf_hparams_t* h_hp, int epochs, int max_rows, int32_t* d_radix_hist,
-                                         void* d_workspace, void* stream) {
-  return ure::mf_owner_prepare_part(d_shards, n_shards, shard0, n_part, h_hp, epochs, max_rows, d_radix_hist, d_workspace,
-                                    stream, 1 | 2 | 4);
 }
 
 // flags (the native batch runtime): 1 = the caller has just cleared the workspace; 2 = no plan kernel (the launch runs
@@ -1965,19 +1697,7 @@ extern "C" int ure_mf_owner_prepare_part(const ure_mf_shard_t* d_shards, int n_s
 // set-up in one cooperative launch
 int ure::mf_owner_prepare_impl(const ure_mf_shard_t* d_shards, int n_shards, const ure_mf_hparams_t* h_hp, int epochs,
                                int max_rows, int32_t* d_radix_hist, void* d_workspace, void* stream, int flags) {
-  return mf_owner_prepare_part(d_shards, n_shards, 0, n_shards, h_hp, epochs, max_rows, d_radix_hist, d_workspace, stream, flags);
-}
-
-// shards [shard0, shard0 + n_sub) of the batch (the whole batch: 0, n_shards).  A caller that uploads the shards one
-// after the other sets them up one by one, each as soon as its records have arrived, while the next one is on the bus.
-int ure::mf_owner_prepare_part(const ure_mf_shard_t* d_all, int n_all, int shard0, int n_shards, const ure_mf_hparams_t* h_hp,
-                               int epochs, int max_rows, int32_t* d_radix_all, void* d_workspace, void* stream, int flags) {
   using namespace ure;
-  URE_REQUIRE(shard0 >= 0 && n_shards >= 1 && shard0 + n_shards <= n_all, URE_EINVAL, "ure_mf_owner_prepare: shard range");
-  const ure_mf_shard_t* const d_shards = d_all + shard0;
-  int32_t* const d_radix_hist = d_radix_all ? d_radix_all + (long long)shard0 * 2 * kRadixBlocks * 256 : nullptr;
-  const bool whole = shard0 == 0 && n_shards == n_all;
-  if (!whole) flags |= 2 | 4 | 1;          // parts: no plan kernel, no inverse orders, the caller cleared the workspace
   URE_REQUIRE(d_shards && h_hp && d_workspace, URE_EINVAL, "ure_mf_owner_prepare: null argument");
   URE_REQUIRE(n_shards >= 1 && n_shards <= num_sms(), URE_EUNSUPPORTED,
               "ure_mf_owner_prepare: n_shards=%d outside [1,%d] (one CTA per shard at least)", n_shards, num_sms());
@@ -2010,7 +1730,7 @@ int ure::mf_owner_prepare_part(const ure_mf_shard_t* d_all, int n_all, int shard
       int n_sh = n_shards, sr = smem_rows, cbv = cb, np = npass;
       const ure_mf_shard_t* dsh = d_shards;
       int32_t* hist = d_radix_hist;
-      unsigned* uns = ws->unsorted + shard0;
+      unsigned* uns = ws->unsorted;
       void* args[] = {&dsh, &n_sh, &sr, &cbv, &np, &hist, &uns};
       URE_CUDA(cudaLaunchCooperativeKernel((void*)owner_setup_kernel, dim3(per_sm * num_sms()), dim3(kRadixThreads), args,
                                            (size_t)smem_ints * 4, st));
@@ -2020,12 +1740,12 @@ int ure::mf_owner_prepare_part(const ure_mf_shard_t* d_all, int n_all, int shard
     if (smem_rows)
       URE_CUDA(cudaFuncSetAttribute(csr_count_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_rows * 4));
     if (!(flags & 1)) URE_CUDA(cudaMemsetAsync(ws->unsorted, 0, sizeof(ws->unsorted), st));
-    csr_count_kernel<<<dim3(cb, n_shards), 1024, (size_t)smem_rows * 4, st>>>(d_shards, smem_rows, ws->unsorted + shard0);
+    csr_count_kernel<<<dim3(cb, n_shards), 1024, (size_t)smem_rows * 4, st>>>(d_shards, smem_rows, ws->unsorted);
     csr_scan_kernel<<<2 * n_shards, 1024, 0, st>>>(d_shards);
     for (int pass = 0; pass < npass; ++pass) {
-      radix_hist_kernel<<<dim3(kRadixBlocks, 2 * n_shards), kRadixThreads, 0, st>>>(d_shards, pass, npass, d_radix_hist, ws->unsorted + shard0);
-      radix_scan_kernel<<<2 * n_shards, 256, 0, st>>>(d_radix_hist, kRadixBlocks, ws->unsorted + shard0);
-      radix_scatter_kernel<<<dim3(kRadixBlocks, 2 * n_shards), kRadixThreads, 0, st>>>(d_shards, pass, npass, d_radix_hist, ws->unsorted + shard0);
+      radix_hist_kernel<<<dim3(kRadixBlocks, 2 * n_shards), kRadixThreads, 0, st>>>(d_shards, pass, npass, d_radix_hist, ws->unsorted);
+      radix_scan_kernel<<<2 * n_shards, 256, 0, st>>>(d_radix_hist, kRadixBlocks, ws->unsorted);
+      radix_scatter_kernel<<<dim3(kRadixBlocks, 2 * n_shards), kRadixThreads, 0, st>>>(d_shards, pass, npass, d_radix_hist, ws->unsorted);
     }
   }
   if (!(flags & 4)) perm_inverse_kernel<<<dim3(blocks, n_shards), 256, 0, st>>>(d_shards, epochs);

@@ -20,19 +20,13 @@
 //     "t + 1 steps applied" knows the row was rewritten during this very step and takes the previous version --
 //     the slot the writer did not touch.  Either way it reads the pre-step weights.
 //   Traffic per interaction: 2 x (1 KB row + tag) gathers + ~1.7 touched rows x 2 KB  ~ 5.4 KB at d = 128.
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "feistel.cuh"
-
-#ifndef URE_RUNS_STCS
-#define URE_RUNS_STCS 0
-#endif
 
 namespace ure {
 namespace {
 
-constexpr int kRunThreads = 512;           // default: 16 warps, no spills (~120 registers: two entries of a run in flight per warp)
+constexpr int kRunThreads = 512;           // 16 warps, no spills (~120 registers: two entries of a run in flight per warp)
 constexpr int KM = URE_MAX_SHARDS;
 constexpr int kRunTile = 32768;          // slots per CTA of the schedule pre-pass
 constexpr int kRunSortThreads = 512;
@@ -305,8 +299,8 @@ __device__ __forceinline__ int find_seg(const T* prefix, int nseg, T x) {
   return lo;
 }
 
-template <int D, int THREADS>
-__global__ void __launch_bounds__(THREADS, 1)
+template <int D>
+__global__ void __launch_bounds__(kRunThreads, 1)
 mf_runs_kernel(const ure_mf_shard_t* __restrict__ shards, int K, ure_mf_hparams_t hp, int epochs, long long step_begin,
                long long step_end, RunsWs* ws) {
   constexpr int G = D / 4;                 // lanes that carry a row (16-byte chunk each)
@@ -318,10 +312,10 @@ mf_runs_kernel(const ure_mf_shard_t* __restrict__ shards, int K, ure_mf_hparams_
   const bool act = lane < G;
   const float4* __restrict__ decay = reinterpret_cast<const float4*>(hp.decay);
   const float wd = hp.weight_decay, mu = hp.momentum, nlr = -hp.lr0;
-  const int n_warps = (int)(((long long)gridDim.x * THREADS) >> 5);
+  const int n_warps = (int)(((long long)gridDim.x * kRunThreads) >> 5);
   const int gwarp = (tid >> 5) * (int)gridDim.x + (int)blockIdx.x;      // CTA-minor: few units still use every SM
   unsigned bar_target = 0;
-  for (int s = tid; s < K; s += THREADS) s_sse_acc[s] = 0.f;
+  for (int s = tid; s < K; s += kRunThreads) s_sse_acc[s] = 0.f;
 
   for (long long t = step_begin; t < step_end; ++t) {
     const int tt = (int)t;
@@ -391,16 +385,8 @@ mf_runs_kernel(const ure_mf_shard_t* __restrict__ shards, int K, ure_mf_hparams_
         w_own.z = fmaf(nlr, b_own.z, w_own.z); w_own.w = fmaf(nlr, b_own.w, w_own.w);
         float* dst = S_own + ((long long)(cur_slot ^ 1) * rows_own + cur_row) * 2 * D;
         if (act) {
-#if URE_RUNS_STCS
-          // experiment (tools/build_variant.sh, -DURE_RUNS_STCS=1): the new version is not read again before the
-          // next step, so streaming stores could leave L2 to the rows of THIS step (each is read twice: by its owner
-          // and by the other side's gather).  Measured SLOWER: 0.66 -> 0.48 G interactions/s on one GPU's share of C4.
-          __stcs(reinterpret_cast<float4*>(dst) + lane, w_own);
-          __stcs(reinterpret_cast<float4*>(dst + D) + lane, b_own);
-#else
           __stcg(reinterpret_cast<float4*>(dst) + lane, w_own);
           __stcg(reinterpret_cast<float4*>(dst + D) + lane, b_own);
-#endif
         }
         __syncwarp();
         if (lane == 0) {
@@ -515,7 +501,7 @@ mf_runs_kernel(const ure_mf_shard_t* __restrict__ shards, int K, ure_mf_hparams_
       if (side == 0 && lane == 0 && sse_l != 0.f) atomicAdd(&s_sse_acc[s], sse_l);
     }
     __syncthreads();
-    for (int s = tid; s < K; s += THREADS) {
+    for (int s = tid; s < K; s += kRunThreads) {
       const float v = s_sse_acc[s];
       if (v != 0.f && s_epoch[s] >= 0) atomicAdd(shards[s].sse + s_epoch[s], (double)v);
       s_sse_acc[s] = 0.f;
@@ -527,16 +513,13 @@ mf_runs_kernel(const ure_mf_shard_t* __restrict__ shards, int K, ure_mf_hparams_
 template <int D>
 int launch_runs(const ure_mf_shard_t* d_shards, int K, const ure_mf_hparams_t& hp, int epochs, long long s0, long long s1,
                 RunsWs* ws, cudaStream_t st) {
-  // URE_RUNS_THREADS=768: 24 warps per SM with ~80 registers (a few spilled values) instead of 16 warps (experiments)
-  static const int threads = getenv("URE_RUNS_THREADS") ? atoi(getenv("URE_RUNS_THREADS")) : kRunThreads;
-  void* kern = threads == 768 ? (void*)mf_runs_kernel<D, 768> : (void*)mf_runs_kernel<D, kRunThreads>;
-  const int nt = threads == 768 ? 768 : kRunThreads;
+  void* kern = (void*)mf_runs_kernel<D>;
   int occ = 0;
-  URE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, nt, 0));
+  URE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kRunThreads, 0));
   URE_REQUIRE(occ >= 1, URE_ECOOP, "mf_runs_kernel<%d> cannot be resident", D);
   URE_CUDA(cudaMemsetAsync(&ws->barrier, 0, sizeof(unsigned), st));
   void* args[] = {(void*)&d_shards, (void*)&K, (void*)&hp, (void*)&epochs, (void*)&s0, (void*)&s1, (void*)&ws};
-  URE_CUDA(cudaLaunchCooperativeKernel(kern, dim3(num_sms()), dim3(nt), args, 0, st));
+  URE_CUDA(cudaLaunchCooperativeKernel(kern, dim3(num_sms()), dim3(kRunThreads), args, 0, st));
   return 0;
 }
 

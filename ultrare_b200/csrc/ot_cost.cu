@@ -17,7 +17,6 @@
 //   with tcgen05.ld, apply the norm epilogue and store the rows of M.
 // The problem is bound by reading X (4*n*d bytes), not by the tensor pipe (Appendix D).
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "tc_ptx.cuh"
@@ -59,7 +58,7 @@ __host__ __device__ inline CostSmemLayout cost_layout(int D, int NB, int stages)
 template <int D>
 __global__ void __launch_bounds__(kCostThreads)
 cost_tc_kernel(const float* __restrict__ X, long long n, const float* __restrict__ C, int k, int kpad, int NB,
-               int stages, uint32_t tmem_cols, float* __restrict__ M, double* __restrict__ inertia, int raw_hi) {
+               int stages, uint32_t tmem_cols, float* __restrict__ M, double* __restrict__ inertia) {
   constexpr int CH = D / 4;                    // 16-byte K chunks per row
   extern __shared__ __align__(128) unsigned char sm[];
   const CostSmemLayout L = cost_layout(D, NB, stages);
@@ -133,9 +132,7 @@ cost_tc_kernel(const float* __restrict__ X, long long n, const float* __restrict
       const float4 v = *reinterpret_cast<const float4*>(raw + r * D + c * 4);
       const float4 hi = make_float4(tf32_hi(v.x), tf32_hi(v.y), tf32_hi(v.z), tf32_hi(v.w));
       const float4 lo = make_float4(v.x - hi.x, v.y - hi.y, v.z - hi.z, v.w - hi.w);
-      // raw_hi (experiment, URE_COST_RAW_HI=1): hand the tensor core the UNTRUNCATED value as the hi operand -- equal
-      // results mean kind::tf32 ignores the low 13 mantissa bits, i.e. the raw tile can serve as the hi tile
-      *reinterpret_cast<float4*>(sm + L.a_hi + c * L.lbo_a + r * 16) = raw_hi ? v : hi;
+      *reinterpret_cast<float4*>(sm + L.a_hi + c * L.lbo_a + r * 16) = hi;
       *reinterpret_cast<float4*>(sm + L.a_lo + c * L.lbo_a + r * 16) = lo;
       float s = (v.x * v.x + v.y * v.y) + (v.z * v.z + v.w * v.w);
 #pragma unroll
@@ -200,8 +197,8 @@ cost_tc_kernel(const float* __restrict__ X, long long n, const float* __restrict
 }
 
 // ------------------------------------------------------------------ v2: tensor-map TMA straight into the UMMA layout
-// Measured on the B200 (tests with URE_COST_RAW_HI=1): tcgen05 kind::tf32 ignores the low 13 mantissa bits of its
-// operands, so the RAW fp32 tile is a valid `hi` operand: hi*B is computed on the truncated values either way.  The
+// Measured on the B200 (v1 handed the UNTRUNCATED tile as its hi operand: same results): tcgen05 kind::tf32 ignores the
+// low 13 mantissa bits of its operands, so the RAW fp32 tile is a valid `hi` operand: hi*B is computed on the truncated values either way.  The
 // tile therefore goes from global memory directly into the K-major core-matrix layout the tensor core reads
 // ([d/4 chunks][128 rows][16 B]: one 2-D TMA box {4 floats, 128 rows} per chunk, cp.async.bulk.tensor), and the only
 // generic-proxy pass left is lo = x - trunc(x) plus the row norms: half the shared-memory stores of v1, none of its
@@ -420,9 +417,8 @@ template <int D>
 int launch_cost_tma(const float* X, long long n, const float* C, int k, int kpad, float* M, double* inertia, cudaStream_t st,
                     int* used) {
   *used = 0;
-  static const int force_v1 = getenv("URE_COST_V1") ? atoi(getenv("URE_COST_V1")) : 0;
   EncodeTiledFn enc = encode_tiled();
-  if (force_v1 || !enc || D < 8 || (reinterpret_cast<uintptr_t>(X) & 15) != 0 || n >= (1ll << 31)) return 0;
+  if (!enc || D < 8 || (reinterpret_cast<uintptr_t>(X) & 15) != 0 || n >= (1ll << 31)) return 0;
   // column block and stages: prefer a footprint that lets two CTAs share an SM
   const int kcols = kpad < 16 ? 16 : kpad;      // kpad == 8: a 16-column MMA block, 8 columns stored
   int NB = kcols > 128 ? 128 : kcols, stages = 2;
@@ -431,13 +427,10 @@ int launch_cost_tma(const float* X, long long n, const float* C, int k, int kpad
   if (cost_layout2(D, NB, stages).total > 219 * 1024) stages = 1;
   if (cost_layout2(D, NB, stages).total > 219 * 1024) return 0;
   const int col_blocks = kcols / NB;
-  static const int one_acc = getenv("URE_COST_1ACC") ? atoi(getenv("URE_COST_1ACC")) : 0;
-  const int nacc = (!one_acc && 3 * NB <= 256) ? 3 : 1;      // two CTAs per SM share the 512 TMEM columns
+  const int nacc = 3 * NB <= 256 ? 3 : 1;      // two CTAs per SM share the 512 TMEM columns
   uint32_t tmem_cols = 32;
   while ((int)tmem_cols < nacc * NB) tmem_cols <<= 1;
-  static const int no_sw = getenv("URE_COST_NOSW") ? atoi(getenv("URE_COST_NOSW")) : 0;
-  constexpr bool kCanSw = D >= 32;             // a 128-byte swizzle atom is 32 floats of K
-  const bool sw = kCanSw && !no_sw;
+  constexpr bool sw = D >= 32;                 // a 128-byte swizzle atom is 32 floats of K
   CUtensorMap tmap;
   const cuuint64_t dims[2] = {(cuuint64_t)D, (cuuint64_t)n};
   const cuuint64_t strides[1] = {(cuuint64_t)D * 4};
@@ -448,11 +441,7 @@ int launch_cost_tma(const float* X, long long n, const float* C, int k, int kpad
           CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
     return 0;
   const CostSmemLayout2 L = cost_layout2(D, NB, stages);
-  void (*kern)(const CUtensorMap, long long, const float*, int, int, int, int, uint32_t, float*, double*, int) =
-      cost_tma_kernel<D, false>;
-  if constexpr (kCanSw) {
-    if (sw) kern = cost_tma_kernel<D, true>;
-  }
+  auto kern = cost_tma_kernel<D, sw>;
   const size_t smem = (size_t)L.total + 1024;
   URE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   URE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
@@ -717,10 +706,9 @@ template <int D>
 int launch_cost_ws(const float* X, long long n, const float* C, int k, int kpad, float* M, double* inertia, cudaStream_t st,
                    int* used) {
   *used = 0;
-  static const int off = getenv("URE_COST_WS") ? !atoi(getenv("URE_COST_WS")) : 0;
   EncodeTiledFn enc = encode_tiled();
   const int NB = kpad < 16 ? 16 : kpad;
-  if (off || !enc || D < 32 || NB > 128 || (reinterpret_cast<uintptr_t>(X) & 15) != 0 || n >= (1ll << 31)) return 0;
+  if (!enc || D < 32 || NB > 128 || (reinterpret_cast<uintptr_t>(X) & 15) != 0 || n >= (1ll << 31)) return 0;
   const CostWsLayout L = cost_ws_layout(D, NB);
   const size_t smem = (size_t)L.total + 1024;
   if (L.S == 0 || smem > 227 * 1024) return 0;
@@ -801,19 +789,15 @@ int launch_cost_tc(const float* X, long long n, const float* C, int k, int kpad,
     if (used == 2) return launch_rowmin(M, n, k, kpad, inertia, st);
   }
   // choose the column block NB (multiple of 16) and the number of raw stages that fit in shared memory
-  // one raw stage leaves room for a second CTA per SM at d = 64 (its latency phases then overlap the other CTA's
-  // work); URE_COST_STAGES=1|2 pins the choice (experiments)
-  static const int want_stages = getenv("URE_COST_STAGES") ? atoi(getenv("URE_COST_STAGES")) : 0;
-  const uint32_t budget = want_stages == 1 ? 110 * 1024 : 220 * 1024;
+  const uint32_t budget = 220 * 1024;
   const int kcols = kpad < 16 ? 16 : kpad;      // kpad == 8: a 16-column MMA block, 8 columns stored
-  int NB = kcols, stages = want_stages == 1 ? 1 : 2;
+  int NB = kcols, stages = 2;
   while (true) {
     if (cost_layout(D, NB, stages).total <= budget) break;
     if (stages == 2 && cost_layout(D, NB, 1).total <= budget) { stages = 1; break; }
-    if (NB <= 16 && want_stages == 1 && budget < 220 * 1024) { stages = 1; break; }      // cannot halve further
     if (NB <= 16) { set_error("ure_cost_matrix: d=%d does not fit shared memory", D); return URE_EUNSUPPORTED; }
     NB = ((NB / 2 + 15) / 16) * 16;
-    stages = want_stages == 1 ? 1 : 2;
+    stages = 2;
   }
   const int col_blocks = (kcols + NB - 1) / NB;
   URE_REQUIRE(col_blocks * NB == kcols, URE_EUNSUPPORTED, "ure_cost_matrix: kpad=%d not divisible into %d-column blocks",
@@ -834,9 +818,8 @@ int launch_cost_tc(const float* X, long long n, const float* C, int k, int kpad,
   if (gx < 1) gx = 1;
   if (gx > n_tiles) gx = n_tiles;
   double* fused_inertia = (col_blocks == 1) ? inertia : nullptr;
-  static const int raw_hi = getenv("URE_COST_RAW_HI") ? atoi(getenv("URE_COST_RAW_HI")) : 0;
   kern<<<dim3((unsigned)gx, (unsigned)col_blocks), kCostThreads, L.total, st>>>(X, n, C, k, kpad, NB, stages, tmem_cols, M,
-                                                                            fused_inertia, raw_hi);
+                                                                            fused_inertia);
   URE_CUDA(cudaGetLastError());
   if (inertia && !fused_inertia) return launch_rowmin(M, n, k, kpad, inertia, st);
   return 0;

@@ -18,8 +18,6 @@
 // the same exponential feeds the row sum (times 2^r, a per-lane constant) and the column sum.  Partial sums
 // travel as (r, s) pairs: lanes -> warp (shuffle) -> CTA (shared memory, fixed order) -> grid (one fp64 atomic
 // per column and CTA of s * 2^r / n, r clamped at -960; the cluster form keeps the pairs to the end).
-#include <stdlib.h>
-
 #include "common.cuh"
 #include <cooperative_groups.h>
 
@@ -236,7 +234,7 @@ __global__ void update_g_kernel(float* g, double* colsum, int k, float eps) {
   }
 }
 
-// --------------------------------------------------------------------------- persistent Sinkhorn
+// --------------------------------------------------------------------------- persistent Sinkhorn, rows of M in shared memory
 struct SkStages {
   float eps[kMaxStages];
   int iters[kMaxStages];
@@ -251,11 +249,11 @@ struct SkWorkspace {
   long long iters_done;
 };
 
-template <int KPAD, bool CACHED>
-__global__ void __launch_bounds__(kSkThreads, CACHED ? 1 : 2)
+template <int KPAD>
+__global__ void __launch_bounds__(kSkThreads, 1)
 sinkhorn_kernel(const float* __restrict__ M, long long n, int k, float* __restrict__ g_io, SkStages stages,
                 SkWorkspace* ws) {
-  extern __shared__ __align__(16) float m_sh[];     // part_r | part_s [warps][KPAD]; CACHED: then this CTA's rows of M
+  extern __shared__ __align__(16) float m_sh[];     // part_r | part_s [warps][KPAD], then this CTA's rows of M
   __shared__ float g_sh[KPAD];
   constexpr int NWARP = kSkThreads / 32;
   float* const part_r = m_sh;
@@ -266,11 +264,9 @@ sinkhorn_kernel(const float* __restrict__ M, long long n, int k, float* __restri
   const long long r0 = per * blockIdx.x < n ? per * blockIdx.x : n;
   const long long r1 = r0 + per < n ? r0 + per : n;
   for (int j = tid; j < KPAD; j += blockDim.x) g_sh[j] = j < k ? g_io[j] : 0.f;
-  if (CACHED) {
-    const long long cnt4 = (r1 - r0) * (KPAD / 4);
-    const float4* src = reinterpret_cast<const float4*>(M + r0 * KPAD);
-    for (long long x = tid; x < cnt4; x += blockDim.x) reinterpret_cast<float4*>(rows_sh)[x] = __ldg(src + x);
-  }
+  const long long cnt4 = (r1 - r0) * (KPAD / 4);
+  const float4* src = reinterpret_cast<const float4*>(M + r0 * KPAD);
+  for (long long x = tid; x < cnt4; x += blockDim.x) reinterpret_cast<float4*>(rows_sh)[x] = __ldg(src + x);
   __syncthreads();
   const double a = 1.0 / (double)n;
   const double logb = -log((double)k);
@@ -282,7 +278,7 @@ sinkhorn_kernel(const float* __restrict__ M, long long n, int k, float* __restri
     for (int it = 0; it < stages.iters[s]; ++it, ++it_global) {
       double* cs = ws->colsum[it_global % 3];
       if (r0 < r1) {
-        colsum_rows<KPAD>(CACHED ? rows_sh : M, CACHED ? r0 : 0, r0, r1, g_sh, k, scale, part_r, part_s);
+        colsum_rows<KPAD>(rows_sh, r0, r0, r1, g_sh, k, scale, part_r, part_s);
         __syncthreads();
         for (int j = tid; j < k; j += blockDim.x) {
           float R, S;
@@ -807,10 +803,10 @@ int check_mk(const void* M, long long n, int k, int kpad, const char* who) {
   return 0;
 }
 
-template <int KPAD, bool CACHED>
+template <int KPAD>
 int launch_sinkhorn(const float* M, long long n, int k, float* g, const SkStages& st, SkWorkspace* ws, int grid,
                     size_t smem, cudaStream_t stream) {
-  auto kern = sinkhorn_kernel<KPAD, CACHED>;
+  auto kern = sinkhorn_kernel<KPAD>;
   URE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int occ = 0;
   URE_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kSkThreads, smem));
@@ -911,19 +907,7 @@ extern "C" int ure_sinkhorn(const float* d_M, int64_t n, int k, int kpad, float*
   if ((long long)need <= (long long)smem_optin - 2048) {     // minus the kernel's static shared memory
     // the cost rows fit the SMs' shared memory (n = 1 M users at k <= 8: 216 KB per SM): one persistent launch, M is
     // read from HBM once for ALL iterations, an iteration costs a shared-memory sweep + one grid barrier
-    URE_KPAD_SWITCH(kpad, return (launch_sinkhorn<KP, true>(d_M, n, k, d_g, stg, ws, grid, need, st)));
-  }
-  {
-    // large problem, one persistent launch (two CTAs per SM, one grid barrier per iteration); URE_SK_PERSIST=0: the
-    // split-phase kernels below (two launches per iteration)
-    static const int persist = getenv("URE_SK_PERSIST") ? atoi(getenv("URE_SK_PERSIST")) : 0;
-    if (persist) {
-      int occ = 1;
-      URE_KPAD_SWITCH(kpad, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, (sinkhorn_kernel<KP, false>), kSkThreads, parts));
-      if (occ < 1) occ = 1;
-      if (occ > 2) occ = 2;
-      URE_KPAD_SWITCH(kpad, return (launch_sinkhorn<KP, false>(d_M, n, k, d_g, stg, ws, grid * occ, parts, st)));
-    }
+    URE_KPAD_SWITCH(kpad, return (launch_sinkhorn<KP>(d_M, n, k, d_g, stg, ws, grid, need, st)));
   }
   // large problem: one streaming pass per iteration at full occupancy (split-phase kernels, no host sync;
   // the early exit needs the column sums on the host, so every scheduled iteration runs)

@@ -175,7 +175,7 @@ def _upload_ring(dst_ptr: int, src_ptr: int, nb: int) -> None:
 
 
 def upload_interactions_many(raws, device, row_of: Optional[torch.Tensor] = None, defer: bool = False,
-                             stream=None, events: Optional[list] = None, eager: Optional[list] = None):
+                             eager: Optional[list] = None):
     """float64 [3, n] arrays (uid, iid, rating/max_rating: what readRating returns, reference read.py:64-68) ->
     int32 [n,4] ure_inter_t records on `device`, packed ON the device (ure_pack_interactions_f64).
 
@@ -185,9 +185,6 @@ def upload_interactions_many(raws, device, row_of: Optional[torch.Tensor] = None
 
     defer=True returns (outs, finish): the staging copies are already running on the worker threads, `finish()`
     waits for them and queues the uploads + pack kernels -- the caller does other host work in between.
-    stream (a torch.cuda.Stream) + events (a list to fill): arrays that live in page-locked memory are shipped on that
-    stream, and events[j] is recorded there behind array j's pack kernel (None for arrays that went the ordinary way):
-    the caller's stream waits for exactly the arrays it needs, while the later ones are still on the bus.
     eager[j] = (device columns, event) of an array whose copy was started earlier (eager_upload): only its pack kernel
     is queued here, behind the event."""
     dev = torch.device(device)
@@ -215,8 +212,6 @@ def upload_interactions_many(raws, device, row_of: Optional[torch.Tensor] = None
     if 8 * tot_d > UPLOAD_ONE_SHOT_BYTES:
         # too large to stage whole: array after array, each through the two-segment ring (or straight from its own
         # page-locked memory) into a device buffer that lives until its pack kernel has run
-        if events is not None:
-            events[:] = [None] * len(arrs)
 
         def one_by_one():
             with torch.cuda.device(dev):
@@ -283,26 +278,11 @@ def upload_interactions_many(raws, device, row_of: Optional[torch.Tensor] = None
     # arrays that already live in page-locked memory need no staging copy: their upload + pack are queued right here
     # (defer or not), so the DMA engine starts while the caller still does its host-side set-up
     shipped = set()
-    if events is not None:
-        events[:] = [None] * len(arrs)
     with torch.cuda.device(dev):
-        if stream is not None and events is not None and any(pinned[j] is not None for j in todo):
-            main = torch.cuda.current_stream()
-            stream.wait_stream(main)                 # the fresh buffers may be recycled blocks of the caller's stream
-            out_all.record_stream(stream)
-            cols_all.record_stream(stream)
-            with torch.cuda.stream(stream):
-                for j in todo:
-                    if pinned[j] is not None:
-                        ship(j)
-                        shipped.add(j)
-                        events[j] = torch.cuda.Event()
-                        events[j].record()
-        else:
-            for j in todo:
-                if pinned[j] is not None:
-                    ship(j)
-                    shipped.add(j)
+        for j in todo:
+            if pinned[j] is not None:
+                ship(j)
+                shipped.add(j)
     futs = None
     if n_tot >= (1 << 16):
         # staging copies on worker threads (ctypes releases the GIL); every array is shipped as soon as ITS
@@ -848,10 +828,6 @@ class ShardBatch:
                 t1 = step_end
                 if self.mode in ("owner", "runs"):
                     t1 = min(step_end, self._schedule_window())
-                if getattr(self, "concurrent", False):
-                    if self.step != 0 or t1 != self.total_steps:
-                        raise RuntimeError("ultrare_b200: a batch built with whole_training=True trains all steps in one call")
-                    self.launches_per_pass += 1        # the concurrent pre-pass
                 check(L.ure_mf_train(_ptr(self.table), self.n_shards, C.byref(self.hp), self.epochs,
                                      self.step, t1, self.warps_group0, _ptr(self.ws), _stream()), "ure_mf_train")
                 self.launches_per_pass += 1
@@ -863,11 +839,6 @@ class ShardBatch:
         L = _lib.lib()
         a, b = self._sched_cover
         rows = self.hp.owner_sched_rows if self.mode == "owner" else self.hp.runs_rows
-        if getattr(self, "concurrent", False):
-            # ure_mf_train launches the pre-pass next to the training kernel: one window, one training call
-            self._sched_cover = (0, self.total_steps)
-            self.hp.owner_sched_step0 = 0
-            return self.total_steps
         if not (a <= self.step < b):
             with torch.cuda.device(self.device):
                 if self.mode == "owner":
@@ -895,8 +866,6 @@ class ShardBatch:
             st.bufP.zero_()
             st.bufQ.zero_()
             st.sse.zero_()
-        if getattr(self, "concurrent", False):
-            self._ready.zero_()                         # the pre-pass runs again next to the training kernel
         self.step = 0
 
     def flush(self) -> None:
@@ -945,10 +914,6 @@ class ShardBatch:
             vals = host[:nb].view(torch.float64).numpy().reshape(K, E).copy()
             err = int(host[nb:nb + 4].view(torch.int32).item()) if owner else 0
             _PINNED_BYTES.setdefault(host.shape[0], []).append((host, None))
-            if err == 3:
-                global CONCURRENT_SCHEDULE
-                CONCURRENT_SCHEDULE = False
-                raise ConcurrentScheduleStall("ultrare_b200: the concurrent schedule pre-pass stalled; repeat the pass")
             if err == 2:
                 _PLAN_HINTS.pop(getattr(self, "_plan_sig", None), None)
                 raise PlanHintMiss("ultrare_b200: the remembered owner plan does not cover this batch; repeat the pass")
@@ -984,15 +949,6 @@ class PlanHintMiss(RuntimeError):
     set-up kernels found: nothing was trained; the caller repeats the pass (the hint is gone, so it waits for the plan)."""
 
 
-class ConcurrentScheduleStall(PlanHintMiss):
-    """The concurrent schedule pre-pass did not deliver a row within the training kernel's patience (it could not be
-    co-scheduled on this device?): nothing usable was trained; CONCURRENT_SCHEDULE is switched off, repeat the pass."""
-
-
-# Schedule pre-pass NEXT TO the training kernel (hparams.owner_ready) instead of before it.  Off by default: measured on
-# the C2 step, the training kernel slows by as much as the pre-pass costs alone (profiles/r2_notes.md).
-CONCURRENT_SCHEDULE = os.environ.get("URE_SCHED_CO", "0") == "1"
-PIPELINE_GROUPS = int(os.environ.get("URE_PIPE_GROUPS", "1"))   # shard groups set up while the next one uploads (1: off)
 _PLAN_HINTS = {}          # batch signature -> (max_rows, max_slots, max_spe, smem) of the last plan read back
 PLAN_HINT_MARGIN = 0.03   # capacities of an optimistic launch: the remembered maxima plus this fraction
 
@@ -1009,18 +965,11 @@ class ArenaShardBatch(ShardBatch):
     def __init__(self, recs, rows_P, n_item: int, d: int, batch: int, epochs: int, shard_ids, perm_seed: int = 42,
                  perms=None, lr: float = 1e-3, lr_decay: float = 0.95, lr_step: int = 50, weight_decay: float = 0.1,
                  momentum: float = 0.9, generator=None, std: float = 1.0, mode: str = "auto", owner_cache: bool = True,
-                 optimistic: bool = False, whole_training: bool = False, ready_events=None):
+                 optimistic: bool = False):
         """optimistic: the caller reads the training losses (train_losses_async) only after everything that depends
         on the training is queued, and repeats the pass on PlanHintMiss.  The launch is then queued with the
         capacities of the last plan read back for the same shapes (+ PLAN_HINT_MARGIN) instead of waiting for this
-        one's -- the kernels compare them with the real plan on the device (hparams.owner_plan).
-        whole_training: the caller will train all steps with ONE train() call.  The schedule pre-pass then runs
-        CONCURRENTLY with the training kernel (hparams.owner_ready) when the batch qualifies
-        (ure_mf_owner_concurrent_ok), on the registers and shared memory the training kernel leaves free.
-        ready_events: per shard, the event behind its records when they are still on their way (uploads on a side
-        stream, read.RatingData.upload_many(stream=...)), else None.  On the optimistic path the shards are then set up
-        ONE BY ONE -- set-up kernels and schedule pre-pass of shard j queued behind event j -- so that the SMs work on
-        the first shards while the later ones are still on the bus; otherwise the stream simply waits for all of them."""
+        one's -- the kernels compare them with the real plan on the device (hparams.owner_plan)."""
         K = self.n_shards = len(recs)
         tq = [("start", time.perf_counter())]                # host stamps of the constructor (diagnostics: ctor_ms)
         stamp = lambda name: tq.append((name, time.perf_counter()))
@@ -1072,7 +1021,7 @@ class ArenaShardBatch(ShardBatch):
         stamp("alloc")
         self.table_ptr = base + int(lay.table)
         self.ws = self.arena[int(lay.ws):int(lay.ws) + int(L.ure_mf_train_workspace_bytes())]
-        self.mode, self.optimistic, self.step, self.concurrent = "dense", False, 0, False
+        self.mode, self.optimistic, self.step = "dense", False, 0
         info = (C.c_int32 * 8)()
         force = OWNER_FORCE if OWNER_FORCE is not None else (-1, 0)
         sig = (K, d, batch, int(n_item), tuple(self._rows_P), self.epochs, perms is not None, bool(owner_cache),
@@ -1095,56 +1044,14 @@ class ArenaShardBatch(ShardBatch):
             if rc == 1:
                 self.optimistic, self.plan_sync_ms = True, 0.0
                 self.hp.owner_plan = self.ws.data_ptr()
-        pending = [e for e in (ready_events or []) if e is not None]
-        self.pipelined = bool(pending and self.optimistic and lay.owner and perms is None and self.total_steps > 0 and
-                              not CONCURRENT_SCHEDULE and PIPELINE_GROUPS > 1 and K > 1)
-        piped_schedule = False
         with torch.cuda.device(dev):
-            main = torch.cuda.current_stream()
-            if pending and not self.pipelined:
-                for e in pending:                        # records still on the bus: the whole set-up waits for them
-                    main.wait_event(e)
             npass = 1
             while npass < 4 and (int(lay.max_rows) - 1) >> (8 * npass):
                 npass += 1
             check(L.ure_mf_batch_setup(hs, K, n_item, C.byref(self.hp), self.epochs, self._perm_seed, C.c_void_p(base),
-                                       C.byref(lay), C.c_void_p(stage.data_ptr()),
-                                       (1 if self.optimistic else 0) | (2 if self.pipelined else 0), _stream()),
+                                       C.byref(lay), C.c_void_p(stage.data_ptr()), 1 if self.optimistic else 0, _stream()),
                   "ure_mf_batch_setup")
-            if self.pipelined:
-                # shard by shard: set-up + pre-pass of shard j behind the arrival of its records
-                n_arr, c_arr = (C.c_int32 * K)(*ns), (C.c_int32 * K)()
-                check(L.ure_mf_owner_cta_split(n_arr, K, c_arr), "ure_mf_owner_cta_split")
-                radix = C.c_void_p(base + int(lay.radix))
-                tab, wsp = C.c_void_p(base + int(lay.table)), C.c_void_p(base + int(lay.ws))
-                # contiguous groups of shards of about equal bytes (a part per shard would pay the latency of eight
-                # small kernels per shard: measured, the gain goes into them)
-                G = max(1, min(PIPELINE_GROUPS, K))
-                tot, acc, groups, g0 = float(sum(ns)) or 1.0, 0, [], 0
-                for j in range(K):
-                    acc += ns[j]
-                    if acc >= tot * (len(groups) + 1) / G or j == K - 1:
-                        groups.append((g0, j + 1))
-                        g0 = j + 1
-                piped_schedule, cta0 = True, 0
-                for a, b in groups:
-                    for j in range(a, b):
-                        if ready_events[j] is not None:
-                            main.wait_event(ready_events[j])
-                    check(L.ure_mf_owner_prepare_part(tab, K, a, b - a, C.byref(self.hp), self.epochs, int(lay.max_rows), radix,
-                                                      wsp, _stream()), "ure_mf_owner_prepare_part")
-                    self.launches_per_pass += 2 + 3 * npass
-                    c_grp = sum(int(c_arr[j]) for j in range(a, b))
-                    if piped_schedule and sum(ns[a:b]) > 0:
-                        self.hp.owner_sched_step0 = 0
-                        rc_s = L.ure_mf_owner_schedule_part(tab, K, C.byref(self.hp), self.epochs, 0, cta0, c_grp, _stream())
-                        if rc_s == 0:
-                            self.launches_per_pass += 1
-                        else:                            # not the short-epoch pre-pass: one launch for all, below
-                            piped_schedule = False
-                    cta0 += c_grp
-                self.prepare_launches = len(groups) * (2 + 3 * npass)
-            elif lay.owner:
+            if lay.owner:
                 # count + scan, radix passes, [inverse visiting orders], [plan]
                 # one cooperative launch for batches of up to 8 M interactions (csrc/mf_batch.cu: flags & 8), unless
                 # URE_SETUP_FUSED says otherwise
@@ -1191,20 +1098,8 @@ class ArenaShardBatch(ShardBatch):
                 self.mode = "owner"
                 self._sched_cover = (0, 0)
                 self._spes = [-(-n // batch) for n in ns if n > 0]
-                self.concurrent = bool(whole_training and CONCURRENT_SCHEDULE and self.total_steps > 0 and
-                                       L.ure_mf_owner_concurrent_ok(C.byref(self.hp), self.epochs))
-                self.owner_plan["concurrent_schedule"] = self.concurrent
-                if self.concurrent:
-                    self.hp.owner_ready = base + int(lay.ready)
-                    self._ready = self.arena[int(lay.ready):int(lay.ready) + 4 * int(lay.grid) * int(lay.sched_rows)]
                 if self.optimistic:
-                    if piped_schedule:
-                        # the pre-pass went out shard by shard above: the window is covered
-                        rows = self.hp.owner_sched_rows
-                        self._sched_cover = (0, min([rows * spe for spe in self._spes if rows < self.epochs] or
-                                                    [self.total_steps]))
-                    else:
-                        self._schedule_window()          # the pre-pass is queued before anything else
+                    self._schedule_window()              # the pre-pass is queued before anything else
                     stamp("schedule_queued")
                     fill_weights()
             elif mode == "owner":

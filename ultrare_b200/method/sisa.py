@@ -252,8 +252,7 @@ class Sisa(Scratch):
         self.dist.all_reduce(out)
         vals = kn.download_many([out])[0]
         if vals[4] > 0:                        # on some rank: every rank repeats the pass (Sisa._retrying)
-            raise kn.PlanHintMiss("ultrare_b200: a rank's remembered owner plan did not cover its batch (or its "
-                                  "concurrent pre-pass stalled)")
+            raise kn.PlanHintMiss("ultrare_b200: a rank's remembered owner plan did not cover its batch")
         n_test = sum(len(t.dataset) for t in test_dlist)
         users = max(vals[3], 1.0)
         return float(np.sqrt(vals[0] / max(1, n_test))), float(vals[1] / users), float(vals[2] / users)
@@ -310,18 +309,11 @@ class Sisa(Scratch):
             # the staging copies of the shards' records run on worker threads while the models are allocated
             from ..read import RatingData
             from .utils import MF
-            # kernels.PIPELINE_GROUPS > 1 (experiment, off by default): page-locked arrays go up on a side stream, one
-            # event per shard, and the batch runtime sets the shards up group by group as they arrive
-            # (kernels.ArenaShardBatch(ready_events=...)) instead of after the last byte
-            from ..read import _mapped_key
-            up_stream = kn.side_stream(self.device) if (batched and mode != 'faithful' and kn.PIPELINE_GROUPS > 1) else None
             uploaded = RatingData.upload_many([train_dlist[i].dataset for i in mine], self.device,
                                               self._row_of if compact else None, 'sisa_local' if compact else None,
-                                              defer=True, stream=up_stream)
+                                              defer=True)
             t_a = time.time()
             uploaded()
-            rec_key = _mapped_key(self.device, 'sisa_local', self._row_of) if compact else str(self.device)
-            ready_events = [train_dlist[i].dataset.take_upload_event(rec_key) for i in mine] if up_stream is not None else None
             recs = [(train_dlist[i].dataset.records_mapped(self.device, self._row_of, 'sisa_local') if compact
                      else train_dlist[i].dataset.records(self.device)) for i in mine]
             batch = train_dlist[mine[0]].batch_size
@@ -340,8 +332,7 @@ class Sisa(Scratch):
                                         perms if any(p is not None for p in perms) else None, self.lr, self.lr_decay,
                                         50, self.lam, self.momentum,
                                         generator=lambda: model_generator(self.seed, mine[0] + 1, self.device),
-                                        optimistic=optimistic, whole_training=mode in ('none', 'final', 'faithful-last'),
-                                        ready_events=ready_events)
+                                        optimistic=optimistic)
                 states = None
             else:
                 for j, i in enumerate(mine):
@@ -603,13 +594,6 @@ class Sisa(Scratch):
             return once(*args)
         except kn.PlanHintMiss:
             kn._PLAN_HINTS.clear()
-            if self.dist.world > 1:
-                # was it a stalled concurrent pre-pass somewhere?  Every rank is here (the flag travelled with the
-                # all-reduced sums), so one more scalar reduction is safe; the mode goes off on all ranks together
-                sb = getattr(self, '_last_batch', None)
-                mine = int(sb.ws[16:20].view(torch.int32).item()) == 3 if sb is not None else False
-                if self.dist.max_float(1.0 if mine else 0.0) > 0:
-                    kn.CONCURRENT_SCHEDULE = False
             self._pending_logs = None
             self._join_writers()
             return once(*args)

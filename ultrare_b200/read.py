@@ -168,22 +168,11 @@ class RatingData:
                 torch.tensor(self.items[idx], dtype=torch.long),
                 torch.tensor(self.ratings[idx], dtype=torch.float32))
 
-    def take_upload_event(self, key):
-        """The event behind records that were shipped on a side stream (upload_many(stream=...)), handed over ONCE: the
-        taker's stream has to wait for it before it touches the records."""
-        return self.__dict__.get('_upload_events', {}).pop(key, None)
-
-    def _wait_upload(self, key):
-        ev = self.take_upload_event(key)
-        if ev is not None:
-            torch.cuda.current_stream(ev.device if hasattr(ev, 'device') else None).wait_event(ev)
-
     def records(self, device) -> torch.Tensor:
         """int32 [n,4] ure_inter_t records resident on `device` (uploaded once)."""
         key = str(device)
         if key not in self._records:
             self._records[key] = kn.upload_interactions(self._raw, device, eager=self._take_eager(device))
-        self._wait_upload(key)
         return self._records[key]
 
     def records_mapped(self, device, row_of: torch.Tensor, tag: str) -> torch.Tensor:
@@ -194,7 +183,6 @@ class RatingData:
             self._drop_mapped(device, tag)
             self._records[key] = kn.upload_interactions(self._raw, device, row_of, eager=self._take_eager(device))
             self._keep_map(key, row_of)
-        self._wait_upload(key)
         return self._records[key]
 
     def _drop_mapped(self, device, tag):
@@ -207,11 +195,10 @@ class RatingData:
         self._maps[key] = row_of              # holds the tensor: its address cannot be reused while the key lives
 
     @staticmethod
-    def upload_many(datasets, device, row_of=None, tag=None, defer=False, stream=None):
+    def upload_many(datasets, device, row_of=None, tag=None, defer=False):
         """records()/records_mapped() of several datasets at once: their host copies run in parallel.
         defer=True: the copies are started and a `finish()` callable is returned; the records are registered (and
-        the uploads queued) when it is called.  stream: page-locked arrays are shipped on that stream; the event
-        behind each dataset's records is kept in ds._upload_events[key] (the caller's stream must wait for it)."""
+        the uploads queued) when it is called."""
         key = str(device) if tag is None else _mapped_key(device, tag, row_of)
         for ds in datasets:
             if isinstance(ds, DeviceRatingData):
@@ -219,12 +206,8 @@ class RatingData:
         todo = [ds for ds in datasets if key not in ds._records]
         if not todo:
             return (lambda: None) if defer else None
-        evs = [] if stream is not None else None
-        recs, fin = kn.upload_interactions_many([ds._raw for ds in todo], device, row_of, defer=True, stream=stream,
-                                                events=evs, eager=[ds._take_eager(device) for ds in todo])
-        for x, ds in enumerate(todo):
-            if evs is not None and evs[x] is not None:
-                ds.__dict__.setdefault('_upload_events', {})[key] = evs[x]
+        recs, fin = kn.upload_interactions_many([ds._raw for ds in todo], device, row_of, defer=True,
+                                                eager=[ds._take_eager(device) for ds in todo])
 
         def finish():
             fin()
