@@ -333,6 +333,14 @@ int ure_partition_blocks(void);
 int ure_partition_interactions(const double* d_cols, int64_t n, int64_t rs, int64_t cs, double max_rating,
                                const int32_t* d_owner, const uint8_t* d_deleted, int32_t n_map, int n_shards,
                                ure_inter_t* d_out, int32_t* d_hist, int64_t* d_shard_off, void* stream);
+/* ure_partition_interactions that also drops deleted ratings (interaction-level unlearning): a row of user u whose
+ * item int(i) lies in d_del_item[d_del_off[u] .. d_del_off[u+1]) goes with the dropped rows.  d_del_off: int64
+ * [n_map + 1], d_del_item: int32, ascending within each user (duplicates allowed) -- the layout ure_seen_lists builds
+ * from the deleted (user, item) pairs.  Both NULL: exactly ure_partition_interactions. */
+int ure_partition_interactions_del(const double* d_cols, int64_t n, int64_t rs, int64_t cs, double max_rating,
+                                   const int32_t* d_owner, const uint8_t* d_deleted, int32_t n_map, int n_shards,
+                                   const int64_t* d_del_off, const int32_t* d_del_item, ure_inter_t* d_out,
+                                   int32_t* d_hist, int64_t* d_shard_off, void* stream);
 /* out[j] = in[j] with user -> d_row_of[user] (the row inside a compact per-shard user table). */
 int ure_remap_users(const ure_inter_t* d_in, int64_t n, const int32_t* d_row_of, int32_t n_map,
                     ure_inter_t* d_out, void* stream);

@@ -100,6 +100,8 @@ SIGNATURES = {
     "ure_pack_interactions_f64": (C.c_int, [_p, _i64, _i64, _p, _i32, _p, _p]),
     "ure_partition_blocks": (C.c_int, []),
     "ure_partition_interactions": (C.c_int, [_p, _i64, _i64, _i64, _f64, _p, _p, _i32, C.c_int, _p, _p, _p, _p]),
+    "ure_partition_interactions_del": (C.c_int, [_p, _i64, _i64, _i64, _f64, _p, _p, _i32, C.c_int, _p, _p, _p, _p, _p,
+                                                 _p]),
     "ure_remap_users": (C.c_int, [_p, _i64, _p, _i32, _p, _p]),
     "ure_host_stage_copy": (C.c_int, [_p, _p, _i64]),
     "ure_user_segments_scratch_bytes": (_i64, [_i64, C.c_int]),

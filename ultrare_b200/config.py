@@ -4,8 +4,9 @@ Same class names, constructor arguments, attributes, result-directory naming and
 entry points ``Instance.runFull(is_save, verbose)`` / ``Instance.runGroup(is_save,
 learn_type, group_type, n_group, verbose)`` (config.py:182-200).  Defects of the reference
 are resolved as SURVEY.md Appendix A lists (A1 del_per is a percentage, A2 dis_type, A11 the
-embedding path follows the current del_per/del_type with the literal path as fallback,
-A13 del_rating is empty).
+embedding path follows the current del_per/del_type with the literal path as fallback).
+The reference always leaves del_rating empty (Appendix A13); here del_type='inter' fills it with deleted
+(user, item) ratings, which the training reads drop and whose users' shards are retrained.
 """
 from __future__ import annotations
 
@@ -27,6 +28,29 @@ DATASETS = {
     'ml1m': ('/ml1m/squ0_train.csv', '/ml1m/squ0_test.csv', 6040, 3416, 30000),
     'toy': ('/toy/0_train.csv', '/toy/0_test.csv', 1508, 2071, 3000),
 }
+
+
+def draw_rating_deletions(train_dir, del_per):
+    """del_type='inter': int64 [n_del, 2] (user, item) of del_per % of the training file's rows, drawn without
+    replacement under np.random.seed(0), in file order."""
+    import pandas as pd
+    ratings = pd.read_csv(train_dir, header=None, sep=',')
+    n = len(ratings)
+    np.random.seed(0)
+    rows = np.sort(np.random.choice(n, int(del_per / 100 * n), replace=False))
+    return np.stack([ratings[0].values[rows], ratings[1].values[rows]], axis=1).astype(np.int64)
+
+
+def routed_users(del_user, del_rating):
+    """The users whose shards an unlearn pass retrains (config.py:190-193): del_user, then the users of del_rating
+    that it does not hold, in order of first appearance.  Exactly list(del_user) when del_rating is empty."""
+    out = list(del_user)
+    if len(del_rating) == 0:
+        return out
+    users = np.asarray(del_rating)[:, 0]
+    _, first = np.unique(users, return_index=True)
+    new = users[np.sort(first)]
+    return out + new[~np.isin(new, np.asarray(out))].tolist()
 
 
 class InsParam(object):
@@ -61,6 +85,8 @@ class InsParam(object):
                 np.random.seed(0)
                 n_del = int(self.del_per / 100 * self.n_user)      # Appendix A1
                 self.del_user = np.random.choice(self.n_user, n_del, replace=False)
+            elif self.del_type == 'inter':
+                self.del_rating = draw_rating_deletions(self.train_dir, self.del_per)
 
     def info(self):
         print(self.dataset, '-----------')
@@ -187,10 +213,7 @@ class Instance(object):
             model.learn(train_dlist, test_dlist, test_data, verbose, save_dir)
             self.timing['learn_s'] = time.time() - t0
         else:
-            del_user = list(self.param.del_user)
-            for rating in self.param.del_rating:
-                if rating[0] not in del_user:
-                    del_user.append(rating[0])
+            del_user = routed_users(self.param.del_user, self.param.del_rating)
             model.unlearn(model_list, train_dlist, test_dlist, test_data, del_user, verbose, save_dir)
             self.timing['unlearn_s'] = time.time() - t0
         if self.recommend_n > 0:

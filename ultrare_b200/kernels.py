@@ -423,14 +423,57 @@ def upload_table(a: np.ndarray, device) -> torch.Tensor:
     return out
 
 
+def deletion_lists(pairs, n_map: int, device=None):
+    """The per-user deleted-item CSR of ure_partition_interactions_del, built on the device by ure_seen_lists:
+    (off int64 [n_map + 1], items int32 ascending within each user), or None when no pair can match a row.
+    `pairs`: array-like [n, >= 2] of (user, item) ids on the host, or such a CUDA tensor; further columns are ignored
+    and the ids are truncated to integers, as the partition truncates the table's.  Negative ids raise ValueError;
+    pairs whose user lies outside [0, n_map) cannot match a kept row and are dropped.  Host pairs are checked on the
+    host and uploaded once; device pairs are checked on the device (one synchronisation)."""
+    on_dev = isinstance(pairs, torch.Tensor)
+    p = pairs if on_dev else np.asarray(pairs)
+    if len(p) == 0:
+        return None
+    if p.ndim != 2 or p.shape[1] < 2:
+        raise ValueError(f"deletion_lists: pairs must be [n, >= 2], got {tuple(p.shape)}")
+    if on_dev:
+        _need_cuda(p)
+        p = p[:, :2].to(torch.int64)
+    else:
+        p = p[:, :2].astype(np.int64)
+    if bool((p < 0).any()):
+        raise ValueError("deletion_lists: user and item ids must be non-negative")
+    if bool((p[:, 1] >= 2 ** 31).any()):
+        raise ValueError("deletion_lists: item ids must be below 2^31")
+    p = p[p[:, 0] < n_map]
+    if p.shape[0] == 0:
+        return None
+    n_item = int(p[:, 1].max()) + 1
+    if on_dev:
+        rec = torch.zeros((p.shape[0], 4), dtype=torch.int32, device=p.device)
+        rec[:, :2] = p.to(torch.int32)
+    else:
+        rec = np.zeros((p.shape[0], 4), dtype=np.int32)
+        rec[:, :2] = p
+        rec = upload_array(rec, torch.device('cuda' if device is None else device))
+    return seen_lists(rec, int(n_map), n_item)
+
+
 def partition_interactions(table: torch.Tensor, max_rating: float, owner: torch.Tensor,
-                           deleted: Optional[torch.Tensor], n_shards: int, columns: bool = True):
+                           deleted: Optional[torch.Tensor], n_shards: int, columns: bool = True, del_lists=None):
     """readRating's filter + split on the device (ure_partition_interactions).  table: float64 [3,n] (columns=True)
-    or [n,3] (rows of the CSV, columns=False); owner int32 [n_map]; deleted uint8 [n_map] or None.  Returns (records int32 [n,4] whose first
-    shard_off[-1] rows are the shards' runs back to back, shard_off int64 device tensor [n_shards+1])."""
+    or [n,3] (rows of the CSV, columns=False); owner int32 [n_map]; deleted uint8 [n_map] or None; del_lists: the
+    deleted ratings as deletion_lists(pairs, n_map) returns them, or None (ure_partition_interactions_del drops every
+    row whose (user, item) is listed).  Returns (records int32 [n,4] whose first shard_off[-1] rows are the shards'
+    runs back to back, shard_off int64 device tensor [n_shards+1])."""
     _need_cuda(table, owner, deleted)
     assert table.dtype == torch.float64 and table.dim() == 2 and table.is_contiguous()
     assert owner.dtype == torch.int32 and (deleted is None or (deleted.dtype == torch.uint8 and deleted.shape == owner.shape))
+    if del_lists is not None:
+        del_off, del_item = del_lists
+        _need_cuda(del_off, del_item)
+        assert del_off.dtype == torch.int64 and del_off.shape == (owner.shape[0] + 1,) and del_off.is_contiguous()
+        assert del_item.dtype == torch.int32 and del_item.is_contiguous() and del_item.device == table.device
     if columns:
         assert table.shape[0] == 3
         n, rs, cs = table.shape[1], 1, max(1, table.shape[1])
@@ -442,9 +485,15 @@ def partition_interactions(table: torch.Tensor, max_rating: float, owner: torch.
     off = torch.empty(n_shards + 1, dtype=torch.int64, device=table.device)
     hist = torch.empty((L.ure_partition_blocks(), 256), dtype=torch.int32, device=table.device)
     with torch.cuda.device(table.device):
-        check(L.ure_partition_interactions(_ptr(table), n, rs, cs, float(max_rating), _ptr(owner), _ptr(deleted),
-                                           owner.shape[0], n_shards, _ptr(out), _ptr(hist), _ptr(off), _stream()),
-              "ure_partition_interactions")
+        if del_lists is None:
+            check(L.ure_partition_interactions(_ptr(table), n, rs, cs, float(max_rating), _ptr(owner), _ptr(deleted),
+                                               owner.shape[0], n_shards, _ptr(out), _ptr(hist), _ptr(off), _stream()),
+                  "ure_partition_interactions")
+        else:
+            check(L.ure_partition_interactions_del(_ptr(table), n, rs, cs, float(max_rating), _ptr(owner), _ptr(deleted),
+                                                   owner.shape[0], n_shards, _ptr(del_off), _ptr(del_item), _ptr(out),
+                                                   _ptr(hist), _ptr(off), _stream()),
+                  "ure_partition_interactions_del")
     return out, off
 
 

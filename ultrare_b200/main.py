@@ -13,8 +13,8 @@ _FLAGS = {
     'verbose': (int, 1, 'verbose type', (0, 1, 2)),
     'group': (int, 2, 'number of groups', lambda v: v >= 0),
     'learn': (str, 'sisa', 'type of learning and unlearning', ('sisa',)),
-    'delper': (int, 2, 'deleted user proportion', (2, 5)),
-    'deltype': (str, 'rand', 'deletion type', ('rand',)),
+    'delper': (int, 2, 'deleted user (or, with --deltype inter, rating) proportion', (2, 5)),
+    'deltype': (str, 'rand', 'deletion type: rand = users, inter = single ratings', ('rand', 'inter')),
 }
 GROUP_TYPES = ('emb-ot',)                      # the only grouping the reference's CLI reaches (main.py:64)
 

@@ -18,8 +18,33 @@ import torch
 from . import kernels as kn
 
 
+def _pair_keys(del_rating):
+    """Deleted ratings as sorted unique int64 keys (int(user) << 32) | int(item), or None when there are none.
+    del_rating: array-like [n, >= 2] of (user, item, ...); negative ids raise ValueError."""
+    if len(del_rating) == 0:
+        return None
+    p = np.asarray(del_rating)
+    if p.ndim != 2 or p.shape[1] < 2:
+        raise ValueError(f"del_rating must be [n, >= 2] (user, item, ...), got shape {p.shape}")
+    p = p[:, :2].astype(np.int64)
+    if (p < 0).any():
+        raise ValueError("del_rating: user and item ids must be non-negative")
+    if (p >= 2 ** 31).any():
+        raise ValueError("del_rating: user and item ids must be below 2^31")
+    return np.unique((p[:, 0] << 32) | p[:, 1])
+
+
+def _row_keys(ratings):
+    """The keys of _pair_keys for every row of the ratings table (ids truncated to int, as the partition kernel does)."""
+    u = ratings[0].values.astype(np.int64)
+    i = ratings[1].values.astype(np.int64)
+    return (u << 32) | (i & 0xFFFFFFFF)
+
+
 def readRating(dir, n_user, max_rating=5, del_user=[], del_rating=[], n_group=1, group_index=[], sort='r'):
-    """reference read.py:9-70.  Returns (rating_lists [n_group] of float64 [3,n_g], group_index)."""
+    """reference read.py:9-70.  Returns (rating_lists [n_group] of float64 [3,n_g], group_index).
+    del_rating: (user, item) pairs whose rows are dropped (interaction-level unlearning); the group order is that
+    of the unfiltered table."""
     if len(group_index) == 0:
         group_len = int(np.ceil(n_user / n_group))
         org_index = np.arange(n_user).tolist()
@@ -46,6 +71,9 @@ def readRating(dir, n_user, max_rating=5, del_user=[], del_rating=[], n_group=1,
     if len(del_user):
         deleted[np.asarray(list(del_user), dtype=np.int64)] = True
     row_owner = np.where(deleted[users.astype(np.int64)], -1, owner[users.astype(np.int64)])
+    del_keys = _pair_keys(del_rating)
+    if del_keys is not None:
+        row_owner = np.where(np.isin(_row_keys(ratings), del_keys), -1, row_owner)
 
     rating_lists = []
     for g in range(n_group):
@@ -65,6 +93,8 @@ def readRatingDevice(dir, n_user, max_rating=5, del_user=[], del_rating=[], n_gr
     (ure_partition_interactions) then does what read.py:36-68 does with K np.in1d scans.  Returns
     (datasets [n_group] of device-backed ``RatingData`` -- same rows, same row order as readRating's arrays --,
     group_index, total) where ``total`` is the RatingData of all groups back to back (config.py:144-148's hstack).
+    del_rating: (user, item) pairs whose rows the same partition drops (ure_partition_interactions_del, with the
+    per-user deleted-item lists of kernels.deletion_lists).
     """
     if len(group_index) == 0:                 # read.py:13-26, same RNG calls as readRating
         group_len = int(np.ceil(n_user / n_group))
@@ -88,15 +118,18 @@ def readRatingDevice(dir, n_user, max_rating=5, del_user=[], del_rating=[], n_gr
     if len(del_user):
         deleted = np.zeros(n_map, dtype=np.uint8)
         deleted[np.asarray(list(del_user), dtype=np.int64)] = 1
+    del_keys = _pair_keys(del_rating)
     dev = torch.device(device)
+    del_lists = None if del_keys is None else kn.deletion_lists(np.asarray(del_rating), n_map, dev)
     tab = np.empty((3, len(users)), dtype=np.float64)        # one cast pass per column (DataFrame.values would
     for j in range(3):                                       # first consolidate the mixed columns into a copy)
         tab[j] = ratings[j].values
     table = kn.upload_table(tab, dev)
     rec, off = kn.partition_interactions(table, max_rating, kn.upload_array(owner, dev),
-                                         None if deleted is None else kn.upload_array(deleted, dev), n_group)
+                                         None if deleted is None else kn.upload_array(deleted, dev), n_group,
+                                         del_lists=del_lists)
     off_h = off.cpu().numpy()
-    src = (ratings, owner, deleted, float(max_rating))
+    src = (ratings, owner, deleted, float(max_rating), del_keys)
     datasets = [DeviceRatingData(rec[int(off_h[g]):int(off_h[g + 1])], src, (g, g + 1)) for g in range(n_group)]
     total = DeviceRatingData(rec[:int(off_h[n_group])], src, (0, n_group))
     return datasets, group_index, total
@@ -243,7 +276,8 @@ class RatingData:
 class DeviceRatingData(RatingData):
     """RatingData whose records were produced on the device by ``readRatingDevice``.  ``records()`` is the
     partition's output; the host columns (``users``/``items``/``ratings``, ``_raw``) are rebuilt on demand:
-    ids from the records, the float64 ratings by the host filter of readRating (read.py:59-68)."""
+    ids from the records, the float64 ratings by the host filter of readRating (read.py:59-68).  src: (ratings table,
+    owner map, deleted-user flags or None, max_rating[, deleted-rating keys of _pair_keys or None])."""
 
     def __init__(self, records, src, groups):
         self._dev = records
@@ -255,9 +289,12 @@ class DeviceRatingData(RatingData):
     def _rows(self):
         """Indices of this dataset's rows in the source table, in record order (host filter of read.py:59-62)."""
         if 'rows' not in self._cols:
-            ratings, owner, deleted, _ = self._src
+            ratings, owner, deleted = self._src[:3]
             users = ratings[0].values.astype(np.int64)
             own = owner[users] if deleted is None else np.where(deleted[users] != 0, -1, owner[users])
+            del_keys = self._src[4] if len(self._src) > 4 else None
+            if del_keys is not None:
+                own = np.where(np.isin(_row_keys(ratings), del_keys), -1, own)
             lo, hi = self._groups
             parts = [np.flatnonzero(own == g) for g in range(lo, hi)]
             self._cols['rows'] = np.concatenate(parts) if parts else np.zeros(0, dtype=np.int64)
