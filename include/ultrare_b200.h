@@ -396,6 +396,34 @@ int ure_topn(const float* d_P, int n_user, const float* d_S, const float* d_S_lo
 int ure_topn_metrics(const int32_t* d_items, const int32_t* d_users, int64_t m, int top_n, const ure_inter_t* d_test,
                      const int32_t* d_order, const int64_t* d_seg, int n_user, double* d_out, void* stream);
 
+/* ---- Learned combination of the shard models (UltraRE's combination estimator; the reference scores with the plain
+ * mean).  Per owner group g: s(u, i) = b_g + sum_k w_gk x_k with x_k = P[u].Q_k[i] (P the merged user table)
+ * = b_g + P[u].T_g[i], T_g = sum_k w_gk Q_k.  The ridge solve of (w_g, b_g) is (K+1) x (K+1) and runs on the host. */
+#define URE_COMBINE_MAX_MODELS 64
+#define URE_COMBINE_GRAM_CTAS 128   /* CTAs per group of ure_combine_gram: fixed, so the summation order is too */
+
+/* Gram of the features over the records of n_groups groups (d_inter / d_n: device arrays of n_groups record
+ * pointers and row counts), K = n_models item tables d_Q (device array of pointers), P [*, d].  Per group g,
+ * d_out[g * E ..] with E = (K+1)(K+2)/2 + (K+1) + 1, fp64: the upper triangle of sum [x;1][x;1]^T row by row, then
+ * sum [x;1] * r, then the row count.  x_k = sum_t P[u,t] * Q_k[i,t] with the fp32 entries multiplied and summed in
+ * fp64; the sums are fp64 without atomics, folded in a fixed order: two calls give the same bits.  d_scratch: n_groups *
+ * URE_COMBINE_GRAM_CTAS * E doubles.  Ids are not checked.  K > URE_COMBINE_MAX_MODELS or d not in
+ * {8,16,32,64,128}: URE_EUNSUPPORTED. */
+int ure_combine_gram(const float* d_P, const float* const* d_Q, int n_models, int d, const ure_inter_t* const* d_inter,
+                     const int64_t* d_n, int n_groups, double* d_out, double* d_scratch, void* stream);
+
+/* d_T [n_out, n_item, d]: T_o = sum_k d_w[o * n_models + k] * d_Q[k] in k order (t = w_0 q_0, then fma), fp32
+ * weights; the weighted sibling of ure_item_sum.  d a multiple of 4. */
+int ure_item_wsum(const float* const* d_Q, int n_models, const float* d_w, int n_out, int64_t n_item, int d,
+                  float* d_T, void* stream);
+
+/* score[j] = d_b[s] + P[u_j].T_s[i_j] with s = d_owner[u_j], or the last slot n_slots - 1 (the mean combination) when
+ * d_owner[u_j] < 0; d_T [n_slots, n_item, d], d_b fp32 [n_slots].  *d_sse += sum_j (score[j] - r_j)^2 as
+ * ure_ensemble_score (d_score and d_sse may be NULL).  Ids and owner values are not checked. */
+int ure_group_score(const float* d_P, const float* d_T, int n_slots, int64_t n_item, int d, const float* d_b,
+                    const int32_t* d_owner, const ure_inter_t* d_inter, int64_t n, float* d_score, double* d_sse,
+                    void* stream);
+
 /* Affected-shard routing (method/sisa.py:76-81): flags[owner[u]] = 1 for u in del. */
 int ure_route_deletions(const int32_t* d_owner, int32_t n_user, const int32_t* d_del, int32_t n_del,
                         int32_t* d_flags, int32_t n_shards, void* stream);

@@ -13,6 +13,8 @@ LIB_PATH = os.path.join(HERE, "libultrare_b200.so")
 
 URE_MAX_SHARDS = 256
 URE_TOP_K = 10
+URE_COMBINE_MAX_MODELS = 64
+URE_COMBINE_GRAM_CTAS = 128
 
 _p = C.c_void_p
 _i32, _i64, _f32, _f64 = C.c_int32, C.c_int64, C.c_float, C.c_double
@@ -113,6 +115,9 @@ SIGNATURES = {
     "ure_topn_scratch_bytes": (_i64, [_i64, _i64, C.c_int, C.c_int]),
     "ure_topn": (C.c_int, [_p, C.c_int, _p, _p, _i64, C.c_int, _p, _i64, _p, _p, C.c_int, _f32, _p, _p, _p, _p]),
     "ure_topn_metrics": (C.c_int, [_p, _p, _i64, C.c_int, _p, _p, _p, C.c_int, _p, _p]),
+    "ure_combine_gram": (C.c_int, [_p, _p, C.c_int, C.c_int, _p, _p, C.c_int, _p, _p, _p]),
+    "ure_item_wsum": (C.c_int, [_p, C.c_int, _p, C.c_int, _i64, C.c_int, _p, _p]),
+    "ure_group_score": (C.c_int, [_p, _p, C.c_int, _i64, C.c_int, _p, _p, _p, _i64, _p, _p, _p]),
     "ure_route_deletions": (C.c_int, [_p, _i32, _p, _i32, _p, _i32, _p]),
     "ure_merge_user_rows": (C.c_int, [_p, _p, _p, _p, _p, _i32, C.c_int, C.c_int, _p]),
     "ure_cost_matrix": (C.c_int, [_p, _i64, C.c_int, _p, C.c_int, C.c_int, _p, _p, _p]),

@@ -98,6 +98,7 @@ class InsParam(object):
 
 class Instance(object):
     recommend_n = 0          # > 0: every pass also writes top-N recommendations and their metrics (main.py --recommend)
+    combine = 'mean'         # how the SISA passes combine the shard models: 'mean' or 'fit' (Sisa.combine, --combine)
 
     def __init__(self, param):
         self.param = param
@@ -208,6 +209,7 @@ class Instance(object):
 
         save_dir = self._save_dir(is_save, saving_name)
         model = Sisa(self.param, model_type, n_group, train_index)
+        model.combine = self.combine
         t0 = time.time()
         if is_del == False:
             model.learn(train_dlist, test_dlist, test_data, verbose, save_dir)

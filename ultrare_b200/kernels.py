@@ -1627,3 +1627,76 @@ def topn_metrics(items, users, test_inter, n_user: int, seg=None, order=None) ->
                                           _ptr(test_inter.contiguous()), _ptr(order), _ptr(seg), n_user, _ptr(out),
                                           _stream()), "ure_topn_metrics")
     return out
+
+
+# ------------------------------------------------------------------------------ learned combination of shard models
+def combine_gram_entries(K: int) -> int:
+    """Entries of one group's ure_combine_gram output: the upper triangle of the (K+1) x (K+1) Gram, the K+1 moments and
+    the row count."""
+    return (K + 1) * (K + 2) // 2 + (K + 1) + 1
+
+
+def combine_gram(P, Q_list, inters) -> torch.Tensor:
+    """fp64 [n_groups, combine_gram_entries(K)] on the device (ure_combine_gram): per record list of `inters` (int32
+    [n, 4] each, one per group) the Gram of z = [x; 1] with x_k = P[u].Q_k[i], the moments sum z * r and the row count.
+    Deterministic: the same bits on every call."""
+    _need_cuda(P, *Q_list, *inters)
+    dev = P.device
+    K, d = len(Q_list), P.shape[1]
+    E = combine_gram_entries(K)
+    P = P.contiguous()
+    qs = [q.contiguous() for q in Q_list]
+    recs = [r.contiguous() for r in inters]
+    out = torch.empty((len(recs), E), dtype=torch.float64, device=dev)
+    if not recs:
+        return out
+    tab = upload_array(np.asarray([q.data_ptr() for q in qs] + [r.data_ptr() for r in recs] +
+                                  [int(r.shape[0]) for r in recs], dtype=np.int64), dev)
+    scratch = torch.empty(len(recs) * _lib.URE_COMBINE_GRAM_CTAS * E if K <= _lib.URE_COMBINE_MAX_MODELS else 1,
+                          dtype=torch.float64, device=dev)
+    G = len(recs)
+    with torch.cuda.device(dev):
+        check(_lib.lib().ure_combine_gram(_ptr(P), _ptr(tab), K, int(d), C.c_void_p(tab.data_ptr() + 8 * K),
+                                          C.c_void_p(tab.data_ptr() + 8 * (K + G)), G, _ptr(out), _ptr(scratch),
+                                          _stream()), "ure_combine_gram")
+    out._keep = (tab, scratch, qs, recs)
+    return out
+
+
+def item_wsum(Q_list, w) -> torch.Tensor:
+    """T [n_out, n_item, d] with T[o] = sum_k w[o, k] Q_k, in k order (ure_item_wsum); w: fp32 [n_out, K] on the device."""
+    _need_cuda(w, *Q_list)
+    dev = Q_list[0].device
+    n_item, d = Q_list[0].shape
+    K = len(Q_list)
+    w = w.to(device=dev, dtype=torch.float32).contiguous()
+    if w.dim() != 2 or w.shape[1] != K:
+        raise ValueError(f"item_wsum: w must be [n_out, {K}]")
+    T = torch.empty((w.shape[0], n_item, d), dtype=torch.float32, device=dev)
+    qs = [q.contiguous() for q in Q_list]
+    tab = pointer_table(qs, dev)
+    with torch.cuda.device(dev):
+        check(_lib.lib().ure_item_wsum(_ptr(tab), K, _ptr(w), int(w.shape[0]), n_item, d, _ptr(T), _stream()),
+              "ure_item_wsum")
+    T._keep = (tab, qs, w)
+    return T
+
+
+def group_score(P, T, b, owner, inter, sse=None):
+    """(score fp32 [n], sse fp64 [1]) of ure_group_score: score = b[s] + P[u].T[s][i] with s = owner[u], or the last
+    slot of T (the mean combination) for users in no group.  T: fp32 [n_slots, n_item, d]; b: fp32 [n_slots];
+    owner: int32 [n_user].  sse: a zeroed fp64 [1] to add into."""
+    _need_cuda(P, T, b, owner, inter, sse)
+    dev = inter.device
+    n = inter.shape[0]
+    score = torch.empty(n, dtype=torch.float32, device=dev)
+    if sse is None:
+        sse = torch.zeros(1, dtype=torch.float64, device=dev)
+    if T.dim() != 3 or b.shape != (T.shape[0],) or P.shape[1] != T.shape[2]:
+        raise ValueError("group_score: T must be [n_slots, n_item, d] with b [n_slots] and P [n_user, d]")
+    with torch.cuda.device(dev):
+        check(_lib.lib().ure_group_score(_ptr(P.contiguous()), _ptr(T.contiguous()), int(T.shape[0]), int(T.shape[1]),
+                                         int(T.shape[2]), _ptr(b.contiguous()), _ptr(owner.contiguous()),
+                                         _ptr(inter.contiguous()), n, _ptr(score), _ptr(sse), _stream()),
+              "ure_group_score")
+    return score, sse

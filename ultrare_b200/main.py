@@ -31,6 +31,10 @@ def _build_parser():
                    help='per-epoch in-training evaluation fidelity of the SISA path')
     p.add_argument('--recommend', type=int, default=0, metavar='N',
                    help='also write every pass\'s top-N recommendations (rec{N}*.npy, seen items excluded); 0 = off')
+    p.add_argument('--combine', default='mean', choices=['mean', 'fit'],
+                   help='how the SISA shard models are combined for the final evaluation and the recommendations: '
+                        'mean = the reference\'s plain mean, fit = a per-group least-squares combination refitted '
+                        'on the retained data after every unlearn (combine.npy)')
     return p
 
 
@@ -59,6 +63,7 @@ def main(argv=None):
         synth.ensure_dataset(a.dataset)
     ins = Instance(InsParam(a.dataset, a.epoch, a.worker, a.layer, a.group, a.delper, a.deltype))
     ins.recommend_n = a.recommend
+    ins.combine = a.combine
     if a.group == 0:
         ins.runFull(is_save=True, verbose=a.verbose)
         return ins

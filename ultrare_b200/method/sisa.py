@@ -38,7 +38,8 @@ from torch import nn
 from .. import dist as udist
 from .. import kernels as kn
 from .scratch import Scratch
-from .utils import _request_users, baseTest, base_test_device, base_test_values, recommend_from_tables
+from .utils import (_request_users, baseTest, base_test_device, base_test_values, fit_combination, recommend_combined,
+                    recommend_from_tables)
 
 
 class _Table:
@@ -148,6 +149,11 @@ class Sisa(Scratch):
         self._group_rows = {}
         self.retrain_gid = set()
         self.timing = {}
+        # how the final evaluation and recommend combine the shard models: 'mean' = the reference's (1/K) sum_k
+        # P[u].Q_k[i]; 'fit' = the learned per-owner-group combination (utils.fit_combination), refitted on the
+        # retained training rows after every learn / unlearn pass
+        self.combine = 'mean'
+        self.combination = None
 
     def _mode(self):
         if self.dist.world > 1 and self.epoch_eval == 'faithful':
@@ -162,7 +168,10 @@ class Sisa(Scratch):
     # ------------------------------------------------------------------ evaluation
     def test(self, test_data, verbose, save_dir):
         """reference sisa.py:18-23."""
-        rmse, ndcg, hr = self._ensemble_test(test_data, verbose)
+        if self._use_fit():
+            rmse, ndcg, hr = self._combined_test(test_data, verbose)
+        else:
+            rmse, ndcg, hr = self._ensemble_test(test_data, verbose)
         log = {'total_rmse': rmse, 'total_ndcg': ndcg, 'total_hr': hr}
         if len(save_dir) > 0 and self.dist.rank == 0:
             np.save(save_dir + '/log0', log)
@@ -202,7 +211,12 @@ class Sisa(Scratch):
         result is the same bit for bit on one GPU and on several.  With several GPUs each rank recommends for the
         requested users whose owner shard it holds (users in no group: rank 0), because it holds those shards' training
         records, and the rows, placed by request position into zero-filled outputs, are all-reduced (every row has one
-        non-zero contribution, so the sum is exact)."""
+        non-zero contribution, so the sum is exact).
+
+        combine == 'fit': the lists of the fitted combination (utils.recommend_combined), one top-N call per owner group
+        with that group's T_g; on several GPUs the same placement by owner shard and the same exact all-reduce."""
+        if self._use_fit():
+            return self._recommend_combined(users, top_n, exclude)
         qsum = self._item_sum_in_shard_order()
         P = self.model_list[0].user_mat.weight.data
         u = _request_users(users, self.n_user, self.device)
@@ -217,6 +231,97 @@ class Sisa(Scratch):
             it, sc = recommend_from_tables(P, qsum, self.n_group, u[pos], top_n, exclude)
             items[pos] = it
             scores[pos] = sc
+        self.dist.all_reduce(items)
+        self.dist.all_reduce(scores)
+        return items, scores
+
+    # ------------------------------------------------------------------ learned combination (combine == 'fit')
+    def _use_fit(self):
+        """True when the evaluation and recommend use the fitted combination; combine must be 'mean' or 'fit'."""
+        if self.combine not in ('mean', 'fit'):
+            raise ValueError(f"Sisa.combine must be 'mean' or 'fit', not {self.combine!r}")
+        return self.combine == 'fit'
+
+    def _fitted(self):
+        """The combination the last learn / unlearn pass fitted, or a clear error when it did not fit one."""
+        if self.combination is None:
+            raise RuntimeError("Sisa.combine == 'fit' but no combination has been fitted: run learn or unlearn with "
+                               "combine='fit' first")
+        return self.combination
+
+    def _item_tables_in_shard_order(self):
+        """[Q_0 .. Q_{K-1}] on this GPU.  On several GPUs the ranks all-gather their item tables chunk by chunk of item
+        rows, as _item_sum_in_shard_order does, into one [K, n_item, d] buffer: every rank then holds the same bits."""
+        K, world, rank = self.n_group, self.dist.world, self.dist.rank
+        if world == 1:
+            return [self.model_list[s].item_mat.weight.data for s in range(K)]
+        slots = -(-K // world)
+        rows = max(1, min(self.n_item, self.RECOMMEND_GATHER_BYTES // (world * slots * self.k * 4)))
+        part = torch.zeros((slots, rows, self.k), dtype=torch.float32, device=self.device)
+        full = torch.empty((world * slots, rows, self.k), dtype=torch.float32, device=self.device)
+        Q = torch.empty((K, self.n_item, self.k), dtype=torch.float32, device=self.device)
+        mine = list(range(rank, K, world))
+        for r0 in range(0, self.n_item, rows):
+            n = min(self.n_item, r0 + rows) - r0
+            for j, s in enumerate(mine):
+                part[j, :n].copy_(self.model_list[s].item_mat.weight.data[r0:r0 + n])
+            self.dist.all_gather_into(full, part)
+            for s in range(K):
+                Q[s, r0:r0 + n].copy_(full[(s % world) * slots + s // world, :n])
+        return list(Q)
+
+    def _fit_combination(self, train_dlist, save_dir):
+        """Fit the combination of every owner group on this pass's training rows (after an unlearn: the retained rows
+        only) -- every group, because retrained shards change every group's features.  Every rank fits every group
+        from the same gathered tables, so all ranks hold the same weights.  combine.npy: fp64 [K, K + 1], (w_g, b_g)."""
+        recs = [train_dlist[g].dataset.records(self.device) for g in range(self.n_group)]
+        self.combination = fit_combination(self.model_list[0].user_mat.weight.data, self._item_tables_in_shard_order(),
+                                           recs)
+        if len(save_dir) > 0 and self.dist.rank == 0:
+            np.save(save_dir + '/combine', self.combination.table())
+
+    def _combined_test(self, test_data, verbose):
+        """The final evaluation under the fitted combination: ure_group_score, then ure_rank_metrics.  On several GPUs
+        with the per-shard test sets partitioning test_data (as in _ensemble_test_sharded), every rank scores the test
+        rows of the groups whose owner shard it holds and the sums are all-reduced; otherwise every rank evaluates the
+        whole test set."""
+        dev, K, c = self.device, self.n_group, self._fitted()
+        P = self.model_list[0].user_mat.weight.data
+        tdl = getattr(self, '_test_dlist', None)
+        sharded = self.dist.world > 1 and self.eval_sharded is not False and tdl is not None and len(tdl) == K and \
+            sum(len(t.dataset) for t in tdl) == len(test_data.dataset)
+        out = torch.zeros(5, dtype=torch.float64, device=dev)
+        if sharded:
+            recs = [tdl[i].dataset.records(dev) for i in self.dist.my_shards(range(K)) if len(tdl[i].dataset) > 0]
+            rows = _eval_rows(recs, self.n_user) if recs else None
+        else:
+            ds = test_data.dataset
+            rows = (ds.records(dev),) + tuple(ds.segments(dev, self.n_user)) if len(ds) > 0 else None
+        if rows is not None:
+            inter, order, seg = rows
+            score, _ = kn.group_score(P, c.T, c.b_slot, self._owner, inter, sse=out[0:1])
+            kn.rank_metrics(inter, score, seg, order, out=out[1:4])
+        if sharded:
+            sb = getattr(self, '_last_batch', None)
+            if sb is not None and getattr(sb, 'optimistic', False):
+                out[4:5].copy_(sb.ws[16:20].view(torch.int32))     # as in _ensemble_test_sharded
+            self.dist.all_reduce(out)
+        vals = kn.download_many([out])[0]
+        if vals[4] > 0:
+            raise kn.PlanHintMiss("ultrare_b200: a rank's remembered owner plan did not cover its batch")
+        rmse, ndcg, hr = base_test_values(vals[:4], len(test_data.dataset))
+        if verbose == 2:
+            print(f'Test - RMSE: {rmse:>.4f}, NDCG: {ndcg:>.3f}, HR: {hr:>.3f}')
+        return rmse, ndcg, hr
+
+    def _recommend_combined(self, users, top_n, exclude):
+        P = self.model_list[0].user_mat.weight.data
+        u = _request_users(users, self.n_user, self.device)
+        if self.dist.world == 1:
+            return recommend_combined(P, self._fitted(), self._owner, u, top_n, exclude)
+        owner = self._owner[u.long()]
+        keep = torch.where(owner >= 0, owner % self.dist.world, torch.zeros_like(owner)) == self.dist.rank
+        items, scores = recommend_combined(P, self._fitted(), self._owner, u, top_n, exclude, keep=keep)
         self.dist.all_reduce(items)
         self.dist.all_reduce(scores)
         return items, scores
@@ -613,6 +718,10 @@ class Sisa(Scratch):
         self._finish(new, unmerged, last_idx, compact, merged, test_dlist, save_dir)
         shared = next(iter(new.values())).user_mat.weight if new else nn.Parameter(merged, requires_grad=False)
         self.model_list = [new[i] if i in new else _RemoteModel(shared) for i in range(self.n_group)]
+        if self._use_fit():
+            t_c = time.perf_counter()
+            self._fit_combination(train_dlist, save_dir)
+            self.timing['combine_fit_ms'] = (time.perf_counter() - t_c) * 1e3
         self.test(test_data, verbose, save_dir)
         self._flush_logs()
         self._join_writers()
@@ -676,11 +785,18 @@ class Sisa(Scratch):
         shared = next(iter(new.values())).user_mat.weight if new else nn.Parameter(merged, requires_grad=False)
         for m in self.model_list:
             m.user_mat.weight = shared
+        t_c = time.perf_counter()
+        fit = self._use_fit()
+        if fit:
+            self._fit_combination(train_dlist, save_dir)
+            self.timing['combine_fit_ms'] = (time.perf_counter() - t_c) * 1e3
         t_t = time.perf_counter()
         self.test(test_data, verbose, save_dir)
-        self.timing['merge_ms'] = (t_t - t_m) * 1e3
-        # kernels of ours outside the training batch: route (large deletion sets only), merge, score, ranking
-        self.timing['own_launches_outside_batch'] = (0 if self._route_flags_host is not None else 1) + 1 + 2
+        self.timing['merge_ms'] = (t_c - t_m) * 1e3
+        # kernels of ours outside the training batch: route (large deletion sets only), merge, score, ranking; with the
+        # fitted combination also the Gram, its fold and the weighted item sum
+        self.timing['own_launches_outside_batch'] = (0 if self._route_flags_host is not None else 1) + 1 + 2 + \
+            (3 if fit else 0)
         self._flush_logs()
         self._join_writers()
         self.timing['test_ms'] = (time.perf_counter() - t_t) * 1e3

@@ -247,6 +247,91 @@ def recommend(models, users=None, top_n=10, exclude=None):
     return recommend_from_tables(P, S, len(models), users, top_n, exclude)
 
 
+COMBINE_RIDGE = 1e-6     # lambda_g = COMBINE_RIDGE * tr(X_g^T X_g) / K: keeps the solve regular, the intercept free
+
+
+class Combination:
+    """A fitted combination of K shard models: per owner group g, s(u, i) = b[g] + sum_k w[g, k] P[u].Q_k[i].
+
+    w fp64 [K, K], b fp64 [K] (host); T fp32 [K + 1, n_item, d] and b_slot fp32 [K + 1] on the device, where
+    T[g] = sum_k w[g, k] Q_k and the last slot is the mean combination (w = 1/K, b = 0) that scores users in no group;
+    gram: the fp64 kernel output the fit was solved from."""
+
+    def __init__(self, w, b, T, b_slot, gram):
+        self.w, self.b, self.T, self.b_slot, self.gram = w, b, T, b_slot, gram
+
+    def table(self):
+        """fp64 [K, K + 1]: row g = (w_g, b_g), the layout of combine.npy."""
+        return np.concatenate([self.w, self.b[:, None]], axis=1)
+
+
+def solve_combination(gram, K):
+    """(w fp64 [n_groups, K], b fp64 [n_groups]) from ure_combine_gram's rows: per group the ridge least squares
+    min sum (b + w.x - r)^2 + lambda ||w||^2, lambda = COMBINE_RIDGE * tr(X^T X) / K, the intercept not penalised,
+    solved in float64 from the (K+1) x (K+1) normal equations.  A group without rows gets the mean (w = 1/K, b = 0)."""
+    gram = np.asarray(gram, dtype=np.float64).reshape(-1, kn.combine_gram_entries(K))
+    iu = np.triu_indices(K + 1)
+    U = len(iu[0])
+    w = np.full((gram.shape[0], K), 1.0 / K)
+    b = np.zeros(gram.shape[0])
+    for g, row in enumerate(gram):
+        if row[-1] == 0:
+            continue
+        A = np.zeros((K + 1, K + 1))
+        A[iu] = row[:U]
+        A = A + np.triu(A, 1).T
+        lam = COMBINE_RIDGE * np.trace(A[:K, :K]) / K
+        A[np.arange(K), np.arange(K)] += lam
+        m = row[U:U + K + 1]
+        try:
+            th = np.linalg.solve(A, m)
+        except np.linalg.LinAlgError:        # all features zero: no ridge either; the minimum-norm solution
+            th = np.linalg.lstsq(A, m, rcond=None)[0]
+        w[g], b[g] = th[:K], th[K]
+    return w, b
+
+
+def fit_combination(P, Q_list, inters):
+    """Fit the per-group combination of the models (P, Q_k), k < K, on the training records of every owner group
+    (inters[g]: int32 [n, 4] device records, one per group, g < K; after an unlearn, the retained rows).  The Gram
+    comes from ure_combine_gram, the ridge solve and the fallbacks are solve_combination's, T from ure_item_wsum."""
+    K = len(Q_list)
+    if len(inters) != K:
+        raise ValueError(f"fit_combination: {len(inters)} record lists for {K} models (one per owner group)")
+    gram = kn.combine_gram(P, Q_list, inters)
+    gram_h = kn.download_many([gram])[0]
+    w, b = solve_combination(gram_h, K)
+    W = np.concatenate([w, np.full((1, K), 1.0 / K)]).astype(np.float32)
+    T = kn.item_wsum(Q_list, kn.upload_array(W, P.device))
+    b_slot = kn.upload_array(np.append(b, 0.0).astype(np.float32), P.device)
+    return Combination(w, b, T, b_slot, gram_h)
+
+
+def recommend_combined(P, comb, owner, users, top_n=10, exclude=None, keep=None):
+    """Top-N lists under a fitted Combination: (items int32 [m, top_n], scores fp32 [m, top_n]).  One ure_topn call per
+    owner group among the requested users (T[g], scale 1), b[g] added to the returned scores but not to the -inf
+    padding; users in no group use the mean slot.  The seen lists are built once.  keep: bool [m] device mask of the
+    rows to compute; the other rows stay zero (several GPUs: each rank fills the rows of the groups it holds)."""
+    dev = P.device
+    u = _request_users(users, P.shape[0], dev)
+    recs = _exclude_records(exclude, dev)
+    seen = kn.seen_lists(recs, P.shape[0], comb.T.shape[1]) if recs is not None else None
+    mean_slot = comb.T.shape[0] - 1
+    o = owner[u.long()]
+    slot = torch.where(o >= 0, o, torch.full_like(o, mean_slot))
+    if keep is not None:
+        slot = torch.where(keep, slot, torch.full_like(slot, -1))
+    slot_h = slot.cpu().numpy()
+    items = torch.zeros((u.shape[0], top_n), dtype=torch.int32, device=dev)
+    scores = torch.zeros((u.shape[0], top_n), dtype=torch.float32, device=dev)
+    for g in np.unique(slot_h[slot_h >= 0]).tolist():
+        pos = torch.from_numpy(np.flatnonzero(slot_h == g)).to(dev)
+        it, sc = kn.recommend_topn(P, comb.T[g], u[pos], top_n, 1.0, seen)
+        items[pos] = it
+        scores[pos] = torch.where(it >= 0, sc + comb.b_slot[g], sc)
+    return items, scores
+
+
 def topn_metrics(items, users, test_data, top_n):
     """Full-catalogue HR@N / Recall@N / NDCG@N of top-N lists (``recommend``'s items for ``users``; None = every user,
     row u for user u) against ``test_data`` (dataset, DataLoader or records tensor): relevant items are a user's
