@@ -515,6 +515,34 @@ int64_t ure_balance_workspace_bytes(int k);
 int ure_balance_labels(const float* d_M, int64_t n, int k, int kpad, int32_t* d_label, int64_t* d_cnt,
                        int max_aug, void* d_workspace, void* stream);
 
+/* ---- 'rating-ot' grouping: the points are the users' sparse rating rows (reference group.py, readSparseMat) ---- */
+#define URE_SPARSE_OT_MAX_K 128   /* centroids of the sparse kernels: the balanced rounding's limit */
+
+/* The cost matrix of ure_cost_matrix -- [n, kpad] row major, columns j >= k +inf, d_inertia (may be NULL)
+ * += sum_i max(min_j M[i,j], 0) -- for sparse rows: M[i,j] = ||x_i||^2 - 2 x_i.c_j + ||c_j||^2.
+ * x_i: the ratings of user i in CSR, entries d_off[i] .. d_off[i+1] (int64 [n + 1]) of d_item (int32, ascending within
+ * a row; adjacent duplicates stand for their fp32 sum, the entry of SciPy's summed row) and d_val (fp32).
+ * d_Ct: the centroids item-major, fp32 [n_item, kpad], columns j >= k zero; d_cnorm: fp64 [k] = ||c_j||^2.  The dot
+ * products and ||x_i||^2 multiply fp32 values and add them in fp64; each cost is rounded to fp32 once.  The inertia is
+ * added in a fixed order (the same bits on every call).  1 <= k <= URE_SPARSE_OT_MAX_K and kpad = the smallest of
+ * 8, 16, .., 128 that holds k (else URE_EUNSUPPORTED).  d_scratch: ure_sparse_cost_scratch_bytes(n) bytes (only read
+ * with d_inertia).  Item ids are not checked. */
+int64_t ure_sparse_cost_scratch_bytes(int64_t n);
+int ure_sparse_cost(const int64_t* d_off, const int32_t* d_item, const float* d_val, int64_t n, const float* d_Ct,
+                    const double* d_cnorm, int k, int kpad, float* d_M, double* d_inertia, void* d_scratch,
+                    void* stream);
+
+/* Centroid sums of the sparse rows for given labels: the ratings in CSC, entries d_off[t] .. d_off[t+1] (int64
+ * [n_item + 1]) of d_user (int32, ascending within a column; the fp32 sum of adjacent duplicates is the entry, as in
+ * ure_sparse_cost) and d_val (fp32) for item t.  d_sum fp64 [n_item, kpad] = per item the sum of its
+ * ratings by label d_label[user] (every entry written, 0 where there is none), each added in the column's order without
+ * floating-point atomics: two calls give the same bits.  d_cnt int64 [k] = the users per label (set, not added).
+ * k, kpad as ure_sparse_cost.  User ids and labels are not checked (a label outside [0, k) is neither summed nor
+ * counted). */
+int ure_sparse_centroid_sums(const int64_t* d_off, const int32_t* d_user, const float* d_val, int64_t n_item,
+                             const int32_t* d_label, int64_t n_user, int k, int kpad, double* d_sum, int64_t* d_cnt,
+                             void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -15,6 +15,7 @@ URE_MAX_SHARDS = 256
 URE_TOP_K = 10
 URE_COMBINE_MAX_MODELS = 64
 URE_COMBINE_GRAM_CTAS = 128
+URE_SPARSE_OT_MAX_K = 128
 
 _p = C.c_void_p
 _i32, _i64, _f32, _f64 = C.c_int32, C.c_int64, C.c_float, C.c_double
@@ -136,6 +137,9 @@ SIGNATURES = {
     "ure_centroid_sums": (C.c_int, [_p, _i64, C.c_int, _p, C.c_int, _p, _p, _p]),
     "ure_balance_workspace_bytes": (_i64, [C.c_int]),
     "ure_balance_labels": (C.c_int, [_p, _i64, C.c_int, C.c_int, _p, _p, C.c_int, _p, _p]),
+    "ure_sparse_cost_scratch_bytes": (_i64, [_i64]),
+    "ure_sparse_cost": (C.c_int, [_p, _p, _p, _i64, _p, _p, C.c_int, C.c_int, _p, _p, _p, _p]),
+    "ure_sparse_centroid_sums": (C.c_int, [_p, _p, _p, _i64, _p, _i64, C.c_int, C.c_int, _p, _p, _p]),
 }
 
 _lib = None

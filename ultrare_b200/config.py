@@ -21,7 +21,7 @@ from .group import DATA_DIR, SAVE_DIR, Group
 from .method.scratch import Scratch
 from .method.sisa import Sisa
 from .method.utils import recommend, saveObject, topn_metrics
-from .read import RatingData, loadData, readRating, readRatingDevice
+from .read import RatingData, loadData, readRating, readRatingDevice, readSparseMat
 
 DATASETS = {
     # name: (train file, test file, n_user, n_item, batch)   reference config.py:26,40-44
@@ -174,6 +174,8 @@ class Instance(object):
 
     def _group_index(self, group_type, n_group):
         """The user grouping of config.py:126-134: [] for 'uniform' (readRating draws it), else Group.grouping.
+        'emb-ot' clusters the user table of a `--group 0` run (user_mat0.npy); 'rating-ot' clusters the users' rows of
+        the whole training file (readSparseMat, config.py:130) and needs no earlier run.
         One process per GPU (torchrun): rank 0 alone computes (or loads) the grouping and writes the cache file;
         every rank then holds the SAME group_index -- the centroid sums are order-dependent fp64 atomics, so two
         ranks clustering on their own could end with different labels and different owner maps."""
@@ -184,10 +186,14 @@ class Instance(object):
         t0 = time.time()
         group_index = None
         if d.rank == 0:
-            user_mat = np.load(self._user_mat_path(), allow_pickle=True)
-            shape = type('Shape', (), {'shape': (self.param.n_user, self.param.n_item)})()   # readSparseMat: shapes only
-            group_index = Group(shape, self.param.dataset, user_mat).grouping(self.param.dataset, n_group,
-                                                                               group_type, verbose=False)
+            if group_type.startswith('rating'):
+                X = readSparseMat(self.param.train_dir, self.param.n_user, self.param.n_item, self.param.max_rating)
+                grp = Group(X, self.param.dataset)
+            else:
+                user_mat = np.load(self._user_mat_path(), allow_pickle=True)
+                shape = type('Shape', (), {'shape': (self.param.n_user, self.param.n_item)})()   # shapes only
+                grp = Group(shape, self.param.dataset, user_mat)
+            group_index = grp.grouping(self.param.dataset, n_group, group_type, verbose=False)
         group_index = d.broadcast_object(group_index, src=0)
         self.timing['grouping_s'] = time.time() - t0
         return group_index

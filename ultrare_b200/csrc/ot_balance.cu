@@ -45,6 +45,7 @@ balance_kernel(const float* __restrict__ M, long long n, int k, int kpad, int32_
   unsigned long long* const s_dist = s_W + k * k;                                          // [k] (ord(dist), pred)
   int* const s_size = reinterpret_cast<int*>(s_dist + k);                                  // [k]
   int* const s_path = s_size + k;                                                          // [2*k] (user, new label)
+  int* const s_par = s_path + 2 * k;                                                       // [k] predecessors (fallback)
   __shared__ int s_ctl[4];                 // [0] phase (0 done, 1 shed surplus, 2 fill deficit), [1] path edges, [2] changed
   const int tid = threadIdx.x;
   const bool multi = gridDim.x > 1;
@@ -91,7 +92,7 @@ balance_kernel(const float* __restrict__ M, long long n, int k, int kpad, int32_
       for (int p = tid; p < k * k; p += kBalThreads) s_W[p] = __ldcg(&W[p]);
       __syncthreads();
     }
-    // ---- Bellman-Ford from every source at once (edges may be negative; there is no negative cycle)
+    // ---- Bellman-Ford from every source at once (edges may be negative; a negative cycle only from fp32 rounding)
     for (int j = tid; j < k; j += kBalThreads) {
       const bool src = phase == 1 ? s_size[j] > hi : s_size[j] > lo;
       s_dist[j] = src ? (((unsigned long long)ord_f32(0.f) << 32) | 0xFFFFu) : kNone;
@@ -136,13 +137,75 @@ balance_kernel(const float* __restrict__ M, long long n, int k, int kpad, int32_
         while (true) {
           const int j = (int)(s_dist[l] & 0xFFFFu);
           if (j == 0xFFFF) break;                                   // reached a source
-          if (edges >= k) { ok = false; break; }                    // a cycle (rounding): give up
+          if (edges >= k) { ok = false; break; }                    // the predecessors loop
           s_path[2 * edges] = (int)(s_W[j * k + l] & 0xFFFFFFFFu);
           s_path[2 * edges + 1] = l;
           ++edges;
           l = j;
         }
         if (ok) { s_size[l] -= 1; s_size[sink] += 1; }
+      }
+      // Exact and near ties -- a sparse rating row that shares no item with any centroid costs ||x||^2 + ||c_j||^2, and
+      // thousands of users have the same cost differences up to the rounding of their row -- defeat the pass above in
+      // three ways: the equal-distance rule closes the predecessors of a zero-weight cycle into a loop, fp32 distances
+      // creep down around such a cycle until the round limit, and the rounding can make a swap of two tied users look an
+      // ulp cheaper (a true negative cycle of the fp32 deltas).  Then this thread runs a strict Bellman-Ford from the
+      // sources, the edge weights added in fp64 and only shorter distances replacing: a relaxation in round k + 1 means
+      // a negative cycle, and one user moves along it (sizes unchanged, cost lower); otherwise the path to the cheapest
+      // sink is a simple shortest path.  Where the pass above succeeds none of this runs.
+      if (!ok && (sink >= 0 || rounds > k + 1)) {
+        double* const d = reinterpret_cast<double*>(s_dist);      // s_dist is not read again in this round
+        for (int j = 0; j < k; ++j) {
+          const bool src = phase == 1 ? s_size[j] > hi : s_size[j] > lo;
+          d[j] = src ? 0.0 : INFINITY;
+          s_par[j] = -1;
+        }
+        int x = -1;
+        for (int r = 0; r <= k; ++r) {
+          x = -1;
+          for (int j = 0; j < k; ++j) {
+            if (d[j] == INFINITY) continue;
+            for (int l = 0; l < k; ++l) {
+              const unsigned long long w = s_W[j * k + l];
+              if (l == j || w == kNone) continue;
+              const double c = d[j] + (double)unord_f32((unsigned)(w >> 32));
+              if (c < d[l]) { d[l] = c; s_par[l] = j; x = l; }
+            }
+          }
+          if (x < 0) break;
+        }
+        if (x >= 0) {
+          for (int t = 0; t < k; ++t) x = s_par[x];                 // onto the negative cycle
+          int l = x;
+          edges = 0;
+          do {
+            const int j = s_par[l];
+            s_path[2 * edges] = (int)(s_W[j * k + l] & 0xFFFFFFFFu);
+            s_path[2 * edges + 1] = l;
+            ++edges;
+            l = j;
+          } while (l != x && edges <= k);
+          ok = l == x;
+        } else {
+          int snk = -1;
+          for (int j = 0; j < k; ++j) {
+            const bool sj = phase == 1 ? s_size[j] < hi : s_size[j] < lo;
+            const bool src = phase == 1 ? s_size[j] > hi : s_size[j] > lo;
+            if (sj && !src && d[j] < INFINITY && (snk < 0 || d[j] < d[snk])) snk = j;
+          }
+          if (snk >= 0) {
+            int l = snk;
+            edges = 0;
+            while (s_par[l] >= 0 && edges < k) {
+              const int j = s_par[l];
+              s_path[2 * edges] = (int)(s_W[j * k + l] & 0xFFFFFFFFu);
+              s_path[2 * edges + 1] = l;
+              ++edges;
+              l = j;
+            }
+            if (s_par[l] < 0) { s_size[l] -= 1; s_size[snk] += 1; ok = true; }
+          }
+        }
       }
       s_ctl[1] = ok ? edges : -1;
     }
@@ -184,7 +247,7 @@ extern "C" int ure_balance_labels(const float* d_M, int64_t n, int k, int kpad, 
   if (k == 1) return 0;
   long long grid = (n + 8191) / 8192;
   if (grid > num_sms()) grid = num_sms();
-  const size_t smem = (size_t)k * k * 8 + (size_t)k * 8 + (size_t)k * 4 + (size_t)k * 8 + 64;
+  const size_t smem = (size_t)k * k * 8 + (size_t)k * 8 + (size_t)k * 4 + (size_t)k * 12 + 64;
   URE_CUDA(cudaFuncSetAttribute(balance_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   long long nn = n;
   auto* cntp = reinterpret_cast<long long*>(d_cnt);

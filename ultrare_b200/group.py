@@ -23,7 +23,7 @@ SAVE_DIR = abspath(join(_ROOT, 'result'))    # reference group.py:10
 
 class Group(object):
     def __init__(self, rating, dataset, user_mat=None):
-        self.rating = rating                   # csr_matrix or anything with .shape (only shapes are used)
+        self.rating = rating                   # csr_matrix ('rating-ot') or anything with .shape ('emb-ot')
         self.dataset = dataset
         self.user_mat = user_mat
         self.n_user = self.rating.shape[0]
@@ -39,12 +39,12 @@ class Group(object):
         trans_var, cluster_var = var.strip().split('-')
         assert cluster_var == 'ot', "only '<x>-ot' grouping is reachable from main.py (main.py:64)"
         if trans_var == 'emb':
-            embedding = self.user_mat
+            points = np.asarray(self.user_mat, dtype=np.float32)
         elif trans_var == 'rating':
-            embedding = np.asarray(self.rating.todense(), dtype=np.float32)
+            points = self.rating                 # the sparse rating rows, clustered without densifying
         else:
             raise ValueError(var)
-        _, label = ot_cluster(np.asarray(embedding, dtype=np.float32), n_group)   # Appendix A3
+        _, label = ot_cluster(points, n_group)                                   # Appendix A3
 
         if verbose == True:
             print(''.join(f'{i}: {int((label == i).sum())}, ' for i in range(n_group)))

@@ -1537,6 +1537,65 @@ def balance_labels(M, k, label, cnt, max_aug: int = 1 << 14):
     return ws[128:140].view(torch.int32)
 
 
+# ------------------------------------------------------------------------------ OT grouping of sparse rows ('rating-ot')
+def sparse_orders(rec: torch.Tensor, n_user: int, n_item: int):
+    """The nonzeros of a sparse [n_user, n_item] matrix in the two orders of the sparse OT kernels, built on the device
+    by the stable radix sort of ure_user_segments (by user, then by item, then by user): (csr, csc) with csr = (off
+    int64 [n_user + 1], item int32, val fp32), a user's items ascending, and csc = (off int64 [n_item + 1], user int32,
+    val fp32), an item's users ascending -- in both, duplicate (user, item) entries are adjacent, in record order.
+    rec: int32 [nnz, 4] device records (user, item, fp32 value bits, any); ids outside [0, n_user) / [0, n_item), or no
+    record at all, raise ValueError (one synchronisation)."""
+    _need_cuda(rec)
+    assert rec.dtype == torch.int32 and rec.dim() == 2 and rec.shape[1] == 4
+    if rec.shape[0] == 0:
+        raise ValueError("sparse_orders: the matrix has no nonzero")
+    u, i = rec[:, 0], rec[:, 1]
+    if bool(((u < 0) | (u >= n_user) | (i < 0) | (i >= n_item)).any()):
+        raise ValueError(f"sparse_orders: user ids must lie in [0, {n_user}) and item ids in [0, {n_item})")
+    rec = rec.contiguous()
+    by_user = rec.index_select(0, user_segments_device(rec, int(n_user))[0].long())
+    ord_c, off_c = user_segments_device(by_user[:, [1, 0, 2, 3]].contiguous(), int(n_item))
+    by_item = by_user.index_select(0, ord_c.long())
+    ord_r, off_r = user_segments_device(by_item, int(n_user))
+    by_user = by_item.index_select(0, ord_r.long())
+    csr = (off_r, by_user[:, 1].contiguous(), by_user[:, 2].contiguous().view(torch.float32))
+    csc = (off_c, by_item[:, 0].contiguous(), by_item[:, 2].contiguous().view(torch.float32))
+    return csr, csc
+
+
+def sparse_cost(csr, Ct, cnorm, k: int, want_inertia=False):
+    """M [n, kpad] fp32 of ure_sparse_cost (columns >= k are +inf) and optionally the fp64 inertia scalar tensor.
+    csr: sparse_orders' first result; Ct fp32 [n_item, kpad] (the centroids item-major, zero pad); cnorm fp64 [k]."""
+    off, item, val = csr
+    _need_cuda(off, item, val, Ct, cnorm)
+    assert Ct.dtype == torch.float32 and cnorm.dtype == torch.float64 and cnorm.shape == (k,)
+    n, kp = off.shape[0] - 1, Ct.shape[1]
+    L = _lib.lib()
+    M = torch.empty((n, kp), dtype=torch.float32, device=off.device)
+    inertia = torch.zeros(1, dtype=torch.float64, device=off.device) if want_inertia else None
+    scratch = torch.empty(max(1, int(L.ure_sparse_cost_scratch_bytes(n))), dtype=torch.uint8, device=off.device)
+    with torch.cuda.device(off.device):
+        check(L.ure_sparse_cost(_ptr(off), _ptr(item), _ptr(val), n, _ptr(Ct.contiguous()), _ptr(cnorm.contiguous()),
+                                int(k), kp, _ptr(M), _ptr(inertia), _ptr(scratch), _stream()), "ure_sparse_cost")
+    return (M, inertia) if want_inertia else M
+
+
+def sparse_centroid_sums(csc, label, k: int):
+    """(sums fp64 [n_item, kpad_for(k)], counts int64 [k]) of ure_sparse_centroid_sums: per item the sum of its ratings
+    by the label of their user, and the users per label.  csc: sparse_orders' second result; label int32 [n_user]."""
+    off, user, val = csc
+    _need_cuda(off, user, val, label)
+    assert label.dtype == torch.int32 and label.is_contiguous()
+    n_item, kp = off.shape[0] - 1, kpad_for(k)
+    sums = torch.empty((n_item, kp), dtype=torch.float64, device=off.device)
+    cnt = torch.empty(k, dtype=torch.int64, device=off.device)
+    with torch.cuda.device(off.device):
+        check(_lib.lib().ure_sparse_centroid_sums(_ptr(off), _ptr(user), _ptr(val), n_item, _ptr(label), label.shape[0],
+                                                  int(k), kp, _ptr(sums), _ptr(cnt), _stream()),
+              "ure_sparse_centroid_sums")
+    return sums, cnt
+
+
 # ------------------------------------------------------------------------------ top-N recommendation
 def _records_of(inters) -> torch.Tensor:
     """One int32 [n, 4] record tensor from one or several (device-to-device copies, no kernel)."""

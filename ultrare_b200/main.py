@@ -16,7 +16,7 @@ _FLAGS = {
     'delper': (int, 2, 'deleted user (or, with --deltype inter, rating) proportion', (2, 5)),
     'deltype': (str, 'rand', 'deletion type: rand = users, inter = single ratings', ('rand', 'inter')),
 }
-GROUP_TYPES = ('emb-ot',)                      # the only grouping the reference's CLI reaches (main.py:64)
+GROUP_TYPES = ('emb-ot', 'rating-ot')          # emb-ot: the grouping the reference's CLI reaches (main.py:64)
 
 
 def _build_parser():
@@ -35,6 +35,10 @@ def _build_parser():
                    help='how the SISA shard models are combined for the final evaluation and the recommendations: '
                         'mean = the reference\'s plain mean, fit = a per-group least-squares combination refitted '
                         'on the retained data after every unlearn (combine.npy)')
+    p.add_argument('--grouping', default='emb-ot', choices=GROUP_TYPES,
+                   help='how users are grouped into shards: emb-ot = OT clustering of the user table of a --group 0 '
+                        'run, rating-ot = OT clustering of the users\' rating rows of the training file (no earlier '
+                        'run needed)')
     return p
 
 
@@ -67,8 +71,7 @@ def main(argv=None):
     if a.group == 0:
         ins.runFull(is_save=True, verbose=a.verbose)
         return ins
-    for group_type in GROUP_TYPES:
-        ins.runGroup(is_save=True, learn_type=a.learn, group_type=group_type, n_group=a.group, verbose=a.verbose)
+    ins.runGroup(is_save=True, learn_type=a.learn, group_type=a.grouping, n_group=a.group, verbose=a.verbose)
     return ins
 
 

@@ -437,6 +437,77 @@ def ot_cluster_device(X, k, max_iters=10, schedule=SINKHORN_SCHEDULE, centroid0=
     Xp = np.zeros((n_local, d_pad), dtype=np.float32)
     Xp[:, :d] = X
     Xd = kn.upload_table(Xp, dev)
+
+    def cost(centroid):
+        Cp = np.zeros((k, d_pad), dtype=np.float32)
+        Cp[:, :d] = centroid
+        return kn.cost_matrix(Xd, kn.upload_array(Cp, dev), want_inertia=True)     # utils.py:637-638
+
+    def new_centroid(sums_h, cnt_h):
+        return (sums_h[:, :d] / cnt_h[:, None]).astype(np.float32)
+
+    return _ot_outer_loop(n, k, centroid, cost, lambda label: kn.centroid_sums(Xd, label, k), new_centroid,
+                          max_iters, schedule, dist if sharded else None, tol, warm_start, balance)
+
+
+def sparse_records(X):
+    """int32 [nnz, 4] records (user, item, fp32 value bits, 0) of the stored entries of a SciPy sparse matrix, duplicates
+    included: what ot_cluster_sparse_device uploads for kernels.sparse_orders."""
+    coo = X.tocoo()
+    rec = np.zeros((coo.nnz, 4), dtype=np.int32)
+    rec[:, 0], rec[:, 1] = coo.row, coo.col
+    rec[:, 2] = np.ascontiguousarray(coo.data, dtype=np.float32).view(np.int32)
+    return rec
+
+
+def ot_cluster_sparse_device(X, k, max_iters=10, schedule=SINKHORN_SCHEDULE, centroid0=None, device=None, dist=None,
+                             tol=None, warm_start=True, balance=True):
+    """``ot_cluster_device`` with the users' rows of a SciPy sparse matrix X [n, n_item] as the points (the reference's
+    'rating-ot' grouping, group.py on readSparseMat); returns (inertia, label int64 ndarray, centroid fp32 [k, n_item],
+    n_outer).  The nonzeros are uploaded once and ordered by user and by item on the device (kernels.sparse_orders);
+    per outer iteration the cost matrix comes from ure_sparse_cost and the centroid sums from ure_sparse_centroid_sums,
+    the rest of the loop is ot_cluster_device's.  Duplicate (user, item) entries count as their sum, as in SciPy; a
+    user without entries is the zero row.  2 <= k <= 128 (the balanced rounding's limit).  One GPU: the grouping runs
+    on rank 0 and is broadcast (config.Instance._group_index), so ``dist`` with several ranks raises."""
+    import scipy.sparse as sp
+    if not sp.issparse(X):
+        raise TypeError("ot_cluster_sparse_device: X must be a SciPy sparse matrix")
+    if dist is not None and dist.world > 1:
+        raise ValueError("ot_cluster_sparse_device runs on one GPU (cluster on rank 0 and broadcast the labels)")
+    if not 2 <= k <= kn._lib.URE_SPARSE_OT_MAX_K:
+        raise ValueError(f"ot_cluster_sparse_device: k={k} outside 2 .. {kn._lib.URE_SPARSE_OT_MAX_K}")
+    dev = _cuda_device(device)
+    X = sp.csr_matrix(X, dtype=np.float32)
+    n, n_item = X.shape
+    if k > n:
+        raise ValueError(f"ot_cluster_sparse_device: k={k} > {n} users")
+    if centroid0 is None:
+        centroid = X[np.random.choice(n, size=k, replace=False)].toarray()  # reference utils.py:632
+    else:
+        centroid = np.asarray(centroid0, dtype=np.float32)
+    csr, csc = kn.sparse_orders(kn.upload_table(sparse_records(X), dev), n, n_item)
+    kp = kn.kpad_for(k)
+
+    def cost(centroid):
+        Ct = np.zeros((n_item, kp), dtype=np.float32)
+        Ct[:, :k] = centroid.T
+        cnorm = np.square(centroid.astype(np.float64)).sum(axis=1)
+        return kn.sparse_cost(csr, kn.upload_array(Ct, dev), kn.upload_array(cnorm, dev), k, want_inertia=True)
+
+    def new_centroid(sums_h, cnt_h):
+        return (sums_h[:, :k].T / cnt_h[:, None]).astype(np.float32)
+
+    return _ot_outer_loop(n, k, np.asarray(centroid, dtype=np.float32), cost,
+                          lambda label: kn.sparse_centroid_sums(csc, label, k), new_centroid,
+                          max_iters, schedule, None, tol, warm_start, balance)
+
+
+def _ot_outer_loop(n, k, centroid, cost, centroid_sums, new_centroid, max_iters, schedule, dist, tol, warm_start,
+                   balance):
+    """The outer loop both ot_cluster paths share (reference utils.py:635-654).  cost(centroid) -> (M [n_local, kpad],
+    fp64 inertia tensor); centroid_sums(label) -> (sums, counts [k]) device tensors; new_centroid(sums, counts) -> the
+    next centroids from their host copies.  dist: a Dist with several ranks (rows sharded), or None."""
+    sharded = dist is not None
     balance = balance and not sharded and 1 < k <= 128
     if tol is None:
         tol = SINKHORN_TOL_BALANCED if balance else SINKHORN_TOL
@@ -445,10 +516,7 @@ def ot_cluster_device(X, k, max_iters=10, schedule=SINKHORN_SCHEDULE, centroid0=
     inertia = 0.0
     it = 0
     for it in range(1, max_iters + 1):
-        Cp = np.zeros((k, d_pad), dtype=np.float32)
-        Cp[:, :d] = centroid
-        Cd = kn.upload_array(Cp, dev)
-        M, inert = kn.cost_matrix(Xd, Cd, want_inertia=True)                # utils.py:637-638
+        M, inert = cost(centroid)
         if sharded:
             dist.all_reduce(inert)
         inertia = float(kn.download_many([inert])[0][0])
@@ -461,7 +529,7 @@ def ot_cluster_device(X, k, max_iters=10, schedule=SINKHORN_SCHEDULE, centroid0=
             g = kn.sinkhorn_sharded(M, k, sched, dist, n, g=g if warm else None)
         label, _, cnt = kn.assign_centroids(M, k, g, None)                  # utils.py:647 (argmax of the plan row)
         status = kn.balance_labels(M, k, label, cnt, BALANCE_MAX_AUGMENTATIONS) if balance else None
-        sums, cnt = kn.centroid_sums(Xd, label, k)                          # utils.py:648
+        sums, cnt = centroid_sums(label)                                    # utils.py:648
         if sharded:
             dist.all_reduce(sums)
             dist.all_reduce(cnt)
@@ -476,16 +544,19 @@ def ot_cluster_device(X, k, max_iters=10, schedule=SINKHORN_SCHEDULE, centroid0=
             import warnings
             warnings.warn(f"ot_cluster: balanced rounding stopped early ({int(got[3][0])} augmentations, "
                           f"{int(got[3][1])} users still to move); group sizes {cnt_h[:k].tolist()}")
-        new_centroid = (sums_h[:, :d] / cnt_h[:, None]).astype(np.float32)
-        if np.allclose(centroid, new_centroid):                              # utils.py:651
+        nxt = new_centroid(sums_h, cnt_h)
+        if np.allclose(centroid, nxt):                                       # utils.py:651
             break
-        centroid = new_centroid
+        centroid = nxt
     return np.float32(inertia), label.cpu().numpy().astype(np.int64), centroid, it
 
 
 @timefn
 def ot_cluster(X, k, max_iters=10):
-    """reference utils.py:628-656: returns (inertia, label)."""
-    inertia, label, _, _ = ot_cluster_device(X, k, max_iters)
+    """reference utils.py:628-656: returns (inertia, label).  X: a dense [n, d] embedding, or a SciPy sparse matrix of
+    the users' rating rows ('rating-ot', ot_cluster_sparse_device)."""
+    import scipy.sparse as sp
+    run = ot_cluster_sparse_device if sp.issparse(X) else ot_cluster_device
+    inertia, label, _, _ = run(X, k, max_iters)
     print(f'{inertia:.3f}', end=' ')
     return inertia, label

@@ -362,7 +362,8 @@ def loadData(data, batch=30000, n_worker=24, shuffle=True, perms=None):
 
 
 def readSparseMat(dir, n_user, n_item, max_rating=5):
-    """reference read.py:136-145; only its shape is used on the 'emb-ot' path (config.py:130)."""
+    """reference read.py:136-145: fp32 CSR [n_user, n_item] of rating / max_rating, duplicate (user, item) rows summed
+    (SciPy's conversion).  The points of the 'rating-ot' grouping; the 'emb-ot' path uses only the shape."""
     from scipy.sparse import coo_matrix
     ratings = pd.read_csv(dir, header=None, sep=',')
     row = ratings[0].astype(int).values
