@@ -99,6 +99,7 @@ class InsParam(object):
 class Instance(object):
     recommend_n = 0          # > 0: every pass also writes top-N recommendations and their metrics (main.py --recommend)
     combine = 'mean'         # how the SISA passes combine the shard models: 'mean' or 'fit' (Sisa.combine, --combine)
+    slices = 1               # SISA slices per shard (Sisa.slices, --slices); the training reads come slice-major
 
     def __init__(self, param):
         self.param = param
@@ -115,27 +116,27 @@ class Instance(object):
         self.timing = {}
 
     # read raw data (config.py:80-96)
-    def _read(self, is_del=False, n_group=1, group_index=[]):
+    def _read(self, is_del=False, n_group=1, group_index=[], n_slice=1):
         del_user = self.param.del_user if is_del == True else []
         del_rating = self.param.del_rating if is_del == True else []
         train_rating, train_index = readRating(self.param.train_dir, self.param.n_user, self.param.max_rating,
-                                               del_user, del_rating, n_group, group_index, 'a')
+                                               del_user, del_rating, n_group, group_index, 'a', n_slice)
         test_rating, _ = readRating(self.param.test_dir, self.param.n_user, self.param.max_rating,
                                     [], [], n_group, train_index)
         return train_rating, train_index, test_rating
 
     # the same read with the filter/split on the GPU: RatingData objects instead of arrays (read.readRatingDevice);
     # URE_HOST_INGEST=1 keeps the host split of `_read`
-    def _read_data(self, is_del=False, n_group=1, group_index=[]):
+    def _read_data(self, is_del=False, n_group=1, group_index=[], n_slice=1):
         import torch
         if os.environ.get('URE_HOST_INGEST', '0') == '1' or not torch.cuda.is_available():
-            train_rating, train_index, test_rating = self._read(is_del, n_group, group_index)
+            train_rating, train_index, test_rating = self._read(is_del, n_group, group_index, n_slice)
             return ([RatingData(r) for r in train_rating], train_index, [RatingData(r) for r in test_rating],
                     RatingData(np.hstack(test_rating)))
         del_user = self.param.del_user if is_del == True else []
         del_rating = self.param.del_rating if is_del == True else []
         train, train_index, _ = readRatingDevice(self.param.train_dir, self.param.n_user, self.param.max_rating,
-                                                 del_user, del_rating, n_group, group_index, 'a')
+                                                 del_user, del_rating, n_group, group_index, 'a', n_slice=n_slice)
         test, _, test_total = readRatingDevice(self.param.test_dir, self.param.n_user, self.param.max_rating,
                                                [], [], n_group, train_index)
         return train, train_index, test, test_total
@@ -204,7 +205,7 @@ class Instance(object):
         print(self.name, saving_name, 'begin:')
         group_index = self._group_index(group_type, n_group)
 
-        train, train_index, test, test_total = self._read_data(is_del, n_group, group_index)
+        train, train_index, test, test_total = self._read_data(is_del, n_group, group_index, self.slices)
 
         train_dlist, test_dlist = [], []
         assert learn_type in ['sisa']
@@ -216,6 +217,7 @@ class Instance(object):
         save_dir = self._save_dir(is_save, saving_name)
         model = Sisa(self.param, model_type, n_group, train_index)
         model.combine = self.combine
+        model.slices = self.slices
         t0 = time.time()
         if is_del == False:
             model.learn(train_dlist, test_dlist, test_data, verbose, save_dir)
@@ -224,6 +226,9 @@ class Instance(object):
             del_user = routed_users(self.param.del_user, self.param.del_rating)
             model.unlearn(model_list, train_dlist, test_dlist, test_data, del_user, verbose, save_dir)
             self.timing['unlearn_s'] = time.time() - t0
+            if self.slices > 1 and len(save_dir) > 0 and model.dist.rank == 0:
+                # int32 [K]: the first retrained slice of every shard (slices = not retrained)
+                np.save(save_dir + '/slices', model.first_slice.astype(np.int32))
         if self.recommend_n > 0:
             # seen items: this pass's training data (after the unlearn pass, deleted users' old items are gone)
             self._save_recommendations(save_dir, *model.recommend(None, self.recommend_n, exclude=train_dlist), test_data)

@@ -1014,8 +1014,11 @@ class ArenaShardBatch(ShardBatch):
     def __init__(self, recs, rows_P, n_item: int, d: int, batch: int, epochs: int, shard_ids, perm_seed: int = 42,
                  perms=None, lr: float = 1e-3, lr_decay: float = 0.95, lr_step: int = 50, weight_decay: float = 0.1,
                  momentum: float = 0.9, generator=None, std: float = 1.0, mode: str = "auto", owner_cache: bool = True,
-                 optimistic: bool = False):
-        """optimistic: the caller reads the training losses (train_losses_async) only after everything that depends
+                 optimistic: bool = False, init=None):
+        """init: per shard (P, Q) device tables the weights start from (copied into the arena) instead of the
+        N(0, std) draw -- a SISA slice stage resumes from the previous stage's checkpoint; momentum and losses start
+        cleared as always.
+        optimistic: the caller reads the training losses (train_losses_async) only after everything that depends
         on the training is queued, and repeats the pass on PlanHintMiss.  The launch is then queued with the
         capacities of the last plan read back for the same shapes (+ PLAN_HINT_MARGIN) instead of waiting for this
         one's -- the kernels compare them with the real plan on the device (hparams.owner_plan)."""
@@ -1027,6 +1030,13 @@ class ArenaShardBatch(ShardBatch):
         if mode not in ("dense", "owner", "auto"):
             raise ValueError(f"mode {mode!r}")
         _need_cuda(*recs)
+        if init is not None:
+            assert len(init) == K and not optimistic
+            for j, (P0, Q0) in enumerate(init):
+                _need_cuda(P0, Q0)
+                assert P0.dtype == Q0.dtype == torch.float32, "init tables must be fp32"
+                assert tuple(P0.shape) == (int(rows_P[j]), d) and tuple(Q0.shape) == (int(n_item), d), \
+                    f"init tables of shard {j}: {tuple(P0.shape)}, {tuple(Q0.shape)}"
         L = _lib.lib()
         self.device = dev = recs[0].device
         self.epochs, self.lazy, self.decay = int(epochs), False, None
@@ -1122,7 +1132,15 @@ class ArenaShardBatch(ShardBatch):
             # path, behind the schedule pre-pass, which does not read them (the host reaches that launch sooner)
             with torch.cuda.device(dev):
                 self._W = self.arena[int(lay.W):int(lay.W) + rows_w * d * 4].view(torch.float32).view(rows_w, d)
-                self._W.normal_(0.0, std, generator=generator() if callable(generator) else generator)
+                if init is None:
+                    self._W.normal_(0.0, std, generator=generator() if callable(generator) else generator)
+                    return
+                o = 0                                        # the arena's layout: user tables, then item tables
+                for j, (P0, Q0) in enumerate(init):
+                    r, q = self._rows_P[j], int(lay.rows_total) + j * self._n_item
+                    self._W[o:o + r].copy_(P0)
+                    self._W[q:q + self._n_item].copy_(Q0)
+                    o += r
 
         if not self.optimistic:
             fill_weights()

@@ -39,6 +39,9 @@ def _build_parser():
                    help='how users are grouped into shards: emb-ot = OT clustering of the user table of a --group 0 '
                         'run, rating-ot = OT clustering of the users\' rating rows of the training file (no earlier '
                         'run needed)')
+    p.add_argument('--slices', type=int, default=1, metavar='R',
+                   help='SISA slices per shard (1 .. 32): every shard trains in R stages and keeps the weights before '
+                        'each, so an unlearn retrains a shard only from its first affected slice; 1 = unsliced')
     return p
 
 
@@ -52,6 +55,10 @@ def _checked(args):
         assert ok(v) if callable(ok) else v in ok, f'--{name} {v!r} is not accepted'
     assert all(isinstance(w, int) for w in args.layer)
     assert 0 <= args.recommend <= 64, f'--recommend {args.recommend!r} is not accepted (0 .. 64)'
+    assert 1 <= args.slices <= 32, f'--slices {args.slices!r} is not accepted (1 .. 32)'
+    if args.slices > 1:
+        assert args.epoch_eval != 'faithful', '--slices > 1 needs --epoch-eval final or none'
+        assert args.group > 0, '--slices > 1 needs SISA shards (--group > 0)'
     return args
 
 
@@ -59,6 +66,8 @@ def main(argv=None):
     a = _checked(parser.parse_args(argv))
     if a.epoch_eval:
         os.environ['ULTRARE_EPOCH_EVAL'] = a.epoch_eval
+    elif a.slices > 1:                  # the sliced passes evaluate the final models only
+        os.environ['ULTRARE_EPOCH_EVAL'] = "final"
     from . import dist as udist
     udist.init_from_env()
     from .config import InsParam, Instance
@@ -68,6 +77,7 @@ def main(argv=None):
     ins = Instance(InsParam(a.dataset, a.epoch, a.worker, a.layer, a.group, a.delper, a.deltype))
     ins.recommend_n = a.recommend
     ins.combine = a.combine
+    ins.slices = a.slices
     if a.group == 0:
         ins.runFull(is_save=True, verbose=a.verbose)
         return ins

@@ -23,6 +23,11 @@ What changes underneath:
 In 'final' / 'none' mode each shard model stores only its owners' user rows (compact
 table): rows a shard does not own never receive a gradient and are dropped by the merge, so
 the merged table, the item tables and every final metric are unchanged.
+
+``slices`` = R > 1 adds SISA's slicing (DESIGN.md §4): each shard's records are read slice-major (read.readRating /
+readRatingDevice with n_slice=R), the shard trains in R stages of ``stage_epochs`` epochs each, stage r on slices
+0..r-1 and starting from the weights after stage r-1, and the weights before every stage are kept as checkpoints with
+the shard model.  An unlearn restarts each affected shard from the checkpoint before its first affected slice.
 """
 from __future__ import annotations
 
@@ -40,6 +45,12 @@ from .. import kernels as kn
 from .scratch import Scratch
 from .utils import (_request_users, baseTest, base_test_device, base_test_values, fit_combination, recommend_combined,
                     recommend_from_tables)
+
+
+def stage_epochs(epochs, slices):
+    """Epochs of one slice stage, SISA's e' = max(1, ceil(2E / (R + 1))): the R stages then train about as many
+    interactions as E unsliced epochs do.  R = 1 gives E."""
+    return max(1, -(-2 * int(epochs) // (int(slices) + 1)))
 
 
 class _Table:
@@ -154,6 +165,8 @@ class Sisa(Scratch):
         # retained training rows after every learn / unlearn pass
         self.combine = 'mean'
         self.combination = None
+        # SISA slicing: R stages per shard with a checkpoint before each (1 = unsliced, the reference's training)
+        self.slices = 1
 
     def _mode(self):
         if self.dist.world > 1 and self.epoch_eval == 'faithful':
@@ -705,6 +718,8 @@ class Sisa(Scratch):
 
     def learn(self, train_dlist, test_dlist, test_data, verbose, save_dir):
         """reference sisa.py:25-63."""
+        if self._sliced():
+            return self._learn_sliced(train_dlist, test_dlist, test_data, verbose, save_dir)
         return self._retrying(self._learn_once, train_dlist, test_dlist, test_data, verbose, save_dir)
 
     def _learn_once(self, train_dlist, test_dlist, test_data, verbose, save_dir):
@@ -735,6 +750,8 @@ class Sisa(Scratch):
         look-ups in the host copy of the same owner map -- no device round trip before the shards can be set up
         (defer_upload: not even the upload of the flags; the caller sends them when the merge needs them)."""
         ids = np.asarray(list(del_user), dtype=np.int64)
+        if self.slices > 1:
+            self.first_slice = self._first_slices(ids)
         if len(ids) <= self.ROUTE_ON_HOST_MAX:
             own = self._owner_np[ids[(ids >= 0) & (ids < self.n_user)]]
             flags_h = np.zeros(self.n_group, dtype=np.int32)
@@ -745,8 +762,22 @@ class Sisa(Scratch):
         d = kn.upload_array(ids.astype(np.int32), self.device)
         return kn.route_deletions(self._owner, d, self.n_group)
 
+    def _first_slices(self, ids):
+        """int32 [n_group]: per shard the first slice holding a routed user, min over u of row_of[u] * R // m_g
+        (R: no routed user), from the host copies of the owner and row maps."""
+        R = self.slices
+        ids = ids[(ids >= 0) & (ids < self.n_user)]
+        own = self._owner_np[ids]
+        ids, own = ids[own >= 0], own[own >= 0]
+        sizes = np.array([max(1, len(g)) for g in self.group_index], dtype=np.int64)
+        first = np.full(self.n_group, R, dtype=np.int32)
+        np.minimum.at(first, own, (self._row_of_np[ids].astype(np.int64) * R // sizes[own]).astype(np.int32))
+        return first
+
     def unlearn(self, model_list, train_dlist, test_dlist, test_data, del_user, verbose, save_dir):
         """reference sisa.py:66-118."""
+        if self._sliced():
+            return self._unlearn_sliced(model_list, train_dlist, test_dlist, test_data, del_user, verbose, save_dir)
         return self._retrying(self._unlearn_once, model_list, train_dlist, test_dlist, test_data, del_user, verbose,
                               save_dir)
 
@@ -800,5 +831,170 @@ class Sisa(Scratch):
         self._flush_logs()
         self._join_writers()
         self.timing['test_ms'] = (time.perf_counter() - t_t) * 1e3
+        self.timing['total_ms'] = (time.perf_counter() - t_begin) * 1e3
+        return self.model_list
+
+    # ------------------------------------------------------------------ SISA slicing (slices > 1)
+    def _sliced(self):
+        """True when learn / unlearn train in slice stages; checks what slicing needs."""
+        R = self.slices
+        if not isinstance(R, (int, np.integer)) or not 1 <= R <= 32:
+            raise ValueError(f"Sisa.slices must be an integer in 1..32, not {R!r}")
+        if R == 1:
+            return False
+        if self.epoch_eval not in ('final', 'none'):
+            raise ValueError(f"Sisa.slices > 1 needs epoch_eval 'final' or 'none', not {self.epoch_eval!r}")
+        if not self.init_on_device or type(self)._new_model is not Scratch._new_model:
+            raise ValueError("Sisa.slices > 1 needs the device-side initialisation of the batched shard training")
+        return True
+
+    def _slice_offsets(self, ds, g):
+        """int64 [R + 1]: the slice boundaries of shard g's records, which must be slice-major (read with
+        n_slice=R): the partition's offsets when the device ingest produced them, else counted from the users."""
+        R = self.slices
+        off = getattr(ds, 'slice_off', None)
+        if off is None:
+            s = self._row_of_np[np.asarray(ds.users, dtype=np.int64)].astype(np.int64) * R // \
+                max(1, len(self.group_index[g]))
+            if len(s) > 1 and (np.diff(s) < 0).any():
+                raise ValueError(f"shard {g}: the training records are not slice-major; read them with n_slice={R}")
+            off = np.concatenate([[0], np.cumsum(np.bincount(s, minlength=R))])
+        off = np.asarray(off, dtype=np.int64)
+        if off.shape != (R + 1,) or off[-1] != len(ds):
+            raise ValueError(f"shard {g}: slice offsets {off.tolist()} do not describe {len(ds)} records in {R} slices")
+        return off
+
+    def _train_sliced(self, ids, first, ckpts, train_dlist, verbose, fresh):
+        """Round j = 1..R trains stage j of every shard of `ids` on this GPU with first[g] < j, in one batch launch:
+        E' epochs on the shard's slices 0..j-1, from the checkpoint ckpts[g][j-1] (fresh: round 1 draws the initial
+        weights as the unsliced learn does, and they become checkpoint 0).  Returns ({shard: model}, {shard:
+        unmerged P}, {shard: index of its last log entry}); every model carries its R checkpoints."""
+        from ..read import RatingData
+        from .scratch import model_generator
+        from .utils import MF
+        R, E1, dev = self.slices, stage_epochs(self.epochs, self.slices), self.device
+        mine = self.dist.my_shards(list(ids))
+        self._last_batch = None
+        t0 = time.time()
+        RatingData.upload_many([train_dlist[g].dataset for g in mine], dev, self._row_of, 'sisa_local')
+        recs, offs, ck = {}, {}, {}
+        for g in mine:
+            if train_dlist[g].explicit_perm(dev, E1) is not None:
+                raise ValueError(f"shard {g}: slice stages visit the keyed shuffled order; explicit orders are not "
+                                 "supported with Sisa.slices > 1")
+            recs[g] = train_dlist[g].dataset.records_mapped(dev, self._row_of, 'sisa_local')
+            offs[g] = self._slice_offsets(train_dlist[g].dataset, g)
+            ck[g] = list(ckpts[g])
+        batch = train_dlist[mine[0]].batch_size if mine else self.batch
+        models, pending, rounds, trained = {}, [], 0, 0
+        for j in range(1, R + 1):
+            due = [g for g in mine if first[g] < j]
+            if not due:
+                continue
+            draw = fresh and j == 1
+            # sliced rounds wait for their owner plan (no optimistic launch): PlanHintMiss cannot arise mid-pass
+            sb = kn.ArenaShardBatch([recs[g][:int(offs[g][j])] for g in due], [len(self.group_index[g]) for g in due],
+                                    self.n_item, self.k, batch, E1, [g + 1 for g in due], self.seed, None, self.lr,
+                                    self.lr_decay, 50, self.lam, self.momentum,
+                                    generator=lambda: model_generator(self.seed, mine[0] + 1, dev),
+                                    init=None if draw else [ck[g][j - 1] for g in due])
+            views = sb.shards
+            if draw:
+                for v, g in zip(views, due):
+                    ck[g][0] = (v.P.clone(), v.Q.clone())
+            sb.train()
+            for v, g in zip(views, due):
+                if j < R:
+                    ck[g][j] = (v.P.clone(), v.Q.clone())
+                else:
+                    models[g] = MF.wrap(v.P, v.Q)
+                    models[g].checkpoints = ck[g]
+            pending.append((due, j, sb.train_losses_async()))
+            rounds += 1
+            trained += sb.interactions_trained()
+        stages = {g: [] for g in mine}
+        for due, j, wait in pending:
+            for g, l in zip(due, wait()):
+                stages[g].append((j, l))
+        self.timing['train_s'] = time.time() - t0
+        self.timing['rounds'] = rounds
+        self.timing['trained_interactions'] = trained
+        self.timing['stage_epochs'] = E1
+        # logs: shard after shard, stage after stage, one train_loss entry per trained epoch (test_* NaN; 'final'
+        # fills each shard's last entry in _finish)
+        nan, last_idx = float('nan'), {}
+        n_ep = sum(len(v) for v in stages.values()) * E1
+        stamp = time.strftime('%H:%M:%S', time.gmtime(self.timing['train_s'] / max(1, n_ep)))
+        for g in mine:
+            for j, l in stages[g]:
+                for e, v in enumerate(np.asarray(l, dtype=np.float64).tolist()):
+                    self.log['train_loss'].append(v)
+                    for key in ('test_rmse', 'test_ndcg', 'test_hr', 'total_rmse', 'total_ndcg', 'total_hr'):
+                        self.log[key].append(nan)
+                    self.log['time'].append(stamp)
+                    if verbose == 1:
+                        print(f'[shard {g+1}] Stage: [{j}/{R}] Epoch: [{e+1:>2d}/{E1:>2d}] train loss: {v:>.9f}')
+            last_idx[g] = len(self.log['train_loss']) - 1
+        return models, {g: models[g].user_mat.weight.data for g in mine}, last_idx
+
+    def _learn_sliced(self, train_dlist, test_dlist, test_data, verbose, save_dir):
+        assert len(train_dlist) == self.n_group
+        assert len(test_dlist) == self.n_group
+        self._test_dlist = test_dlist
+        K, R = self.n_group, self.slices
+        new, unmerged, last_idx = self._train_sliced(range(K), [0] * K, {g: [None] * R for g in range(K)},
+                                                     train_dlist, verbose, fresh=True)
+        merged = self._merged_from(None, unmerged, True, None)
+        self._finish(new, unmerged, last_idx, True, merged, test_dlist, save_dir)
+        shared = next(iter(new.values())).user_mat.weight if new else nn.Parameter(merged, requires_grad=False)
+        self.model_list = [new[i] if i in new else _RemoteModel(shared) for i in range(K)]
+        if self._use_fit():
+            t_c = time.perf_counter()
+            self._fit_combination(train_dlist, save_dir)
+            self.timing['combine_fit_ms'] = (time.perf_counter() - t_c) * 1e3
+        self.test(test_data, verbose, save_dir)
+        self._join_writers()
+        return self.model_list
+
+    def _unlearn_sliced(self, model_list, train_dlist, test_dlist, test_data, del_user, verbose, save_dir):
+        """Every shard with a routed user retrains from the checkpoint before its first affected slice a[g], on the
+        retained records, stages a[g]+1 .. R; its checkpoints from a[g]+1 on are replaced.  Equal to a sliced learn
+        on the retained data: no checkpoint it resumes from saw a deleted record."""
+        self.model_list = list(model_list)
+        assert len(train_dlist) == self.n_group
+        assert len(test_dlist) == self.n_group
+        self._test_dlist = test_dlist
+        R = self.slices
+        t_begin = time.perf_counter()
+        flags = self.route(del_user, defer_upload=True)
+        first = self.first_slice
+        self.retrain_gid = set(int(s) for s in np.flatnonzero(first < R))
+        self.timing['route_ms'] = (time.perf_counter() - t_begin) * 1e3
+        order = sorted(self.retrain_gid)
+        ckpts = {}
+        for g in self.dist.my_shards(order):
+            c = getattr(self.model_list[g], 'checkpoints', None)
+            if c is None or len(c) != R:
+                have = 'none' if c is None else f'{len(c)} slices'
+                raise RuntimeError(f"Sisa.unlearn with slices={R}: shard {g}'s model holds no checkpoints for {R} "
+                                   f"slices ({have}); learn with the same Sisa.slices first")
+            ckpts[g] = c
+        base = self.model_list[0].user_mat.weight.data
+        new, unmerged, last_idx = self._train_sliced(order, first, ckpts, train_dlist, verbose, fresh=False)
+        if flags is None:
+            flags = kn.upload_array(self._route_flags_host, self.device, side=True)
+        merged = self._merged_from(base, unmerged, True, flags)
+        self._finish(new, unmerged, last_idx, True, merged, test_dlist, save_dir)
+        for i, m in new.items():
+            self.model_list[i] = m
+        shared = next(iter(new.values())).user_mat.weight if new else nn.Parameter(merged, requires_grad=False)
+        for m in self.model_list:
+            m.user_mat.weight = shared
+        if self._use_fit():
+            t_c = time.perf_counter()
+            self._fit_combination(train_dlist, save_dir)
+            self.timing['combine_fit_ms'] = (time.perf_counter() - t_c) * 1e3
+        self.test(test_data, verbose, save_dir)
+        self._join_writers()
         self.timing['total_ms'] = (time.perf_counter() - t_begin) * 1e3
         return self.model_list

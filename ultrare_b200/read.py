@@ -41,10 +41,28 @@ def _row_keys(ratings):
     return (u << 32) | (i & 0xFFFFFFFF)
 
 
-def readRating(dir, n_user, max_rating=5, del_user=[], del_rating=[], n_group=1, group_index=[], sort='r'):
+def _slice_owner(owner, group_index, n_slice):
+    """Composite owner g * n_slice + slice(u) of every user of the owner map (-1 stays -1): SISA slicing, where
+    slice(u) = row_of[u] * n_slice // m_g, row_of[u] = u's position in group_index[g] (its compact row, as
+    method/sisa.py's owner maps count it) and m_g = len(group_index[g]).  Fixed by the grouping alone, so learn and
+    every later unlearn agree on it.  n_slice * n_group bins must fit the partition's 254."""
+    n_group = len(group_index)
+    if n_group * n_slice > 254:
+        raise ValueError(f"n_group * n_slice = {n_group} * {n_slice} = {n_group * n_slice} exceeds the limit of 254 "
+                         "shard-slice bins of the ingest partition")
+    slc = np.zeros(len(owner), dtype=np.int64)
+    for g in range(n_group - 1, -1, -1):
+        ids = np.asarray(group_index[g], dtype=np.int64)
+        slc[ids] = np.arange(len(ids), dtype=np.int64) * n_slice // max(1, len(ids))
+    return np.where(owner >= 0, owner.astype(np.int64) * n_slice + slc, -1).astype(owner.dtype)
+
+
+def readRating(dir, n_user, max_rating=5, del_user=[], del_rating=[], n_group=1, group_index=[], sort='r', n_slice=1):
     """reference read.py:9-70.  Returns (rating_lists [n_group] of float64 [3,n_g], group_index).
     del_rating: (user, item) pairs whose rows are dropped (interaction-level unlearning); the group order is that
-    of the unfiltered table."""
+    of the unfiltered table.
+    n_slice > 1 (SISA slicing): every group's rows are in slice-major order (_slice_owner), file order within a
+    slice."""
     if len(group_index) == 0:
         group_len = int(np.ceil(n_user / n_group))
         org_index = np.arange(n_user).tolist()
@@ -75,9 +93,17 @@ def readRating(dir, n_user, max_rating=5, del_user=[], del_rating=[], n_group=1,
     if del_keys is not None:
         row_owner = np.where(np.isin(_row_keys(ratings), del_keys), -1, row_owner)
 
+    if n_slice > 1:
+        comp = _slice_owner(owner, group_index, n_slice)
+        row_bin = np.where(row_owner >= 0, comp[users.astype(np.int64)], -1)
     rating_lists = []
     for g in range(n_group):
-        ratings_group = vals[row_owner == g].T.astype(np.float64).copy()
+        if n_slice > 1:
+            sel = np.flatnonzero(row_owner == g)
+            sel = sel[np.argsort(row_bin[sel], kind='stable')]
+        else:
+            sel = row_owner == g
+        ratings_group = vals[sel].T.astype(np.float64).copy()
         if ratings_group.size == 0:
             ratings_group = np.zeros((3, 0), dtype=np.float64)
         ratings_group[2] /= max_rating
@@ -86,7 +112,7 @@ def readRating(dir, n_user, max_rating=5, del_user=[], del_rating=[], n_group=1,
 
 
 def readRatingDevice(dir, n_user, max_rating=5, del_user=[], del_rating=[], n_group=1, group_index=[], sort='r',
-                     device='cuda'):
+                     device='cuda', n_slice=1):
     """``readRating`` (reference read.py:9-70) with the row filter and the group split ON the device.
 
     The CSV is parsed on the host (pandas, as in the reference) and uploaded ONCE; one stable partition kernel
@@ -95,6 +121,9 @@ def readRatingDevice(dir, n_user, max_rating=5, del_user=[], del_rating=[], n_gr
     group_index, total) where ``total`` is the RatingData of all groups back to back (config.py:144-148's hstack).
     del_rating: (user, item) pairs whose rows the same partition drops (ure_partition_interactions_del, with the
     per-user deleted-item lists of kernels.deletion_lists).
+    n_slice > 1 (SISA slicing): the same partition splits by the composite owner g * n_slice + slice(u) over
+    n_group * n_slice bins (at most 254), so every group's records come out slice-major, file order within a slice;
+    each dataset's ``slice_off`` (int64 [n_slice + 1]) holds its slice boundaries.
     """
     if len(group_index) == 0:                 # read.py:13-26, same RNG calls as readRating
         group_len = int(np.ceil(n_user / n_group))
@@ -114,6 +143,9 @@ def readRatingDevice(dir, n_user, max_rating=5, del_user=[], del_rating=[], n_gr
     owner = np.full(n_map, -1, dtype=np.int32)
     for g in range(n_group - 1, -1, -1):      # a user belongs to the first group that lists it
         owner[np.asarray(group_index[g], dtype=np.int64)] = g
+    if n_slice > 1:
+        owner = _slice_owner(owner, group_index, n_slice)
+    n_bins = n_group * n_slice
     deleted = None
     if len(del_user):
         deleted = np.zeros(n_map, dtype=np.uint8)
@@ -126,12 +158,17 @@ def readRatingDevice(dir, n_user, max_rating=5, del_user=[], del_rating=[], n_gr
         tab[j] = ratings[j].values
     table = kn.upload_table(tab, dev)
     rec, off = kn.partition_interactions(table, max_rating, kn.upload_array(owner, dev),
-                                         None if deleted is None else kn.upload_array(deleted, dev), n_group,
+                                         None if deleted is None else kn.upload_array(deleted, dev), n_bins,
                                          del_lists=del_lists)
     off_h = off.cpu().numpy()
     src = (ratings, owner, deleted, float(max_rating), del_keys)
-    datasets = [DeviceRatingData(rec[int(off_h[g]):int(off_h[g + 1])], src, (g, g + 1)) for g in range(n_group)]
-    total = DeviceRatingData(rec[:int(off_h[n_group])], src, (0, n_group))
+    R = n_slice
+    datasets = [DeviceRatingData(rec[int(off_h[g * R]):int(off_h[(g + 1) * R])], src, (g * R, (g + 1) * R))
+                for g in range(n_group)]
+    if R > 1:
+        for g, ds in enumerate(datasets):
+            ds.slice_off = off_h[g * R:(g + 1) * R + 1].astype(np.int64) - int(off_h[g * R])
+    total = DeviceRatingData(rec[:int(off_h[n_bins])], src, (0, n_bins))
     return datasets, group_index, total
 
 
