@@ -53,6 +53,61 @@ def routed_users(del_user, del_rating):
     return out + new[~np.isin(new, np.asarray(out))].tolist()
 
 
+def save_recommendations(save_dir, N, items, scores, test_data):
+    """rec{N}.npy (int32 [n_user, N] item ids), rec{N}_score.npy (fp32) and rec{N}_metrics.npy (fp64 [4]: HR@N,
+    Recall@N, NDCG@N over the whole catalogue, users counted) into the pass's save directory."""
+    from . import dist as udist
+    met = topn_metrics(items, None, test_data, N)
+    print(f'Top-{N} over the catalogue - HR: {met["hr"]:>.4f}, Recall: {met["recall"]:>.4f}, '
+          f'NDCG: {met["ndcg"]:>.4f} ({met["users"]} users)')
+    if len(save_dir) > 0 and udist.get().rank == 0:
+        np.save(f'{save_dir}/rec{N}', items.cpu().numpy())
+        np.save(f'{save_dir}/rec{N}_score', scores.cpu().numpy())
+        np.save(f'{save_dir}/rec{N}_metrics',
+                np.array([met['hr'], met['recall'], met['ndcg'], met['users']], dtype=np.float64))
+
+
+def check_out_dir(out_dir):
+    """A request run writes into a directory that does not exist yet or is empty: it never mixes with, or
+    overwrites, another run's files."""
+    if os.path.exists(out_dir) and (not os.path.isdir(out_dir) or os.listdir(out_dir)):
+        raise ValueError(f"the output directory {out_dir} exists and is not empty; a request run writes into a new or "
+                         "empty directory")
+
+
+def run_request(state_dir, out_dir, users=(), pairs=(), recommend_n=0, verbose=1):
+    """Apply one deletion request to the SISA state in `state_dir` (Sisa.load_state, Sisa.apply_request) and write
+    into `out_dir`: the artefacts of an unlearn pass (log*.npy; user_mat*, item_mat*, model*.pth of the retrained
+    shards; combine.npy; slices.npy; rec{N}*.npy), deletion.npy (the effective request, sisa_state.deletion_table)
+    and state/, the updated state.  The input state is only read.  Returns the Sisa."""
+    from . import dist as udist
+    from .method import sisa_state as st
+    d = udist.get()
+    check_out_dir(out_dir)
+    d.barrier()
+    print(state_dir, 'deletion request begin:')
+    model = Sisa.load_state(state_dir)
+    users, pairs = model.effective_request(users, pairs)
+    os.makedirs(out_dir, exist_ok=True)
+    if len(users) == 0 and len(pairs) == 0:
+        print('The request holds only deletions the state has already applied: no shard is retrained, '
+              'the state is unchanged')
+    else:
+        print(f'Effective request: {len(users)} users, {len(pairs)} ratings')
+        train_dlist, test_dlist, test_data = model.retained_data(users, pairs)
+        model.apply_request(users, pairs, train_dlist, test_dlist, test_data, verbose, out_dir)
+        if model.slices > 1 and d.rank == 0:
+            np.save(out_dir + '/slices', model.first_slice.astype(np.int32))
+        if recommend_n > 0:
+            save_recommendations(out_dir, recommend_n, *model.recommend(None, recommend_n, exclude=train_dlist),
+                                 test_data)
+    if d.rank == 0:
+        np.save(out_dir + '/deletion', st.deletion_table(users, pairs))
+    model.save_state(out_dir + '/state')
+    print('End of request', out_dir)
+    return model
+
+
 class InsParam(object):
     def __init__(self, dataset='toy', epochs=50, n_worker=24, layers=[32], n_group=2, del_per=2, del_type='test'):
         # model param (config.py:19-21)
@@ -100,6 +155,7 @@ class Instance(object):
     recommend_n = 0          # > 0: every pass also writes top-N recommendations and their metrics (main.py --recommend)
     combine = 'mean'         # how the SISA passes combine the shard models: 'mean' or 'fit' (Sisa.combine, --combine)
     slices = 1               # SISA slices per shard (Sisa.slices, --slices); the training reads come slice-major
+    save_state = False       # every SISA pass also writes its model as state/ in its directory (--save-state)
 
     def __init__(self, param):
         self.param = param
@@ -218,6 +274,8 @@ class Instance(object):
         model = Sisa(self.param, model_type, n_group, train_index)
         model.combine = self.combine
         model.slices = self.slices
+        model.source = dict(dataset=self.param.dataset, train_file=self.param.train_dir, test_file=self.param.test_dir,
+                            max_rating=self.param.max_rating, grouping=group_type, group_index=group_index)
         t0 = time.time()
         if is_del == False:
             model.learn(train_dlist, test_dlist, test_data, verbose, save_dir)
@@ -229,25 +287,18 @@ class Instance(object):
             if self.slices > 1 and len(save_dir) > 0 and model.dist.rank == 0:
                 # int32 [K]: the first retrained slice of every shard (slices = not retrained)
                 np.save(save_dir + '/slices', model.first_slice.astype(np.int32))
+            if self.save_state:
+                model.record_deletions(self.param.del_user, self.param.del_rating)      # the ledger of the state
         if self.recommend_n > 0:
             # seen items: this pass's training data (after the unlearn pass, deleted users' old items are gone)
             self._save_recommendations(save_dir, *model.recommend(None, self.recommend_n, exclude=train_dlist), test_data)
+        if self.save_state and len(save_dir) > 0:
+            model.save_state(save_dir + '/state')
         self.last_sisa = model
         return model.model_list
 
     def _save_recommendations(self, save_dir, items, scores, test_data):
-        """rec{N}.npy (int32 [n_user, N] item ids), rec{N}_score.npy (fp32) and rec{N}_metrics.npy (fp64 [4]: HR@N,
-        Recall@N, NDCG@N over the whole catalogue, users counted) into the pass's save directory."""
-        from . import dist as udist
-        N = self.recommend_n
-        met = topn_metrics(items, None, test_data, N)
-        print(f'Top-{N} over the catalogue - HR: {met["hr"]:>.4f}, Recall: {met["recall"]:>.4f}, '
-              f'NDCG: {met["ndcg"]:>.4f} ({met["users"]} users)')
-        if len(save_dir) > 0 and udist.get().rank == 0:
-            np.save(f'{save_dir}/rec{N}', items.cpu().numpy())
-            np.save(f'{save_dir}/rec{N}_score', scores.cpu().numpy())
-            np.save(f'{save_dir}/rec{N}_metrics',
-                    np.array([met['hr'], met['recall'], met['ndcg'], met['users']], dtype=np.float64))
+        save_recommendations(save_dir, self.recommend_n, items, scores, test_data)
 
     # ---------------------------------------------------------------- calling functions
     def runFull(self, is_save=True, verbose=1):

@@ -1,6 +1,8 @@
 """Command line of the drop-in: the reference's flags with the reference's defaults and value checks
 (reference main.py:5-14 flags, :21-53 checks, :56-70 dispatch), plus optional flags whose defaults keep the
 reference behaviour.  `python main.py --dataset ml1m --epoch 50 --group 5 --learn sisa --delper 2 --deltype rand`
+A request run applies a deletion request to a saved SISA state:
+`python main.py --unlearn-from DIR --out OUT [--forget-users FILE] [--forget-ratings FILE] [--recommend N]`
 """
 import argparse
 import os
@@ -42,10 +44,35 @@ def _build_parser():
     p.add_argument('--slices', type=int, default=1, metavar='R',
                    help='SISA slices per shard (1 .. 32): every shard trains in R stages and keeps the weights before '
                         'each, so an unlearn retrains a shard only from its first affected slice; 1 = unsliced')
+    p.add_argument('--save-state', action='store_true',
+                   help='every SISA pass also writes its model as state/ in its pass directory (Sisa.save_state)')
+    p.add_argument('--unlearn-from', default=None, metavar='DIR',
+                   help='request run: load the SISA state in DIR (a pass\'s state/) and unlearn the deletions of '
+                        '--forget-users / --forget-ratings from it; dataset, shards, slices, epochs, combine and grouping '
+                        'come from the state')
+    p.add_argument('--out', default=None, metavar='OUT',
+                   help='request run: the new, or empty, directory the unlearn pass and the updated state/ go to')
+    p.add_argument('--forget-users', default=None, metavar='FILE',
+                   help='request run: users to delete (.npy, or text with one id per line)')
+    p.add_argument('--forget-ratings', default=None, metavar='FILE',
+                   help='request run: ratings to delete (.npy [n, 2], or text with user,item per line)')
     return p
 
 
 parser = _build_parser()
+
+# request run: flag -> the manifest entry it must agree with when it is given
+_FROM_STATE = {'dataset': 'dataset', 'group': 'K', 'slices': 'slices', 'epoch': 'epochs', 'combine': 'combine',
+               'grouping': 'grouping', 'epoch_eval': 'epoch_eval'}
+_NOT_WITH_REQUEST = ('delper', 'deltype', 'save_state')
+
+
+def _given(argv):
+    """{dest: value} of the flags given on the command line (defaults left out)."""
+    p = _build_parser()
+    for act in p._actions:
+        act.default = argparse.SUPPRESS
+    return vars(p.parse_args(argv))
 
 
 def _checked(args):
@@ -59,11 +86,43 @@ def _checked(args):
     if args.slices > 1:
         assert args.epoch_eval != 'faithful', '--slices > 1 needs --epoch-eval final or none'
         assert args.group > 0, '--slices > 1 needs SISA shards (--group > 0)'
+    request = (args.out, args.forget_users, args.forget_ratings)
+    if args.unlearn_from is None:
+        assert request == (None, None, None), '--out, --forget-users and --forget-ratings need --unlearn-from'
+    else:
+        assert args.out is not None, '--unlearn-from needs --out'
+        assert args.forget_users is not None or args.forget_ratings is not None, \
+            '--unlearn-from needs --forget-users or --forget-ratings'
     return args
+
+
+def _check_against_state(given, man, state_dir):
+    """A request run takes its settings from the state's manifest: a flag given with another value is an error."""
+    for flag in _NOT_WITH_REQUEST:
+        assert flag not in given, f'--{flag.replace("_", "-")} has no meaning with --unlearn-from'
+    for flag, key in _FROM_STATE.items():
+        if flag in given:
+            assert given[flag] == man[key], (f'--{flag.replace("_", "-")} {given[flag]!r} conflicts with the state in '
+                                             f'{state_dir}, which has {key} = {man[key]!r}')
+
+
+def _request(a, argv):
+    from .config import check_out_dir, run_request
+    from .method import sisa_state as st
+    man = st.read_manifest(a.unlearn_from)
+    _check_against_state(_given(argv), man, a.unlearn_from)
+    check_out_dir(a.out)
+    users = st.parse_request_file(a.forget_users, 'users') if a.forget_users else ()
+    pairs = st.parse_request_file(a.forget_ratings, 'ratings') if a.forget_ratings else ()
+    return run_request(a.unlearn_from, a.out, users, pairs, a.recommend, a.verbose)
 
 
 def main(argv=None):
     a = _checked(parser.parse_args(argv))
+    if a.unlearn_from is not None:
+        from . import dist as udist
+        udist.init_from_env()
+        return _request(a, argv)
     if a.epoch_eval:
         os.environ['ULTRARE_EPOCH_EVAL'] = a.epoch_eval
     elif a.slices > 1:                  # the sliced passes evaluate the final models only
@@ -78,6 +137,7 @@ def main(argv=None):
     ins.recommend_n = a.recommend
     ins.combine = a.combine
     ins.slices = a.slices
+    ins.save_state = a.save_state
     if a.group == 0:
         ins.runFull(is_save=True, verbose=a.verbose)
         return ins

@@ -28,9 +28,14 @@ the merged table, the item tables and every final metric are unchanged.
 readRatingDevice with n_slice=R), the shard trains in R stages of ``stage_epochs`` epochs each, stage r on slices
 0..r-1 and starting from the weights after stage r-1, and the weights before every stage are kept as checkpoints with
 the shard model.  An unlearn restarts each affected shard from the checkpoint before its first affected slice.
+
+``save_state`` / ``load_state`` write and read the whole model (merged user table, item tables, checkpoints, fitted
+combination, grouping, ledger of applied deletions) as a directory (DESIGN.md §4.10, method/sisa_state.py);
+``apply_request`` unlearns a deletion request from it, minus what the ledger already holds.
 """
 from __future__ import annotations
 
+import json
 import os
 import time
 import types
@@ -167,6 +172,14 @@ class Sisa(Scratch):
         self.combination = None
         # SISA slicing: R stages per shard with a checkpoint before each (1 = unsliced, the reference's training)
         self.slices = 1
+        # where the training data comes from (save_state records it; apply_request reads the retained data from it):
+        # dict(dataset, train_file, test_file, max_rating, grouping, group_index) -- group_index is the grouping
+        # before the reader's count sort ([]: the reader's uniform draw)
+        self.source = None
+        # the ledger: every deletion applied since the learn (sorted unique users, sorted unique (user, item) pairs)
+        self.deleted_users = np.zeros(0, dtype=np.int64)
+        self.deleted_pairs = np.zeros((0, 2), dtype=np.int64)
+        self.requests = 0
 
     def _mode(self):
         if self.dist.world > 1 and self.epoch_eval == 'faithful':
@@ -998,3 +1011,181 @@ class Sisa(Scratch):
         self._join_writers()
         self.timing['total_ms'] = (time.perf_counter() - t_begin) * 1e3
         return self.model_list
+
+    # ------------------------------------------------------------------ state on disk and deletion requests
+    def save_state(self, state_dir):
+        """Write the model as a state directory (DESIGN.md §4.10): this rank's shards' item tables and checkpoints; on
+        rank 0 the merged user table, the grouping, the ledger, the fitted combination and -- after every rank's
+        files, last -- manifest.json.  One device-to-host transfer per rank; the files are written by the artefact
+        writer thread.  A directory that already holds a manifest is refused: states are never overwritten."""
+        from . import sisa_state as st
+        src = self.source
+        if src is None:
+            raise ValueError("Sisa.save_state needs Sisa.source: the training data the model was learned from")
+        if os.path.exists(os.path.join(state_dir, st.MANIFEST)):
+            raise FileExistsError(f"{state_dir} already holds a SISA state; states are never overwritten")
+        if len(self.model_list) != self.n_group:
+            raise RuntimeError("Sisa.save_state: no trained model (run learn, or load a state, first)")
+        K, R, rank = self.n_group, self.slices, self.dist.rank
+        os.makedirs(state_dir, exist_ok=True)
+        names, tensors = [], []
+        for g in self.dist.my_shards(range(K)):
+            m = self.model_list[g]
+            names.append(f'item{g}')
+            tensors.append(m.item_mat.weight.data)
+            if R > 1:
+                ck = getattr(m, 'checkpoints', None)
+                if ck is None or len(ck) != R:
+                    raise RuntimeError(f"Sisa.save_state with slices={R}: shard {g}'s model holds no {R} checkpoints")
+                for r, (P, Q) in enumerate(ck):
+                    names += [f'ckpt{g}_{r}_P', f'ckpt{g}_{r}_Q']
+                    tensors += [P, Q]
+        if rank == 0:
+            names.append('merged')
+            tensors.append(self.model_list[0].user_mat.weight.data)
+        arrays = dict(zip(names, kn.download_many(tensors, copy=False)))
+        if rank == 0:
+            arrays['group_index_ids'], arrays['group_index_off'] = st.flat_index(src['group_index'])
+            arrays['train_index_ids'], arrays['train_index_off'] = st.flat_index(self.group_index)
+            arrays['deleted_users'] = np.asarray(self.deleted_users, dtype=np.int64)
+            arrays['deleted_pairs'] = np.asarray(self.deleted_pairs, dtype=np.int64).reshape(-1, 2)
+            if self._use_fit():
+                arrays['combine'] = self._fitted().table()
+                arrays['combine_gram'] = np.asarray(self._fitted().gram, dtype=np.float64)
+
+        def write(arrays=arrays):
+            for name, a in arrays.items():
+                np.save(os.path.join(state_dir, name + '.npy'), a, allow_pickle=False)
+
+        self._writers.append(_writer_pool().submit(write))
+        self._join_writers()
+        self.dist.barrier()                                     # every rank's files are on disk
+        if rank == 0:
+            if 'train_sha256' not in src:
+                src['train_bytes'], src['train_sha256'] = st.file_digest(src['train_file'])
+            man = dict(format=st.FORMAT_VERSION, K=K, slices=R, k=self.k, n_user=self.n_user, n_item=self.n_item,
+                       epochs=self.epochs, batch=self.batch, lr=self.lr, lr_decay=self.lr_decay, lam=self.lam,
+                       momentum=self.momentum, seed=self.seed, combine=self.combine, epoch_eval=self.epoch_eval,
+                       dataset=src['dataset'], grouping=src['grouping'], max_rating=src['max_rating'],
+                       train_file=dict(path=os.path.abspath(src['train_file']), bytes=int(src['train_bytes']),
+                                       sha256=src['train_sha256']),
+                       test_file=os.path.abspath(src['test_file']), requests=int(self.requests),
+                       saved_world_size=self.dist.world)
+            path = os.path.join(state_dir, st.MANIFEST)
+            with open(path + '.tmp', 'w') as f:
+                json.dump(man, f, indent=1)
+            os.replace(path + '.tmp', path)
+        self.dist.barrier()
+
+    @classmethod
+    def load_state(cls, state_dir, param=None, dist=None):
+        """The Sisa a state directory describes, ready for test / recommend / unlearn / apply_request: one MF per shard
+        this rank holds (dist.my_shards, whatever the world size the state was saved at) sharing the merged user
+        table, with its checkpoints when slices > 1; _RemoteModel for the other shards; the fitted combination
+        rebuilt (ure_item_wsum) when combine == 'fit'.  ValueError for an incomplete state, another format version,
+        a changed training file, or a `param` whose hyper-parameters differ from the state's."""
+        from . import sisa_state as st
+        from .utils import MF, combination_from
+        man = st.read_manifest(state_dir)
+        st.check_training_file(man)
+        hp = types.SimpleNamespace(**{k: man[k] for k in ('n_user', 'n_item', 'k', 'lam', 'seed', 'lr', 'lr_decay',
+                                                           'momentum', 'epochs', 'batch')})
+        for k, v in vars(hp).items():
+            if param is not None and hasattr(param, k) and getattr(param, k) != v:
+                raise ValueError(f"param.{k} = {getattr(param, k)!r}, but the state in {state_dir} has {k} = {v!r}")
+        K, R = int(man['K']), int(man['slices'])
+        group_index = st.unflat_index(st.load_array(state_dir, 'group_index_ids'),
+                                      st.load_array(state_dir, 'group_index_off'))
+        train_index = st.unflat_index(st.load_array(state_dir, 'train_index_ids'),
+                                      st.load_array(state_dir, 'train_index_off'))
+        if len(train_index) != K:
+            raise ValueError(f"{state_dir}: train_index has {len(train_index)} groups, the manifest K = {K}")
+        s = cls(hp, 'mf', K, train_index)
+        if dist is not None:
+            s.dist = dist
+        s.epoch_eval, s.slices, s.combine = man['epoch_eval'], R, man['combine']
+        s.source = dict(dataset=man['dataset'], train_file=man['train_file']['path'], test_file=man['test_file'],
+                        max_rating=man['max_rating'], grouping=man['grouping'], group_index=group_index,
+                        train_bytes=man['train_file']['bytes'], train_sha256=man['train_file']['sha256'])
+        s.deleted_users = st.load_array(state_dir, 'deleted_users').astype(np.int64)
+        s.deleted_pairs = st.load_array(state_dir, 'deleted_pairs').astype(np.int64).reshape(-1, 2)
+        s.requests = int(man['requests'])
+
+        def table(name, shape):
+            a = st.load_array(state_dir, name)
+            if a.dtype != np.float32 or a.shape != shape:
+                raise ValueError(f"{state_dir}/{name}.npy is {a.dtype} {a.shape}, expected float32 {shape}")
+            return a
+
+        dev, d = s.device, s.k
+        merged = kn.upload_table(table('merged', (s.n_user, d)), dev)
+        shared = nn.Parameter(merged, requires_grad=False)
+        mine = s.dist.my_shards(range(K))
+        # this rank's item tables back to back in ONE allocation, as a learn's batch arena holds them
+        Q = kn.upload_table(np.stack([table(f'item{g}', (s.n_item, d)) for g in mine]), dev) if mine else None
+        s.model_list = []
+        for g in range(K):
+            if g not in mine:
+                s.model_list.append(_RemoteModel(shared))
+                continue
+            m = MF.wrap(merged, Q[mine.index(g)])
+            m.user_mat.weight = shared
+            if R > 1:
+                rows = (len(train_index[g]), d)
+                m.checkpoints = [(kn.upload_table(table(f'ckpt{g}_{r}_P', rows), dev),
+                                  kn.upload_table(table(f'ckpt{g}_{r}_Q', (s.n_item, d)), dev)) for r in range(R)]
+            s.model_list.append(m)
+        if s._use_fit():
+            tab = st.load_array(state_dir, 'combine')
+            if tab.shape != (K, K + 1):
+                raise ValueError(f"{state_dir}/combine.npy is {tab.shape}, expected ({K}, {K + 1})")
+            s.combination = combination_from(np.ascontiguousarray(tab[:, :K]), np.ascontiguousarray(tab[:, K]),
+                                             s._item_tables_in_shard_order(), st.load_array(state_dir, 'combine_gram'))
+        return s
+
+    def effective_request(self, users=(), pairs=()):
+        """(users int64 [n], pairs int64 [n, 2]) of a deletion request, validated (sisa_state.validate_request), sorted,
+        unique and minus what the ledger holds: deleted users, deleted pairs and pairs of deleted users."""
+        from . import sisa_state as st
+        u, p = st.validate_request(users, pairs, self.n_user, self.n_item)
+        return st.effective_request(u, p, self.deleted_users, self.deleted_pairs)
+
+    def retained_data(self, users=(), pairs=()):
+        """(train loaders, test loaders, test loader) of the training file minus the ledger's deletions and the given
+        ones, read slice-major as the state was trained; ValueError when the reader's count-sorted grouping is not
+        the state's train_index (the training file changed)."""
+        from . import sisa_state as st
+        if self.source is None:
+            raise ValueError("Sisa.retained_data needs Sisa.source: the training data the model was learned from")
+        du, dp = st.ledger_union(self.deleted_users, self.deleted_pairs,
+                                 *st.validate_request(users, pairs, self.n_user, self.n_item))
+        tl, sl, total, train_index = st.read_retained(self.source, self.n_user, self.n_group, self.slices, self.batch,
+                                                      du, dp, self.device)
+        st.check_train_index(train_index, self.group_index)
+        return tl, sl, total
+
+    def record_deletions(self, users=(), pairs=()):
+        """Add an applied request to the ledger."""
+        from . import sisa_state as st
+        u, p = st.validate_request(users, pairs, self.n_user, self.n_item)
+        self.deleted_users, self.deleted_pairs = st.ledger_union(self.deleted_users, self.deleted_pairs, u, p)
+        self.requests += 1
+
+    def apply_request(self, users=(), pairs=(), train_dlist=None, test_dlist=None, test_data=None, verbose=0,
+                      save_dir=''):
+        """Unlearn a deletion request: deleted users and deleted (user, item) ratings.  Only the effective request
+        (effective_request: minus the ledger) is routed, so shards touched only by earlier requests are not retrained;
+        the retained data is the training file minus the ledger and the request (retained_data, read here unless the
+        loaders are given).  Runs unlearn, then adds the request to the ledger.  Returns the effective request; when
+        it is empty nothing is retrained and the model and the ledger stay as they were."""
+        from ..config import routed_users
+        users, pairs = self.effective_request(users, pairs)
+        if len(users) == 0 and len(pairs) == 0:
+            self.retrain_gid = set()
+            self.first_slice = np.full(self.n_group, self.slices, dtype=np.int32)
+            return users, pairs
+        if train_dlist is None:
+            train_dlist, test_dlist, test_data = self.retained_data(users, pairs)
+        self.unlearn(self.model_list, train_dlist, test_dlist, test_data, routed_users(users, pairs), verbose, save_dir)
+        self.record_deletions(users, pairs)
+        return users, pairs

@@ -301,10 +301,18 @@ def fit_combination(P, Q_list, inters):
     gram = kn.combine_gram(P, Q_list, inters)
     gram_h = kn.download_many([gram])[0]
     w, b = solve_combination(gram_h, K)
+    return combination_from(w, b, Q_list, gram_h)
+
+
+def combination_from(w, b, Q_list, gram):
+    """The Combination of given weights (w fp64 [K, K], b fp64 [K]) over the item tables Q_list: T from
+    ure_item_wsum, b_slot uploaded; what fit_combination builds after its solve, and what a loaded state rebuilds."""
+    K = len(Q_list)
+    dev = Q_list[0].device
     W = np.concatenate([w, np.full((1, K), 1.0 / K)]).astype(np.float32)
-    T = kn.item_wsum(Q_list, kn.upload_array(W, P.device))
-    b_slot = kn.upload_array(np.append(b, 0.0).astype(np.float32), P.device)
-    return Combination(w, b, T, b_slot, gram_h)
+    T = kn.item_wsum(Q_list, kn.upload_array(W, dev))
+    b_slot = kn.upload_array(np.append(b, 0.0).astype(np.float32), dev)
+    return Combination(w, b, T, b_slot, gram)
 
 
 def recommend_combined(P, comb, owner, users, top_n=10, exclude=None, keep=None):
