@@ -168,6 +168,31 @@ int ure_mf_train(const ure_mf_shard_t* d_shards, int n_shards, const ure_mf_hpar
                  int epochs, int64_t step_begin, int64_t step_end, int warps_group0,
                  void* d_workspace, void* stream);
 
+/* ---- BPR training (implicit feedback): the pairwise ranking objective over (user, rated item, unrated item) triples.
+ * Per shard, the seen lists of ure_seen_lists built from the records the launch trains (never the whole file: a
+ * negative excluded by data of a later SISA slice would make the slice checkpoints depend on it). */
+typedef struct {
+  const int64_t* seen_off;  /* [n_user + 1] row offsets into seen_items (user = the row in the shard's user table) */
+  const int32_t* seen_items;/* the items of each user's training records, ascending                                */
+} ure_bpr_shard_t;
+
+/* ure_mf_train with the BPR objective, DENSE schedule only (hparams.mode = URE_MF_DENSE, else URE_EUNSUPPORTED);
+ * d_bpr: DEVICE table [n_shards] of ure_bpr_shard_t.  Every record (u, i) is a positive (its rating is not used).
+ * Epoch e's negative of record idx is the first of 16 candidates c_t = mulhi32(mix32(h + t * 0x85EBCA77), n_item),
+ * h = mix32(key ^ (idx * 0x9E3779B1 + 0x7F4A7C15)), key = perm_key(perm_seed, shard_id, e) (csrc/feistel.cuh), that
+ * is not in u's seen list; if all 16 are seen the triple is dropped.  With x = P[u].(Q[i] - Q[j]), c = sigmoid(-x):
+ * loss softplus(-x), gradients -c (Q[i] - Q[j]) for P[u], -c P[u] for Q[i], +c P[u] for Q[j], PRE-step weights;
+ * then the same dense SGD (momentum, L2, StepLR).  sse[e] += the sum of softplus(-x) over the epoch's triples. */
+int ure_mf_train_bpr(const ure_mf_shard_t* d_shards, const ure_bpr_shard_t* d_bpr, int n_shards,
+                     const ure_mf_hparams_t* h_hp, int epochs, int64_t step_begin, int64_t step_end, int warps_group0,
+                     void* d_workspace, void* stream);
+
+/* Diagnostics and tests: d_neg[idx] = the negative of record idx of one shard in epoch `epoch` (-1: dropped), as
+ * ure_mf_train_bpr draws it.  d_tries (may be NULL): the number of candidates drawn for each record. */
+int ure_bpr_negatives(const ure_inter_t* d_inter, int32_t n, int32_t n_item, const int64_t* d_seen_off,
+                      const int32_t* d_seen_items, uint32_t perm_seed, int32_t shard_id, int32_t epoch, int32_t* d_neg,
+                      int32_t* d_tries, void* stream);
+
 /* Owner mode set-up, once per shard table (asynchronous, no host sync): builds inter_u / inter_i /
  * off_u / off_i (row histogram + scan; STABLE radix sort of the records by user and by item, so the whole
  * training is reproducible bit for bit) and perm_inv for shards with an explicit perm, then plans the CTA ownership and writes into the first 16 bytes of d_workspace

@@ -65,6 +65,11 @@ class MFBatchLayout(C.Structure):
                [(nm, _i32) for nm in ("spe_cap", "max_rows", "max_n", "grid", "owner", "sched_rows")]
 
 
+class BprShard(C.Structure):
+    """ure_bpr_shard_t"""
+    _fields_ = [("seen_off", _p), ("seen_items", _p)]
+
+
 MF_DENSE, MF_LAZY, MF_OWNER, MF_RUNS = 0, 1, 2, 3
 
 assert C.sizeof(MFShard) == 176 and C.sizeof(MFHParams) == 136 and C.sizeof(MFRuns) == 64
@@ -76,6 +81,8 @@ SIGNATURES = {
     "ure_abi_version": (C.c_int, []),
     "ure_mf_train_workspace_bytes": (_i64, []),
     "ure_mf_train": (C.c_int, [_p, C.c_int, C.POINTER(MFHParams), C.c_int, _i64, _i64, C.c_int, _p, _p]),
+    "ure_mf_train_bpr": (C.c_int, [_p, _p, C.c_int, C.POINTER(MFHParams), C.c_int, _i64, _i64, C.c_int, _p, _p]),
+    "ure_bpr_negatives": (C.c_int, [_p, _i32, _i32, _p, _p, C.c_uint32, _i32, _i32, _p, _p, _p]),
     "ure_mf_owner_radix_bytes": (_i64, [C.c_int]),
     "ure_mf_owner_prepare": (C.c_int, [_p, C.c_int, C.POINTER(MFHParams), C.c_int, C.c_int, _p, _p, _p]),
     "ure_mf_owner_smem_bytes": (_i64, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),

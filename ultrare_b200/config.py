@@ -109,6 +109,10 @@ def run_request(state_dir, out_dir, users=(), pairs=(), recommend_n=0, verbose=1
 
 
 class InsParam(object):
+    # training objective of every model (Scratch.loss / Sisa.loss, main.py --loss): 'mse' = the reference's squared
+    # rating error, 'bpr' = pairwise ranking with sampled negatives (implicit feedback)
+    loss = 'mse'
+
     def __init__(self, dataset='toy', epochs=50, n_worker=24, layers=[32], n_group=2, del_per=2, del_type='test'):
         # model param (config.py:19-21)
         self.k = 16
@@ -161,6 +165,8 @@ class Instance(object):
         self.param = param
         prefix = '/test/' if self.param.del_type == 'test' else '/' + str(self.param.del_per) + '/' + self.param.del_type + '/'
         self.name = prefix + self.param.dataset + '_g' + str(self.param.n_group)
+        if self.param.loss == 'bpr':           # BPR runs keep their artefacts apart from the MSE runs'
+            self.name += '_bpr'
         param_dir = SAVE_DIR + self.name
         os.makedirs(param_dir, exist_ok=True)
         saveObject(param_dir + '/param', self.param)

@@ -557,6 +557,42 @@ OWNER_SCHED_BYTES = 512 << 20  # device memory one ShardBatch may spend on owner
 RUNS_LIST_BYTES = 2 << 30      # device memory one ShardBatch may spend on the RUNS schedule's step lists
 OWNER_FORCE = None             # test hook: (owner_flags, list_cap) the owner schedule must use
 DEFAULT_MF_MODE = "auto"       # schedule ShardBatch picks when the caller does not say (see ShardBatch)
+LOSSES = ("mse", "bpr")        # training objectives: squared rating error (baseTrain) or BPR (ure_mf_train_bpr)
+
+
+def _bpr_mode(loss: str, mode: Optional[str]) -> Optional[str]:
+    """The schedule a batch with this loss trains with: BPR runs the DENSE schedule only (owner-computes cannot own a
+    row that a random negative touches), so it takes 'dense' for None / 'auto' and refuses the others."""
+    if loss not in LOSSES:
+        raise ValueError(f"loss must be one of {LOSSES}, not {loss!r}")
+    if loss == "mse":
+        return mode
+    if mode not in (None, "auto", "dense"):
+        raise ValueError(f"loss='bpr' trains with the dense schedule only, not mode={mode!r}")
+    return "dense"
+
+
+def _bpr_table(recs, rows_P, n_item: int, device):
+    """BPR: per shard the seen lists of the records it trains (kernels.seen_lists) and the device table of
+    ure_bpr_shard_t the training launch takes.  Returns (table, tensors to keep alive)."""
+    arr = (_lib.BprShard * len(recs))()
+    keep = []
+    bad = torch.zeros((), dtype=torch.bool, device=device)       # the id check of seen_lists, one sync for all shards
+    for rec, rows in zip(recs, rows_P):
+        if rec.shape[0] > 0:
+            u, i = rec[:, 0], rec[:, 1]
+            bad |= ((u < 0) | (u >= int(rows)) | (i < 0) | (i >= int(n_item))).any()
+    if bool(bad):
+        raise ValueError(f"BPR seen lists: user ids must lie in [0, rows of the shard's table) and item ids in "
+                         f"[0, {n_item})")
+    for j, (rec, rows) in enumerate(zip(recs, rows_P)):
+        off, items = seen_lists(rec, int(rows), int(n_item), validate=False)
+        if items.numel() == 0:                       # an empty shard: any valid address (never read)
+            items = torch.zeros(1, dtype=torch.int32, device=device)
+        keep += [off, items]
+        arr[j].seen_off, arr[j].seen_items = off.data_ptr(), items.data_ptr()
+    table = upload_array(np.frombuffer(bytes(arr), dtype=np.uint8), device)
+    return table, keep
 
 
 class ShardState:
@@ -616,12 +652,18 @@ class ShardBatch:
 
     def __init__(self, shards: List[ShardState], d: int, batch: int, lr: float = 1e-3, lr_decay: float = 0.95,
                  lr_step: int = 50, weight_decay: float = 0.1, momentum: float = 0.9, lazy: bool = False,
-                 mode: Optional[str] = None, owner_cache: bool = True, after_prepare=None):
+                 mode: Optional[str] = None, owner_cache: bool = True, after_prepare=None, loss: str = "mse"):
         """after_prepare: optional callable run once the set-up kernels that only read the records are queued
-        (alloc_shard_batch(defer_init=True)'s fills), before the set-up waits for the plan."""
+        (alloc_shard_batch(defer_init=True)'s fills), before the set-up waits for the plan.
+        loss: 'mse' (the reference's squared rating error) or 'bpr' (pairwise ranking with sampled negatives,
+        ure_mf_train_bpr; DENSE schedule only: mode None / 'auto' select it, 'lazy', 'owner' and 'runs' raise)."""
         self._after_prepare = after_prepare
         if not 1 <= len(shards) <= _lib.URE_MAX_SHARDS:
             raise ValueError(f"1..{_lib.URE_MAX_SHARDS} shards per launch")
+        if loss == "bpr" and lazy:
+            raise ValueError("loss='bpr' trains with the dense schedule only, not lazy")
+        mode = _bpr_mode(loss, mode)
+        self.loss = loss
         mode = ("lazy" if lazy else DEFAULT_MF_MODE) if mode is None else mode
         if mode not in ("dense", "lazy", "owner", "auto", "runs"):
             raise ValueError(f"mode {mode!r}")
@@ -664,6 +706,9 @@ class ShardBatch:
                 s.touched = torch.zeros(4 * (1 + batch), dtype=torch.int32, device=self.device)
             self.hp.mode, self.hp.decay, self.hp.decay_len = _lib.MF_LAZY, self.decay.data_ptr(), len(self.decay)
         self._upload_table()
+        if loss == "bpr":
+            self._bpr, self._bpr_keep = _bpr_table([s.inter for s in shards], [s.P.shape[0] for s in shards],
+                                                   shards[0].Q.shape[0], self.device)
         self.step = 0
 
     def _run_after_prepare(self):
@@ -877,8 +922,13 @@ class ShardBatch:
                 t1 = step_end
                 if self.mode in ("owner", "runs"):
                     t1 = min(step_end, self._schedule_window())
-                check(L.ure_mf_train(_ptr(self.table), self.n_shards, C.byref(self.hp), self.epochs,
-                                     self.step, t1, self.warps_group0, _ptr(self.ws), _stream()), "ure_mf_train")
+                if self.loss == "bpr":
+                    check(L.ure_mf_train_bpr(_ptr(self.table), _ptr(self._bpr), self.n_shards, C.byref(self.hp),
+                                             self.epochs, self.step, t1, self.warps_group0, _ptr(self.ws), _stream()),
+                          "ure_mf_train_bpr")
+                else:
+                    check(L.ure_mf_train(_ptr(self.table), self.n_shards, C.byref(self.hp), self.epochs,
+                                         self.step, t1, self.warps_group0, _ptr(self.ws), _stream()), "ure_mf_train")
                 self.launches_per_pass += 1
                 self.step = t1
 
@@ -957,6 +1007,7 @@ class ShardBatch:
                 ev = torch.cuda.Event()
                 ev.record(back)
         ns = self._shard_sizes()
+        bpr = self.loss == "bpr"
 
         def wait() -> List[np.ndarray]:
             ev.synchronize()
@@ -968,6 +1019,8 @@ class ShardBatch:
                 raise PlanHintMiss("ultrare_b200: the remembered owner plan does not cover this batch; repeat the pass")
             if err != 0:
                 raise RuntimeError("ultrare_b200: owner schedule asked for a step outside its scheduled window")
+            if bpr:                                  # mean softplus(-x) per triple, dropped triples counting zero
+                return [vals[j] / ns[j] for j in range(K)]
             return [np.sqrt(vals[j] / ns[j]) for j in range(K)]
         return wait
 
@@ -978,7 +1031,8 @@ class ShardBatch:
         return [max(1, s.n) for s in self.shards]
 
     def train_losses(self) -> List[np.ndarray]:
-        """Per shard: sqrt(sse_epoch / n) for every epoch (utils.py:108).  Synchronises (one D2H)."""
+        """Per shard: sqrt(sse_epoch / n) for every epoch (utils.py:108); BPR: the epoch's summed softplus(-x) / n.
+        Synchronises (one D2H)."""
         return self.train_losses_async()()
 
 
@@ -1014,14 +1068,16 @@ class ArenaShardBatch(ShardBatch):
     def __init__(self, recs, rows_P, n_item: int, d: int, batch: int, epochs: int, shard_ids, perm_seed: int = 42,
                  perms=None, lr: float = 1e-3, lr_decay: float = 0.95, lr_step: int = 50, weight_decay: float = 0.1,
                  momentum: float = 0.9, generator=None, std: float = 1.0, mode: str = "auto", owner_cache: bool = True,
-                 optimistic: bool = False, init=None):
+                 optimistic: bool = False, init=None, loss: str = "mse"):
         """init: per shard (P, Q) device tables the weights start from (copied into the arena) instead of the
         N(0, std) draw -- a SISA slice stage resumes from the previous stage's checkpoint; momentum and losses start
         cleared as always.
         optimistic: the caller reads the training losses (train_losses_async) only after everything that depends
         on the training is queued, and repeats the pass on PlanHintMiss.  The launch is then queued with the
         capacities of the last plan read back for the same shapes (+ PLAN_HINT_MARGIN) instead of waiting for this
-        one's -- the kernels compare them with the real plan on the device (hparams.owner_plan)."""
+        one's -- the kernels compare them with the real plan on the device (hparams.owner_plan).
+        loss: 'mse' or 'bpr' (as ShardBatch: BPR takes the dense schedule for mode 'auto' and refuses 'owner'); the
+        seen lists BPR samples against are built from `recs` in ordinary device allocations."""
         K = self.n_shards = len(recs)
         tq = [("start", time.perf_counter())]                # host stamps of the constructor (diagnostics: ctor_ms)
         stamp = lambda name: tq.append((name, time.perf_counter()))
@@ -1029,6 +1085,8 @@ class ArenaShardBatch(ShardBatch):
             raise ValueError(f"1..{_lib.URE_MAX_SHARDS} shards per launch")
         if mode not in ("dense", "owner", "auto"):
             raise ValueError(f"mode {mode!r}")
+        mode = _bpr_mode(loss, mode)
+        self.loss = loss
         _need_cuda(*recs)
         if init is not None:
             assert len(init) == K and not optimistic
@@ -1171,6 +1229,8 @@ class ArenaShardBatch(ShardBatch):
                     fill_weights()
             elif mode == "owner":
                 raise RuntimeError(f"owner mode does not fit this problem: {self.owner_plan}")
+        if loss == "bpr":
+            self._bpr, self._bpr_keep = _bpr_table(self._recs, self._rows_P, self._n_item, dev)
         _PINNED_BYTES.setdefault(stage.shape[0], []).append((stage, ev))
         stamp("end")
         self.ctor_ms = {b[0]: round((b[1] - a[1]) * 1e3, 4) for a, b in zip(tq[:-1], tq[1:])}
@@ -1630,14 +1690,16 @@ def _records_of(inters) -> torch.Tensor:
     return out
 
 
-def seen_lists(inter, n_user: int, n_item: int):
+def seen_lists(inter, n_user: int, n_item: int, validate: bool = True):
     """(off int64 [n_user + 1], items int32 [n]): every user's training items in ascending order, built on the device by
     ure_seen_lists (the owner set-up's stable radix sort, by item and then by user).  `inter`: an int32 [n, 4] record
-    tensor or a list of them (the shards' training sets); ids outside [0, n_user) / [0, n_item) raise ValueError."""
+    tensor or a list of them (the shards' training sets); ids outside [0, n_user) / [0, n_item) raise ValueError.
+    validate=False skips that check (one host synchronisation) for a caller that has checked the ids itself."""
     inter = _records_of(inter)
     _need_cuda(inter)
     n, dev = inter.shape[0], inter.device
-    if n > 0:           # the radix passes are sized by n_user / n_item: an id outside them would be mis-sorted silently
+    # the radix passes are sized by n_user / n_item: an id outside them would be mis-sorted silently
+    if n > 0 and validate:
         u, i = inter[:, 0], inter[:, 1]
         if bool(((u < 0) | (u >= n_user) | (i < 0) | (i >= n_item)).any()):
             raise ValueError(f"seen_lists: user ids must lie in [0, {n_user}) and item ids in [0, {n_item})")
@@ -1649,6 +1711,26 @@ def seen_lists(inter, n_user: int, n_item: int):
         check(L.ure_seen_lists(_ptr(inter), n, n_user, n_item, _ptr(off), _ptr(items), _ptr(scratch), _stream()),
               "ure_seen_lists")
     return off, items[:n]
+
+
+def bpr_negatives(inter: torch.Tensor, n_item: int, seen, perm_seed: int, shard_id: int, epoch: int,
+                  want_tries: bool = False):
+    """The negatives ure_mf_train_bpr draws in `epoch` for the records `inter` of one shard (int32 [n]; -1 = dropped
+    triple), against the seen lists `seen` = seen_lists(...) of that shard; with want_tries also the number of
+    candidates drawn per record."""
+    inter = inter.contiguous()
+    off, items = seen
+    _need_cuda(inter, off, items)
+    n, dev = int(inter.shape[0]), inter.device
+    neg = torch.empty(n, dtype=torch.int32, device=dev)
+    tries = torch.empty(n, dtype=torch.int32, device=dev) if want_tries else None
+    if items.numel() == 0:
+        items = torch.zeros(1, dtype=torch.int32, device=dev)
+    with torch.cuda.device(dev):
+        check(_lib.lib().ure_bpr_negatives(_ptr(inter), n, int(n_item), _ptr(off), _ptr(items), int(perm_seed) & 0xFFFFFFFF,
+                                           int(shard_id), int(epoch), _ptr(neg), _ptr(tries), _stream()),
+              "ure_bpr_negatives")
+    return (neg, tries) if want_tries else neg
 
 
 def item_sum(Q_list) -> torch.Tensor:

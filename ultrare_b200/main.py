@@ -37,6 +37,10 @@ def _build_parser():
                    help='how the SISA shard models are combined for the final evaluation and the recommendations: '
                         'mean = the reference\'s plain mean, fit = a per-group least-squares combination refitted '
                         'on the retained data after every unlearn (combine.npy)')
+    p.add_argument('--loss', default='mse', choices=['mse', 'bpr'],
+                   help='training objective: mse = the reference\'s squared error on the rating, bpr = pairwise '
+                        'ranking of each rated item over a sampled unrated one (implicit feedback, for --recommend); '
+                        'BPR runs write under their own run name (..._bpr)')
     p.add_argument('--grouping', default='emb-ot', choices=GROUP_TYPES,
                    help='how users are grouped into shards: emb-ot = OT clustering of the user table of a --group 0 '
                         'run, rating-ot = OT clustering of the users\' rating rows of the training file (no earlier '
@@ -63,7 +67,7 @@ parser = _build_parser()
 
 # request run: flag -> the manifest entry it must agree with when it is given
 _FROM_STATE = {'dataset': 'dataset', 'group': 'K', 'slices': 'slices', 'epoch': 'epochs', 'combine': 'combine',
-               'grouping': 'grouping', 'epoch_eval': 'epoch_eval'}
+               'grouping': 'grouping', 'epoch_eval': 'epoch_eval', 'loss': 'loss'}
 _NOT_WITH_REQUEST = ('delper', 'deltype', 'save_state')
 
 
@@ -83,6 +87,8 @@ def _checked(args):
     assert all(isinstance(w, int) for w in args.layer)
     assert 0 <= args.recommend <= 64, f'--recommend {args.recommend!r} is not accepted (0 .. 64)'
     assert 1 <= args.slices <= 32, f'--slices {args.slices!r} is not accepted (1 .. 32)'
+    assert not (args.loss == 'bpr' and args.combine == 'fit'), \
+        '--loss bpr cannot be combined with --combine fit (a least-squares fit on ratings; BPR scores are not ratings)'
     if args.slices > 1:
         assert args.epoch_eval != 'faithful', '--slices > 1 needs --epoch-eval final or none'
         assert args.group > 0, '--slices > 1 needs SISA shards (--group > 0)'
@@ -133,7 +139,9 @@ def main(argv=None):
     if a.synth:
         from . import synth
         synth.ensure_dataset(a.dataset)
-    ins = Instance(InsParam(a.dataset, a.epoch, a.worker, a.layer, a.group, a.delper, a.deltype))
+    param = InsParam(a.dataset, a.epoch, a.worker, a.layer, a.group, a.delper, a.deltype)
+    param.loss = a.loss
+    ins = Instance(param)
     ins.recommend_n = a.recommend
     ins.combine = a.combine
     ins.slices = a.slices

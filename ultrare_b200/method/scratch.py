@@ -39,6 +39,9 @@ class Scratch(object):
         self.momentum = param.momentum
         self.epochs = param.epochs
         self.batch = getattr(param, 'batch', 30000)
+        self.loss = getattr(param, 'loss', 'mse')
+        if self.loss not in ('mse', 'bpr'):
+            raise ValueError(f"loss must be 'mse' or 'bpr', not {self.loss!r}")
         self.device = _cuda_device()
         self.dis_type = getattr(param, 'dis_type', 'nor')
         self.attr = [] if self.dis_type == 'nor' else getattr(param, 'attr', [])
@@ -57,6 +60,7 @@ class Scratch(object):
         return isinstance(test_total, (list, tuple)) and len(test_total) == 0
 
     init_on_device = True     # False: host generator (same weights on any device, slower)
+    loss = 'mse'              # training objective (param.loss): 'mse' = the reference's, 'bpr' = pairwise ranking
 
     def _new_model(self, id, user_rows=None):
         gen = model_generator(self.seed, id, self.device if self.init_on_device else 'cpu')
@@ -70,7 +74,7 @@ class Scratch(object):
         else:
             model = given_model.to(self.device)
         opt = FusedSGD(model, lr=self.lr, weight_decay=self.lam, momentum=self.momentum, lr_decay=self.lr_decay,
-                       lr_step=50, epochs=self.epochs, perm_seed=self.seed, shard_id=id)
+                       lr_step=50, epochs=self.epochs, perm_seed=self.seed, shard_id=id, loss=self.loss)
 
         for t in range(self.epochs):
             if verbose == 2:

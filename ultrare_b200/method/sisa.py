@@ -266,6 +266,9 @@ class Sisa(Scratch):
         """True when the evaluation and recommend use the fitted combination; combine must be 'mean' or 'fit'."""
         if self.combine not in ('mean', 'fit'):
             raise ValueError(f"Sisa.combine must be 'mean' or 'fit', not {self.combine!r}")
+        if self.combine == 'fit' and self.loss == 'bpr':
+            raise ValueError("Sisa.combine='fit' cannot combine BPR shard models: the fit is least squares on the "
+                             "ratings, and BPR scores are not ratings; use combine='mean'")
         return self.combine == 'fit'
 
     def _fitted(self):
@@ -463,7 +466,7 @@ class Sisa(Scratch):
                                         perms if any(p is not None for p in perms) else None, self.lr, self.lr_decay,
                                         50, self.lam, self.momentum,
                                         generator=lambda: model_generator(self.seed, mine[0] + 1, self.device),
-                                        optimistic=optimistic)
+                                        optimistic=optimistic, loss=self.loss)
                 states = None
             else:
                 for j, i in enumerate(mine):
@@ -471,7 +474,8 @@ class Sisa(Scratch):
                     P, Q = models[i].user_mat.weight.data, models[i].item_mat.weight.data
                     states.append(kn.ShardState(recs[j], P, Q, E, shard_id=i + 1, perm_seed=self.seed,
                                                 perm=train_dlist[i].explicit_perm(self.device, E)))
-                sb = kn.ShardBatch(states, self.k, batch, self.lr, self.lr_decay, 50, self.lam, self.momentum)
+                sb = kn.ShardBatch(states, self.k, batch, self.lr, self.lr_decay, 50, self.lam, self.momentum,
+                                   loss=self.loss)
             self.timing['setup_alloc_ms'] = (t_a - t0) * 1e3
             self.timing['setup_upload_states_ms'] = (t_b - t_a) * 1e3
             self.timing['setup_batch_ms'] = (time.time() - t_b) * 1e3
@@ -731,6 +735,7 @@ class Sisa(Scratch):
 
     def learn(self, train_dlist, test_dlist, test_data, verbose, save_dir):
         """reference sisa.py:25-63."""
+        self._use_fit()                     # refuse a combine / loss conflict before anything trains
         if self._sliced():
             return self._learn_sliced(train_dlist, test_dlist, test_data, verbose, save_dir)
         return self._retrying(self._learn_once, train_dlist, test_dlist, test_data, verbose, save_dir)
@@ -789,6 +794,7 @@ class Sisa(Scratch):
 
     def unlearn(self, model_list, train_dlist, test_dlist, test_data, del_user, verbose, save_dir):
         """reference sisa.py:66-118."""
+        self._use_fit()
         if self._sliced():
             return self._unlearn_sliced(model_list, train_dlist, test_dlist, test_data, del_user, verbose, save_dir)
         return self._retrying(self._unlearn_once, model_list, train_dlist, test_dlist, test_data, del_user, verbose,
@@ -910,7 +916,7 @@ class Sisa(Scratch):
                                     self.n_item, self.k, batch, E1, [g + 1 for g in due], self.seed, None, self.lr,
                                     self.lr_decay, 50, self.lam, self.momentum,
                                     generator=lambda: model_generator(self.seed, mine[0] + 1, dev),
-                                    init=None if draw else [ck[g][j - 1] for g in due])
+                                    init=None if draw else [ck[g][j - 1] for g in due], loss=self.loss)
             views = sb.shards
             if draw:
                 for v, g in zip(views, due):
@@ -1066,6 +1072,7 @@ class Sisa(Scratch):
             man = dict(format=st.FORMAT_VERSION, K=K, slices=R, k=self.k, n_user=self.n_user, n_item=self.n_item,
                        epochs=self.epochs, batch=self.batch, lr=self.lr, lr_decay=self.lr_decay, lam=self.lam,
                        momentum=self.momentum, seed=self.seed, combine=self.combine, epoch_eval=self.epoch_eval,
+                       loss=self.loss,
                        dataset=src['dataset'], grouping=src['grouping'], max_rating=src['max_rating'],
                        train_file=dict(path=os.path.abspath(src['train_file']), bytes=int(src['train_bytes']),
                                        sha256=src['train_sha256']),
@@ -1089,7 +1096,7 @@ class Sisa(Scratch):
         man = st.read_manifest(state_dir)
         st.check_training_file(man)
         hp = types.SimpleNamespace(**{k: man[k] for k in ('n_user', 'n_item', 'k', 'lam', 'seed', 'lr', 'lr_decay',
-                                                           'momentum', 'epochs', 'batch')})
+                                                           'momentum', 'epochs', 'batch', 'loss')})
         for k, v in vars(hp).items():
             if param is not None and hasattr(param, k) and getattr(param, k) != v:
                 raise ValueError(f"param.{k} = {getattr(param, k)!r}, but the state in {state_dir} has {k} = {v!r}")

@@ -68,6 +68,9 @@ def read_manifest(state_dir):
     missing = [k for k in MANIFEST_KEYS if k not in man]
     if missing:
         raise ValueError(f"{path} is incomplete: it lacks {missing}")
+    man.setdefault('loss', 'mse')           # the training objective; states written before BPR training were MSE
+    if man['loss'] not in ('mse', 'bpr'):
+        raise ValueError(f"{path} has loss {man['loss']!r}; this build trains 'mse' or 'bpr'")
     return man
 
 

@@ -114,11 +114,13 @@ class FusedSGD:
 
     Holds the hyper-parameters; momentum buffers, gradient scratch and the step counter live
     in the ShardState the first ``baseTrain`` call binds to the (loader, model) pair.
+    loss: 'mse' (the reference's squared rating error) or 'bpr' (pairwise ranking, kernels.ShardBatch(loss='bpr')).
     """
 
     def __init__(self, model: MF, lr=1e-3, weight_decay=0.1, momentum=0.9, lr_decay=0.95, lr_step=50,
-                 epochs=1, perm_seed=42, shard_id=0):
+                 epochs=1, perm_seed=42, shard_id=0, loss='mse'):
         self.model = model
+        self.loss = loss
         self.lr, self.weight_decay, self.momentum = lr, weight_decay, momentum
         self.lr_decay, self.lr_step, self.epochs = lr_decay, lr_step, epochs
         self.perm_seed, self.shard_id = perm_seed, shard_id
@@ -132,7 +134,7 @@ class FusedSGD:
                                self.model.item_mat.weight.data, self.epochs, shard_id=self.shard_id,
                                perm_seed=self.perm_seed, perm=loader.explicit_perm(dev, self.epochs))
             self.batch_obj = kn.ShardBatch([st], self.model.k, loader.batch_size, self.lr, self.lr_decay,
-                                           self.lr_step, self.weight_decay, self.momentum)
+                                           self.lr_step, self.weight_decay, self.momentum, loss=self.loss)
         return self.batch_obj
 
 
@@ -141,7 +143,8 @@ def baseTrain(dataloader, model, loss_fn, is_rmse, opt, device, verbose, var='no
 
     ``opt`` is a FusedSGD; ``loss_fn`` is accepted for signature parity (the kernel computes
     MSELoss(reduction='sum'), scratch.py:45).  One persistent launch per call, one sync for
-    the epoch's loss (the reference syncs every batch, utils.py:82).
+    the epoch's loss (the reference syncs every batch, utils.py:82).  With ``opt.loss == 'bpr'`` both values are
+    the epoch's mean BPR loss, sum softplus(-x) / n.
     """
     assert var in ['nor'], "only the 'nor' path exists in the reference's reachable code"
     assert is_rmse, "the MF path uses MSELoss (scratch.py:44-46)"
@@ -153,7 +156,10 @@ def baseTrain(dataloader, model, loss_fn, is_rmse, opt, device, verbose, var='no
     sb.train((ep + 1) * st.steps_per_epoch(sb.hp.batch))
     opt.epoch += 1
     sse = float(st.sse[ep].item())
-    train_loss = float(np.sqrt(sse / max(1, st.n)))
+    if opt.loss == 'bpr':
+        train_loss = sse / max(1, st.n)
+    else:
+        train_loss = float(np.sqrt(sse / max(1, st.n)))
     return train_loss, train_loss
 
 
