@@ -318,7 +318,8 @@ int ure_score_finalize(const float* d_sum, const ure_inter_t* d_inter, int64_t n
 /* HR@10 / NDCG@10 of baseTest (method/utils.py:166-184) over user segments.
  * Segment s covers rows d_order[d_seg[s] .. d_seg[s+1]) (d_order NULL = identity).
  * d_out[0] += sum_u ndcg_u ; d_out[1] += sum_u hr_u ; d_out[2] += #users.
- * Tie rule: descending value, later index first (np.argsort(kind='stable')[::-1]). */
+ * Tie rule: descending value, later index first (np.argsort(kind='stable')[::-1]), in NumPy's order
+ * of floats: a NaN score ranks above +inf and ties with every other NaN; -0 and +0 tie. */
 int ure_rank_metrics(const ure_inter_t* d_inter, const float* d_score, const int32_t* d_order,
                      const int64_t* d_seg, int64_t n_seg, double* d_out, void* stream);
 

@@ -89,6 +89,7 @@ ensemble_score_jobs_kernel(const ure_eval_job_t* __restrict__ jobs) {
 // ---------------------------------------------------------------------------
 // HR@10 / NDCG@10 per user segment, one warp per user (utils.py:166-181).
 //   rank_v(e) = #{e' : v(e') > v(e) or (v(e') == v(e) and e' > e)}   ("later index first")
+//   where > and == are NumPy's sort order: NaN above +inf and equal to every NaN, -0 == +0 (rank_key)
 //   top_pred[p] / top_rating[p] = element of rank p  (p < 10)
 //   relevance[p] = r[top_pred[p]] ; hit = relevance >= 4/5 ; HR = #hit / 10
 //   common[p] = top_rating[p] in set(top_pred)        (positional, utils.py:179)
@@ -104,12 +105,28 @@ __constant__ double kDcgWeight[URE_TOP_K] = {1.0, 1.0, 0.6309297535714575, 0.5, 
                                              0.31546487678572877, 0.3010299956639812};
 constexpr double kIdcg = 5.254494511770457;
 
+// Unsigned key whose order is the order np.sort puts float values in: every NaN maps to the top key (a NaN score ranks
+// first, as in argsort(kind='stable')[::-1]), -0 and +0 share a key.  The order on keys is total, so the ranks of a
+// segment are a permutation and every slot of the top-10 lists is written exactly once (float comparisons are false for
+// NaN: several elements would share a rank and slots would stay unwritten).  Every key is > 0.
+// (selects, not branches: branches here keep the compiler from unrolling the staging loop)
+__device__ __forceinline__ unsigned rank_key(float v) {
+  const unsigned b = __float_as_uint(v);
+  const unsigned k = b ^ ((unsigned)((int)b >> 31) | 0x80000000u);      // negative: ~b, positive: b | sign bit
+  return v != v ? 0xffffffffu : (v == 0.f ? 0x80000000u : k);
+}
+
+// the value of a key (not NaN; -0 comes back as +0): the relevance of a staged rating without another global load
+__device__ __forceinline__ float key_value(unsigned k) {
+  return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
+}
+
 __device__ __forceinline__ void rank_metrics_body(const ure_inter_t* __restrict__ inter, const float* __restrict__ score,
                                                   const int32_t* __restrict__ order, const long long* __restrict__ seg,
                                                   long long n_seg, double* __restrict__ out) {
   __shared__ int top_pred[8][URE_TOP_K];
   __shared__ int top_rating[8][URE_TOP_K];
-  __shared__ float2 s_vt[8][kSegStage];
+  __shared__ uint2 s_key[8][kSegStage];
   const int lane = threadIdx.x & 31;
   const int w = threadIdx.x >> 5;
   const long long n_warps = ((long long)gridDim.x * blockDim.x) >> 5;
@@ -123,16 +140,32 @@ __device__ __forceinline__ void rank_metrics_body(const ure_inter_t* __restrict_
     if (L <= 0) continue;
     if (lane < URE_TOP_K) { top_pred[w][lane] = -1; top_rating[w][lane] = -1; }
     const bool staged = L <= kSegStage;
-    // (score, rating) of element f of the segment: from shared memory, or -- very long segments -- from global memory
-    auto value_of = [&](int f) {
-      if (staged) return s_vt[w][f];
-      const long long rf = order ? order[b + f] : b + f;
-      return make_float2(score[rf], inter[rf].rating);
+    auto row_of = [&](int f) { return order ? (long long)order[b + f] : b + f; };
+    // rank keys of (score, rating) of element f of the segment: from shared memory, or -- very long segments -- from
+    // global memory
+    auto staged_key = [&](int f) { return s_key[w][f]; };
+    auto global_key = [&](int f) {
+      const long long rf = row_of(f);
+      return make_uint2(rank_key(score[rf]), rank_key(inter[rf].rating));
+    };
+    // every lane counts the elements ranked before its own, both orders in one sweep
+    auto count_ranks = [&](auto key_of) {
+      for (int e = lane; e < L; e += 32) {
+        const uint2 me = key_of(e);
+        int rp = 0, rr = 0;
+        for (int f = 0; f < L; ++f) {
+          const uint2 o = key_of(f);
+          rp += (o.x > me.x) || (o.x == me.x && f > e);
+          rr += (o.y > me.y) || (o.y == me.y && f > e);
+        }
+        if (rp < URE_TOP_K) top_pred[w][rp] = e;
+        if (rr < URE_TOP_K) top_rating[w][rr] = e;
+      }
     };
     if (staged)
       for (int e = lane; e < L; e += 32) {
-        const long long re = order ? order[b + e] : b + e;
-        s_vt[w][e] = make_float2(score[re], inter[re].rating);
+        const long long re = row_of(e);
+        s_key[w][e] = make_uint2(rank_key(score[re]), rank_key(inter[re].rating));
       }
     __syncwarp();
     if (staged && L > kSegCount) {
@@ -142,16 +175,16 @@ __device__ __forceinline__ void rank_metrics_body(const ure_inter_t* __restrict_
       unsigned taken_p = 0, taken_r = 0;     // bit k: element lane + 32 k is already placed in that order
       const int P = L < URE_TOP_K ? L : URE_TOP_K;
       for (int p = 0; p < P; ++p) {
-        float vp = -INFINITY, vr = -INFINITY;
+        unsigned vp = 0u, vr = 0u;           // below every key: an untaken element always wins its round
         int ep = -1, er = -1;
         for (int k = 0, e = lane; e < L; ++k, e += 32) {
-          const float2 x = s_vt[w][e];
+          const uint2 x = s_key[w][e];
           if (!((taken_p >> k) & 1u) && (x.x > vp || (x.x == vp && e > ep))) { vp = x.x; ep = e; }
           if (!((taken_r >> k) & 1u) && (x.y > vr || (x.y == vr && e > er))) { vr = x.y; er = e; }
         }
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) {
-          const float ovp = __shfl_xor_sync(0xffffffffu, vp, o), ovr = __shfl_xor_sync(0xffffffffu, vr, o);
+          const unsigned ovp = __shfl_xor_sync(0xffffffffu, vp, o), ovr = __shfl_xor_sync(0xffffffffu, vr, o);
           const int oep = __shfl_xor_sync(0xffffffffu, ep, o), oer = __shfl_xor_sync(0xffffffffu, er, o);
           if (ovp > vp || (ovp == vp && oep > ep)) { vp = ovp; ep = oep; }
           if (ovr > vr || (ovr == vr && oer > er)) { vr = ovr; er = oer; }
@@ -160,26 +193,18 @@ __device__ __forceinline__ void rank_metrics_body(const ure_inter_t* __restrict_
         if (ep >= 0 && (ep & 31) == lane) taken_p |= 1u << (ep >> 5);
         if (er >= 0 && (er & 31) == lane) taken_r |= 1u << (er >> 5);
       }
+    } else if (staged) {
+      // short segments (the common case: a few test rows per user): broadcast reads of shared memory
+      count_ranks(staged_key);
     } else {
-      // short segments (the common case: a few test rows per user) and the very long ones that are not staged: every
-      // lane counts the elements ranked before its own, both orders in one sweep (broadcast reads of shared memory)
-      for (int e = lane; e < L; e += 32) {
-        const float2 me = value_of(e);
-        int rp = 0, rr = 0;
-        for (int f = 0; f < L; ++f) {
-          const float2 o = value_of(f);
-          rp += (o.x > me.x) || (o.x == me.x && f > e);
-          rr += (o.y > me.y) || (o.y == me.y && f > e);
-        }
-        if (rp < URE_TOP_K) top_pred[w][rp] = e;
-        if (rr < URE_TOP_K) top_rating[w][rr] = e;
-      }
+      // the very long ones that are not staged (a loop of their own: the key arithmetic stays out of the staged one)
+      count_ranks(global_key);
     }
     __syncwarp();
     double rel = 0.0, hit = 0.0;
     if (lane < URE_TOP_K && lane < L) {
       const int ep = top_pred[w][lane];
-      const double relevance = (double)value_of(ep).y;
+      const double relevance = staged ? key_value(s_key[w][ep].y) : inter[row_of(ep)].rating;
       const bool h = relevance >= (4.0 / 5.0);
       const int tr = top_rating[w][lane];
       bool common = false;
